@@ -22,7 +22,7 @@ TRACK (`match.track_sharded`, SURVEY §8e's alternative).  Identity is checked i
 every query, a 256-query subsample against ONE index holding all rows on rank 0, and a checksum of all results that is
 the same number at every N.
 
-Launch: python bench.py [--gpus N --steps K --warmup W]; for N>1 under torchrun.
+Launch: python bench.py [--gpus N --steps K --warmup W --dump-outputs DIR]; for N>1 under torchrun.
 """
 from __future__ import annotations
 
@@ -77,7 +77,15 @@ def parse():
     ap.add_argument("--match-check-queries", type=int, default=256, help="N>1: subsample checked against one full index")
     ap.add_argument("--match-cpu-tracks", type=int, default=2714, help="index size of the CPU baseline (configs[2])")
     ap.add_argument("--no-peer", action="store_true", help="N>1: skip the peer-memory (fused exchange) variant of the hash-prefix path")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32/float64, "
+                         "a fixed seeded sample where the whole does not fit 64 MB; N>1: rank 0's tracks, every query)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
+    return args
 
 
 # ------------------------------------------------------------------------------------------
@@ -261,6 +269,36 @@ def per_kernel_roofline(kernel_ms, audio_s, n_hashes, peak_gbs, digest_table):
     return out
 
 
+# --dump-outputs: bytes of data per group of row-aligned outputs; 63 MB in all, so that with the .npy headers the files
+# stay under 64 MB
+DUMP_BYTES = {"fingerprint": 44_000_000, "fingerprint_tracks": 4_000_000, "match": 15_000_000}
+
+
+def dump_rows(out_dir, group, columns, seed):
+    """Writes ``out_dir/<group>_<name>.npy`` for every column (a numpy array or a tensor, rows first, all with the same
+    number of rows) and ``<group>_index.npy``, the row numbers written: every row when they fit the group's share of
+    DUMP_BYTES, else a fixed sample (``seed``) of as many rows as fit, in row order.  8- and 16-bit integers are
+    written as float32, everything else as float64: both hold the values exactly."""
+    def out_dtype(c):
+        return np.float32 if c.dtype.itemsize <= 2 else np.float64
+
+    def row_bytes(c):
+        return int(np.prod(c.shape[1:], dtype=np.int64)) * np.dtype(out_dtype(c)).itemsize
+
+    n = len(next(iter(columns.values())))
+    k = max(1, DUMP_BYTES[group] // (8 + sum(row_bytes(c) for c in columns.values())))
+    idx = np.arange(n) if n <= k else np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"{group}_index.npy"), idx.astype(np.float64))
+    for name, c in columns.items():
+        if isinstance(c, np.ndarray):
+            rows = c[idx]
+        else:
+            import torch
+            rows = c[torch.from_numpy(idx).to(c.device)].cpu().numpy()
+        np.save(os.path.join(out_dir, f"{group}_{name}.npy"), rows.astype(out_dtype(c)))
+
+
 def measured_peak_gbs():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -322,12 +360,15 @@ def fingerprint_leg(args, rank, world, local_rank, dev, config):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step_device()
+        last = step_device()
     e1.record()
     barrier()
     ms_total = e0.elapsed_time(e1)
     clocks = sampler.stop()
     kms, klaunch = fp.timing(False)
+    if args.dump_outputs and rank == 0:
+        dump_rows(args.dump_outputs, "fingerprint", {"hash": last.hash, "t1": last.t1}, seed=1)
+        dump_rows(args.dump_outputs, "fingerprint_tracks", {"starts": last.starts}, seed=2)
     t_dev = torch.tensor([ms_total], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t_dev, op=dist.ReduceOp.MAX)
@@ -804,6 +845,10 @@ def match_leg(args, rank, world, local_rank, dev):
     nth = cnt[:, topn - 1]
     nth_hist = {str(int(v)): int(c) for v, c in zip(*np.unique(np.minimum(nth, 16), return_counts=True))}
     total_hashes = sum(r["hashes"] for r in allr)
+    if args.dump_outputs:
+        order = np.argsort(qids, kind="stable")          # row q = query q
+        dump_rows(args.dump_outputs, "match", {name: a[order] for name, a in zip(("song", "diff", "count", "rows", "nres"), cat)},
+                  seed=3)
 
     out = {"metric": "match_queries_per_second", "value": Q / (ms_step * 1e-3), "unit": "queries/s", "n_gpus": world,
            "steps": args.steps, "warmup": max(args.warmup, 3), "ms_per_step": ms_step, "ms_per_step_median": ms_med,

@@ -1,8 +1,8 @@
 #!/usr/bin/env python
 """Generate the committed golden vectors by EXECUTING THE REFERENCE'S OWN CODE.
 
-Run in the dev container only (``/root/reference`` does not exist on the GPU
-box):  ``python tests/golden/make_golden.py``
+Needs a checkout of the reference project, named by ``SIA_REFERENCE_DIR``:
+``SIA_REFERENCE_DIR=<checkout> python tests/golden/make_golden.py [out_dir]``
 
 How: the reference scripts cannot be imported (they open PortAudio / MySQL at
 import and need matplotlib, pydub, ... which are absent), so the pure functions
@@ -40,7 +40,7 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF = "/root/reference"
+REF = os.environ.get("SIA_REFERENCE_DIR", "")
 
 from oracle import sia_oracle as O  # noqa: E402
 

@@ -45,6 +45,32 @@ def test_results_digest_is_order_independent():
     assert bench.results_digest(qids, res, topn) != d0
 
 
+def test_dump_rows_exact_values_fixed_sample_and_size(tmp_path):
+    rng = np.random.default_rng(1)
+    n = 2_000_000                                       # 56 bytes per row: more than the group's 44 MB
+    h = rng.integers(0, 256, (n, 10)).astype(np.uint8)
+    t1 = rng.integers(0, 1 << 31, n).astype(np.int32)
+    for d in ("a", "b"):
+        bench.dump_rows(str(tmp_path / d), "fingerprint", {"hash": h, "t1": t1}, seed=1)
+    idx = np.load(tmp_path / "a" / "fingerprint_index.npy")
+    assert idx.dtype == np.float64 and len(idx) == 44_000_000 // 56 and np.all(np.diff(idx) > 0)
+    k = idx.astype(np.int64)
+    got_h, got_t1 = np.load(tmp_path / "a" / "fingerprint_hash.npy"), np.load(tmp_path / "a" / "fingerprint_t1.npy")
+    assert got_h.dtype == np.float32 and np.array_equal(got_h, h[k]) and got_t1.dtype == np.float64 and np.array_equal(got_t1, t1[k])
+    for f in os.listdir(tmp_path / "a"):
+        assert open(tmp_path / "a" / f, "rb").read() == open(tmp_path / "b" / f, "rb").read(), f
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= 44_000_000 + 3 * 128
+    bench.dump_rows(str(tmp_path / "c"), "match", {"song": t1[:10].reshape(5, 2)}, seed=3)     # small: every row
+    assert np.array_equal(np.load(tmp_path / "c" / "match_index.npy"), np.arange(5))
+    assert np.array_equal(np.load(tmp_path / "c" / "match_song.npy"), t1[:10].reshape(5, 2))
+
+
+def test_steps_below_one_are_refused():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"],
+                         capture_output=True, text=True, timeout=120)
+    assert out.returncode == 2 and "--steps must be at least 1" in out.stderr
+
+
 def test_reference_arm_prints_the_contract_line():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0",
                           "--track-samples", "220500", "--cpu-sample-tracks", "2"], capture_output=True, text=True, timeout=300)
