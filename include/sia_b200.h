@@ -152,8 +152,37 @@ int sia_fingerprint_batch_host(sia_ctx *ctx, const int16_t *h_pcm, const int64_t
                                int64_t *h_track_hash_starts, int64_t *h_total);
 
 /* per-kernel device time (ms, CUDA events on the launching stream) accumulated since the
- * last reset; order: stft, peaks(bitmap), peaks(compact), pairs+sha1, scans.  n <= 8. */
+ * last reset; order: stft, peaks(bitmap), peaks(compact), pairs+sha1, scans, stream-state copies
+ * (staging, row assembly, peak splice and commit of sia_stream_push).  n <= 8. */
 int sia_ctx_timing(sia_ctx *ctx, int enable, double *h_ms_out, int32_t *h_launches_out, int32_t n);
+
+/* ---- streaming: many concurrent streams, fed block by block ------------------------------------------------------
+ * A stream handle holds n_streams independent streams on one context.  Each push gives every stream a block of int16
+ * PCM (possibly empty); h_end[b] != 0 marks the block as stream b's last, after which the stream starts over at frame 0.
+ * A push returns, per stream, the hashes that became final in it: with F complete frames so far, rows up to
+ * H = F - 1 - nbhd have their whole neighbourhood, their peaks are final, and an anchor is final once it has
+ * fan_value - 1 peaks behind it or t <= H - MAX_HASH_TIME_DELTA; at the end everything is.  So for ANY cut of a
+ * stream's PCM into blocks, the concatenation of everything emitted up to and including the end push equals
+ * sia_fingerprint_batch on the whole PCM with the same parameters (digests, t1 = frame index from the stream's start,
+ * order), short-input padding included.  Streams longer than the context workspace are fine: a push only needs the
+ * carried 2*nbhd rows + its new frames of each stream to fit max_chunk_frames.
+ *
+ * The handle keeps per-stream state in HBM (allocated at create, two copies: ~2 * (8 KB + nbhd * 16.6 KB) per stream,
+ * plus one max_chunk_frames spectrogram for new rows) and uses its context's workspaces: calls on a context and its
+ * stream handles must be serialised by the caller, and stream handles are destroyed before their context.
+ * Parameters as sia_fingerprint_batch (wsize 4096, wratio 0.5 only). */
+typedef struct sia_stream sia_stream;
+int sia_stream_create(sia_ctx *ctx, int32_t n_streams, const sia_fp_params *p, sia_stream **out);
+int sia_stream_destroy(sia_stream *st);
+/* Block b of the push: samples [h_block_starts[b], +h_block_len[b]) of d_pcm (starts multiples of 8, as in the batch
+ * path; ignored for empty blocks).  h_end: n_streams flags, or NULL for none.  Outputs like sia_fingerprint_batch:
+ * digests and t1 on the device, h_stream_hash_starts (n_streams+1, optional) and *h_total on the host after ONE
+ * synchronisation.  A push that fails leaves every stream exactly as it was: SIA_E_CAPACITY when cap_hashes is too
+ * small (*h_total = rows needed), when a stream's carried + new rows exceed the workspace (push smaller blocks) or the
+ * peak workspace overflows; the push can then be retried. */
+int sia_stream_push(sia_stream *st, const int16_t *d_pcm, const int64_t *h_block_starts, const int64_t *h_block_len,
+                    const uint8_t *h_end, uint8_t *d_hash, int32_t *d_t1, int64_t cap_hashes,
+                    int64_t *h_stream_hash_starts, int64_t *h_total, void *stream);
 
 /* ---- noise-robustness harness (SURVEY §8f-3) -------------------------------------------------------------------- */
 /* get_noise_from_sound + the mix (recognizer_test.py:426-435, 554) for a batch of clips: clip c reads n_samples int16

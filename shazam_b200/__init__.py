@@ -5,6 +5,7 @@ Layout (only what the hot path needs):
   _native.py       ctypes binding of the C ABI — no CPU fallback
   fingerprinter.py array-typed host driver (K1 STFT->dB, K2 peaks, K3 pairs+SHA-1)
   compat.py        the reference's function names/signatures on top of it
+  stream.py        StreamFingerprinter: many concurrent streams fed block by block, same hashes as whole tracks
 """
 __version__ = "0.1.0"
 
@@ -17,7 +18,7 @@ def __getattr__(name):
                 "as_pcm_int16"):
         from . import fingerprinter
         return getattr(fingerprinter, name)
-    if name in ("compat", "fingerprinter", "database", "recognize", "distributed"):
+    if name in ("compat", "fingerprinter", "database", "recognize", "distributed", "stream"):
         import importlib
         return importlib.import_module(f"{__name__}.{name}")
     raise AttributeError(name)

@@ -56,6 +56,9 @@ SIGNATURES = {
     "sia_fingerprint_batch_host": (C.c_int, [_p, _p, _i64p, _i64p, C.c_int32, C.POINTER(FpParams), _p, _p,
                                              C.c_int64, _i64p, _i64p]),
     "sia_ctx_timing": (C.c_int, [_p, C.c_int, C.POINTER(C.c_double), _i32p, C.c_int32]),
+    "sia_stream_create": (C.c_int, [_p, C.c_int32, C.POINTER(FpParams), C.POINTER(_p)]),
+    "sia_stream_destroy": (C.c_int, [_p]),
+    "sia_stream_push": (C.c_int, [_p, _p, _i64p, _i64p, _p, _p, _p, C.c_int64, _i64p, _i64p, _p]),
     "sia_mix_noise": (C.c_int, [C.c_int, _p, C.c_int64, _p, C.c_int64, C.c_int32, C.c_int64, C.c_double, _p, C.c_int64, _p, _p]),
     "sia_index_create": (C.c_int, [C.c_int, C.c_int64, C.POINTER(_p)]),
     "sia_index_destroy": (C.c_int, [_p]),

@@ -3,8 +3,7 @@
 // (H2D | kernels | D2H on three streams).  This is the native runtime behind
 // fingerprint()/_fingerprint_worker (__init__.py:212-284): the reference fans tracks out
 // over a multiprocessing.Pool; here a batch is one call and the chunk loop is the pool.
-#include "sia_common.cuh"
-#include "stft.cuh"
+#include "ctx.cuh"
 
 #include <algorithm>
 #include <cstdlib>
@@ -27,79 +26,7 @@ int cuda_fail(cudaError_t e, const char *what, const char *file, int line) {
 
 using namespace sia;
 
-enum { T_STFT = 0, T_PEAKS = 1, T_COMPACT = 2, T_PAIRS = 3, T_SCAN = 4, T_NCAT = 5 };
-
-struct TimedSpan { cudaEvent_t a, b; int cat; };
-
-struct sia_ctx {
-  int device = 0;
-  int64_t max_frames = 0;
-  int64_t cap_peaks = 0;
-  int64_t cap_chunk_hashes = 0;
-  StftTables<float> tf;
-  StftTables<double> td;
-  // chunk workspace
-  float *spec = nullptr;
-  uint32_t *bitmap = nullptr;
-  uint32_t *row_count = nullptr;
-  int64_t *row_off = nullptr;
-  int32_t *peak_t = nullptr, *peak_f = nullptr;
-  uint32_t *pair_count = nullptr;
-  int64_t *pair_off = nullptr;
-  void *scan_tmp = nullptr;
-  int32_t *status = nullptr;      // device flag word
-  int64_t *hash_base = nullptr;   // device scalar: running output offset
-  void *digest_table = nullptr;   // optional: sha1 of every (f1, f2, dt) the pipeline can produce (sia_ctx_digest_table)
-  // batch metadata (grown on demand)
-  int64_t *d_meta = nullptr;
-  size_t d_meta_cap = 0;
-  // host pipeline
-  cudaStream_t s_h2d = nullptr, s_comp = nullptr, s_d2h = nullptr;
-  int16_t *pcm_stage[2] = {nullptr, nullptr};
-  int64_t pcm_stage_samples = 0;
-  uint8_t *hash_stage[2] = {nullptr, nullptr};
-  int32_t *t1_stage[2] = {nullptr, nullptr};
-  int64_t *h_pinned = nullptr;    // pinned scratch: counts and track_hash_starts per chunk
-  size_t h_pinned_cap = 0;
-  // timing
-  bool timing = false;
-  std::vector<TimedSpan> spans;
-  std::vector<cudaEvent_t> ev_pool;
-  double ms[T_NCAT] = {0, 0, 0, 0, 0};
-  int launches[T_NCAT] = {0, 0, 0, 0, 0};
-};
-
-namespace {
-
-struct Timer {
-  sia_ctx *c; cudaStream_t s; int cat; int nlaunch; cudaEvent_t a = nullptr, b = nullptr;
-  Timer(sia_ctx *c_, cudaStream_t s_, int cat_, int nlaunch_) : c(c_), s(s_), cat(cat_), nlaunch(nlaunch_) {
-    c->launches[cat] += nlaunch;
-    if (!c->timing) return;
-    auto get = [&]() {
-      cudaEvent_t e;
-      if (!c->ev_pool.empty()) { e = c->ev_pool.back(); c->ev_pool.pop_back(); } else cudaEventCreate(&e);
-      return e;
-    };
-    a = get(); b = get();
-    cudaEventRecord(a, s);
-  }
-  ~Timer() {
-    if (!c->timing) return;
-    cudaEventRecord(b, s);
-    c->spans.push_back({a, b, cat});
-  }
-};
-
-void collect_timing(sia_ctx *c) {
-  for (auto &sp : c->spans) {
-    float ms = 0;
-    if (cudaEventElapsedTime(&ms, sp.a, sp.b) == cudaSuccess) c->ms[sp.cat] += ms;
-    c->ev_pool.push_back(sp.a);
-    c->ev_pool.push_back(sp.b);
-  }
-  c->spans.clear();
-}
+namespace sia {
 
 int check_params(const sia_fp_params *p) {
   SIA_REQUIRE(p != nullptr, SIA_E_INVALID, "params is NULL");
@@ -135,6 +62,20 @@ int ensure_pinned(sia_ctx *c, size_t n_i64) {
   return SIA_OK;
 }
 
+}  // namespace sia
+
+namespace {
+
+void collect_timing(sia_ctx *c) {
+  for (auto &sp : c->spans) {
+    float ms = 0;
+    if (cudaEventElapsedTime(&ms, sp.a, sp.b) == cudaSuccess) c->ms[sp.cat] += ms;
+    c->ev_pool.push_back(sp.a);
+    c->ev_pool.push_back(sp.b);
+  }
+  c->spans.clear();
+}
+
 // One chunk = tracks [b0, b1) whose frames fit the workspace.
 struct Chunk {
   int b0, b1;
@@ -167,7 +108,8 @@ int plan_chunks(sia_ctx *c, const int64_t *h_len, int n_tracks, int64_t max_samp
       const int64_t fr = sia_num_frames(h_len[ch.b1]);
       if (fr > c->max_frames) {
         char buf[256];
-        snprintf(buf, sizeof buf, "track %d has %lld frames; the context workspace holds %lld (raise max_chunk_frames)",
+        snprintf(buf, sizeof buf, "track %d has %lld frames; the context workspace holds %lld (raise max_chunk_frames, "
+                 "or fingerprint it block by block with sia_stream_push)",
                  ch.b1, (long long)fr, (long long)c->max_frames);
         set_error(buf);
         return SIA_E_CAPACITY;

@@ -19,13 +19,16 @@ namespace {
 
 __global__ void __launch_bounds__(256)
 pairs_count_kernel(const int32_t *__restrict__ peak_t, const int64_t *__restrict__ track_peak_starts, int n_tracks,
-                   int fan_value, uint32_t *__restrict__ pair_count) {
+                   int fan_value, const int64_t *__restrict__ final_t, uint32_t *__restrict__ pair_count) {
   const int64_t n_peaks = track_peak_starts[n_tracks];
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_peaks; i += (int64_t)gridDim.x * blockDim.x) {
     const int trk = find_segment(track_peak_starts, n_tracks, i);
     const int64_t e = track_peak_starts[trk + 1];
     const int t1 = peak_t[i];
     int m = 0;
+    // streaming: an anchor whose partners are not all known yet (fewer than fan_value-1 peaks behind it, and a later
+    // peak could still lie within MAX_HASH_TIME_DELTA) gets no pairs in this pass
+    if (final_t && i + fan_value - 1 >= e && t1 > final_t[trk]) { pair_count[i] = 0; continue; }
     for (int j = 1; j < fan_value; ++j) {
       if (i + j >= e) break;
       const int dt = peak_t[i + j] - t1;
@@ -167,11 +170,13 @@ __global__ void track_hash_starts_kernel(const int64_t *__restrict__ track_peak_
 }  // namespace
 
 int pairs_count_launch(const int32_t *d_peak_t, const int64_t *d_track_peak_starts, int n_tracks,
-                       int64_t n_peaks_max, int fan_value, uint32_t *d_pair_count, cudaStream_t s) {
+                       int64_t n_peaks_max, int fan_value, uint32_t *d_pair_count, cudaStream_t s,
+                       const int64_t *d_final_t) {
   if (n_peaks_max == 0) return SIA_OK;
   int64_t blocks = ceil_div(n_peaks_max, 256);
   if (blocks > kNumSMs * 16) blocks = kNumSMs * 16;
-  pairs_count_kernel<<<(unsigned)blocks, 256, 0, s>>>(d_peak_t, d_track_peak_starts, n_tracks, fan_value, d_pair_count);
+  pairs_count_kernel<<<(unsigned)blocks, 256, 0, s>>>(d_peak_t, d_track_peak_starts, n_tracks, fan_value, d_final_t,
+                                                      d_pair_count);
   SIA_CHECK_LAUNCH();
   return SIA_OK;
 }

@@ -464,12 +464,27 @@ int launch_generic(const PeaksLaunch &a, cudaStream_t s) {
 // Two bitmap layouts, both with a row stride of kBitmapRowWords words:
 //   plain   : word w, bit b            <-> bin 32*w + b              (65 words; tile / generic kernels)
 //   striped : word 4*s + e, bit l      <-> bin 96*s + 4*l + e        (22 strips x 4 words; warp kernel)
-template <bool STRIPED>
+// WIN (streaming): rows outside their segment's emit window count 0 and yield nothing (PeakWindow, stft.cuh)
+__device__ __forceinline__ bool row_in_window(const PeakWindow &w, int64_t g, int &seg, int64_t &k) {
+  seg = find_segment(w.frame_starts, w.n, g);
+  k = g - w.frame_starts[seg];
+  return k >= w.emit_lo[seg] && k < w.emit_hi[seg];
+}
+
+template <bool STRIPED, bool WIN>
 __global__ void __launch_bounds__(256)
-rowcount_kernel(const uint32_t *__restrict__ bitmap, int64_t total_frames, uint32_t *__restrict__ row_count) {
+rowcount_kernel(const uint32_t *__restrict__ bitmap, int64_t total_frames, uint32_t *__restrict__ row_count,
+                const PeakWindow win) {
   const int lane = threadIdx.x & 31;
   const int64_t g = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (g >= total_frames) return;
+  if (WIN) {
+    int seg; int64_t k;
+    if (!row_in_window(win, g, seg, k)) {
+      if (lane == 0) row_count[g] = 0;
+      return;
+    }
+  }
   const uint32_t *row = bitmap + g * kBitmapRowWords;
   int c = 0;
   if (STRIPED) {
@@ -486,19 +501,28 @@ rowcount_kernel(const uint32_t *__restrict__ bitmap, int64_t total_frames, uint3
   if (lane == 0) row_count[g] = (uint32_t)c;
 }
 
-template <bool STRIPED>
+template <bool STRIPED, bool WIN>
 __global__ void __launch_bounds__(256)
 extract_kernel(const uint32_t *__restrict__ bitmap, const int64_t *__restrict__ row_off,
                const int64_t *__restrict__ frame_starts, int n_tracks, int64_t total_frames, int64_t peak_base,
                int32_t *__restrict__ peak_t, int32_t *__restrict__ peak_f, int64_t cap,
-               int64_t *__restrict__ track_peak_starts, int32_t *__restrict__ status) {
+               int64_t *__restrict__ track_peak_starts, int32_t *__restrict__ status, const PeakWindow win) {
   const int lane = threadIdx.x & 31;
   const int64_t g = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (g >= total_frames) return;
-  const int trk = find_segment(frame_starts, n_tracks, g);
-  const int k = (int)(g - frame_starts[trk]);
+  int trk;
+  int k;
   int64_t base = row_off[g] + peak_base;
-  if (lane == 0) {
+  if (WIN) {
+    int64_t kl;
+    if (!row_in_window(win, g, trk, kl)) return;
+    k = (int)(kl + win.t_base[trk]);
+    base += win.peak_off[trk];
+  } else {
+    trk = find_segment(frame_starts, n_tracks, g);
+    k = (int)(g - frame_starts[trk]);
+  }
+  if (!WIN && lane == 0) {
     // prefix offsets never point past the workspace: the peaks beyond `cap` are dropped (status bit 1), and the
     // kernels that follow (pair counting, scans, SHA-1) read these counts from the device
     if (k == 0) track_peak_starts[trk] = min(base, cap);
@@ -575,11 +599,17 @@ int peaks_bitmap_launch(const PeaksLaunch &a, cudaStream_t s, bool *striped) {
 }
 
 int peaks_rowcount_launch(const uint32_t *d_bitmap, bool striped, int64_t total_frames, uint32_t *d_row_count,
-                          cudaStream_t s) {
+                          cudaStream_t s, const PeakWindow *win) {
   if (total_frames == 0) return SIA_OK;
   const unsigned blocks = (unsigned)ceil_div(total_frames * 32, 256);
-  if (striped) rowcount_kernel<true><<<blocks, 256, 0, s>>>(d_bitmap, total_frames, d_row_count);
-  else rowcount_kernel<false><<<blocks, 256, 0, s>>>(d_bitmap, total_frames, d_row_count);
+  const PeakWindow w = win ? *win : PeakWindow{};
+  if (win) {
+    if (striped) rowcount_kernel<true, true><<<blocks, 256, 0, s>>>(d_bitmap, total_frames, d_row_count, w);
+    else rowcount_kernel<false, true><<<blocks, 256, 0, s>>>(d_bitmap, total_frames, d_row_count, w);
+  } else {
+    if (striped) rowcount_kernel<true, false><<<blocks, 256, 0, s>>>(d_bitmap, total_frames, d_row_count, w);
+    else rowcount_kernel<false, false><<<blocks, 256, 0, s>>>(d_bitmap, total_frames, d_row_count, w);
+  }
   SIA_CHECK_LAUNCH();
   return SIA_OK;
 }
@@ -587,15 +617,19 @@ int peaks_rowcount_launch(const uint32_t *d_bitmap, bool striped, int64_t total_
 int peaks_extract_launch(const uint32_t *d_bitmap, bool striped, const int64_t *d_row_off,
                          const int64_t *d_frame_starts, int n_tracks, int64_t total_frames, int64_t peak_base, int32_t *d_peak_t,
                          int32_t *d_peak_f, int64_t cap_peaks, int64_t *d_track_peak_starts, int32_t *d_status,
-                         cudaStream_t s) {
+                         cudaStream_t s, const PeakWindow *win) {
   if (total_frames == 0) return SIA_OK;
   const unsigned blocks = (unsigned)ceil_div(total_frames * 32, 256);
-  if (striped)
-    extract_kernel<true><<<blocks, 256, 0, s>>>(d_bitmap, d_row_off, d_frame_starts, n_tracks, total_frames, peak_base,
-                                                d_peak_t, d_peak_f, cap_peaks, d_track_peak_starts, d_status);
-  else
-    extract_kernel<false><<<blocks, 256, 0, s>>>(d_bitmap, d_row_off, d_frame_starts, n_tracks, total_frames, peak_base,
-                                                 d_peak_t, d_peak_f, cap_peaks, d_track_peak_starts, d_status);
+  const PeakWindow w = win ? *win : PeakWindow{};
+#define SIA_EXTRACT(ST, WN)                                                                                       \
+  extract_kernel<ST, WN><<<blocks, 256, 0, s>>>(d_bitmap, d_row_off, d_frame_starts, n_tracks, total_frames, peak_base, \
+                                                d_peak_t, d_peak_f, cap_peaks, d_track_peak_starts, d_status, w)
+  if (win) {
+    if (striped) SIA_EXTRACT(true, true); else SIA_EXTRACT(false, true);
+  } else {
+    if (striped) SIA_EXTRACT(true, false); else SIA_EXTRACT(false, false);
+  }
+#undef SIA_EXTRACT
   SIA_CHECK_LAUNCH();
   return SIA_OK;
 }

@@ -52,18 +52,30 @@ constexpr int kPeakTileF = 128;   // output bins per tile
 // *striped tells which bitmap layout was written (see peaks.cu)
 int peaks_bitmap_launch(const PeaksLaunch &a, cudaStream_t s, bool *striped);
 
+// Streaming (stream.cu): of segment b (rows [frame_starts[b], frame_starts[b+1])) only the segment-local rows
+// [emit_lo[b], emit_hi[b]) yield peaks, their t is t_base[b] + local row, and they are placed peak_off[b] entries after
+// their scan offset.  The caller then fills the segments' peak starts itself (track_peak_starts may be NULL).
+struct PeakWindow {
+  const int64_t *frame_starts;   // [n+1]
+  const int64_t *emit_lo, *emit_hi, *t_base, *peak_off;   // [n]
+  int n;
+};
+
 // bitmap -> ordered (t, f) lists.  d_row_count/d_row_off: [total_frames(+1)] workspaces.
 int peaks_rowcount_launch(const uint32_t *d_bitmap, bool striped, int64_t total_frames, uint32_t *d_row_count,
-                          cudaStream_t s);
+                          cudaStream_t s, const PeakWindow *win = nullptr);
 int peaks_extract_launch(const uint32_t *d_bitmap, bool striped, const int64_t *d_row_off,
                          const int64_t *d_frame_starts, int n_tracks, int64_t total_frames, int64_t peak_base, int32_t *d_peak_t,
                          int32_t *d_peak_f, int64_t cap_peaks, int64_t *d_track_peak_starts, int32_t *d_status,
-                         cudaStream_t s);
+                         cudaStream_t s, const PeakWindow *win = nullptr);
 
 // ---- K3 ------------------------------------------------------------------------------------
 // d_n_peaks: device scalar (total peaks, = track_peak_starts[n_tracks]); launches are sized by n_peaks_max.
+// d_final_t (streaming, [n_tracks]): anchors of track b with t > d_final_t[b] and fewer than fan_value-1 peaks behind
+// them in the track are not final yet and get no pairs; NULL = every anchor is final.
 int pairs_count_launch(const int32_t *d_peak_t, const int64_t *d_track_peak_starts, int n_tracks,
-                       int64_t n_peaks_max, int fan_value, uint32_t *d_pair_count, cudaStream_t s);
+                       int64_t n_peaks_max, int fan_value, uint32_t *d_pair_count, cudaStream_t s,
+                       const int64_t *d_final_t = nullptr);
 int pairs_sha1_launch(const int32_t *d_peak_t, const int32_t *d_peak_f, const int64_t *d_track_peak_starts,
                       int n_tracks, int64_t n_peaks_max, int fan_value, const uint32_t *d_pair_count,
                       const int64_t *d_pair_off, int64_t hash_base_static, const int64_t *d_hash_base,
