@@ -266,7 +266,25 @@ int sia_index_query_batch(sia_index *ix, const uint8_t *d_hash, const int32_t *d
                           int32_t *d_out_song, int32_t *d_out_diff, int32_t *d_out_count,
                           int32_t *d_out_rows, int32_t *d_out_nres, int64_t *h_stats, void *stream);
 
-/* device time (ms, CUDA events on the call's stream) of the last sia_index_query_batch: [0] pack + sort + lookup,
+/* The a-priori early exit of recognizer_apriori.py:246-310 for Q queries at once: each query's distinct hashes are
+ * read in batches of batch_hashes, and the query stops after the first batch at which the best song has more than
+ * twice the matched DB rows of the runner-up (recognizer_apriori.py:305, in integers: rows(s1) > 2 * rows(s2), at
+ * least two songs matched).  Batch k of a query is its distinct hashes [k*B, (k+1)*B) in ASCENDING DIGEST ORDER (the
+ * reference iterates a Python set, whose order Python does not define; sorted order makes the result independent
+ * of how the caller orders the pairs).  The state after batch k is the vote of sia_index_query_batch over the vote
+ * tuples and matched rows of batches 0..k only.  Inputs and the five outputs as sia_index_query_batch, taken at the
+ * exit batch (or after the last batch if the rule never fires), plus per query:
+ *   out_batches[q] — batches read (0 for an empty query),   out_exit[q] — 1 if the rule fired.
+ * The rule always looks at the top two, whatever topn.  batch_hashes >= 1, topn >= 1.
+ * h_stats (optional, 4 x int64): query (hash, offset) pairs, DB rows read up to each query's exit, vote tuples read
+ * up to each query's exit, batches read in all. */
+int sia_index_query_apriori(sia_index *ix, const uint8_t *d_hash, const int32_t *d_qoff, const int64_t *h_query_starts,
+                            int32_t n_queries, int32_t topn, int32_t batch_hashes,
+                            int32_t *d_out_song, int32_t *d_out_diff, int32_t *d_out_count, int32_t *d_out_rows,
+                            int32_t *d_out_nres, int32_t *d_out_batches, int32_t *d_out_exit,
+                            int64_t *h_stats, void *stream);
+
+/* device time (ms, CUDA events on the call's stream) of the last sia_index_query_batch or sia_index_query_apriori: [0] pack + sort + lookup,
  * [1] vote (all passes of the call) */
 int sia_index_query_timing(const sia_index *ix, double *h_ms2);
 

@@ -71,6 +71,8 @@ SIGNATURES = {
     "sia_index_export": (C.c_int, [_p, C.c_int64, C.c_int64, _p, _p, _p, _p]),
     "sia_index_select_host": (C.c_int, [_p, _p, C.c_int64, _p, _p, _p, C.c_int64, _i64p]),
     "sia_index_query_batch": (C.c_int, [_p, _p, _p, _i64p, C.c_int32, C.c_int32, _p, _p, _p, _p, _p, _i64p, _p]),
+    "sia_index_query_apriori": (C.c_int, [_p, _p, _p, _i64p, C.c_int32, C.c_int32, C.c_int32, _p, _p, _p, _p, _p, _p, _p,
+                                          _i64p, _p]),
     "sia_index_query_timing": (C.c_int, [_p, C.POINTER(C.c_double)]),
     "sia_index_trim": (C.c_int, [_p]),
     "sia_index_keys": (C.c_int64, [_p]),

@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "_lib")
 LIB = os.path.join(LIBDIR, "libsia_b200.so")
-SOURCES = ["api.cu", "scan.cu", "stft.cu", "peaks.cu", "pairs_sha1.cu", "sort.cu", "index_store.cu", "index_query.cu", "index_pvote.cu", "index_dist.cu", "noise.cu",
+SOURCES = ["api.cu", "scan.cu", "stft.cu", "peaks.cu", "pairs_sha1.cu", "sort.cu", "index_store.cu", "index_query.cu", "index_apriori.cu", "index_pvote.cu", "index_dist.cu", "noise.cu",
            "stream.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-O3"]

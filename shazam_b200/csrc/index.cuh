@@ -157,6 +157,108 @@ __device__ __forceinline__ const uint64_t *slot_keys(const uint64_t *__restrict_
   return base + 1;
 }
 
+// ---- the table vote's per-query HBM tables (index_query.cu), shared with the a-priori rounds (index_apriori.cu) ----------
+namespace tvote {
+
+constexpr int kQidBits = SIA_KEY_QID_BITS, kSongBits = SIA_KEY_SONG_BITS, kDiffBits = SIA_KEY_DIFF_BITS;
+constexpr int64_t kMaxQueriesPerPass = 1ll << kQidBits;
+constexpr uint64_t kDiffMask = (1ull << kDiffBits) - 1;
+constexpr int kTopK = 4;                  // results extracted per scan of a query's song table
+
+struct QMeta {
+  int64_t bin_base, song_base, filt_base;   // first slot / word of the query's sub-tables inside the group's tables
+  int64_t cand_base;                        // first entry of the query's candidate list
+  uint32_t bin_cap, song_cap, filt_words, cand;   // cand: tuples in twice-hit buckets (pass 1), sizes the bin table
+  uint32_t cursor, pad_;                    // candidates collected so far (pass 2)
+};
+
+struct Tables {
+  unsigned long long *bins;       // [nb] key words ((song << 25 | biased diff) + 1; 0 = empty)
+  uint32_t *bin_cnt;              // [nb]
+  unsigned long long *song_best;  // [ns]
+  uint32_t *song_key;             // [ns] open addressing only (song + 1)
+  uint32_t *filter;               // [nf]
+  unsigned long long *cand;       // [nb / 2] candidate vote keys (query | song | biased diff), per-query lists
+};
+
+// queries [qa, qb) of a pass as one group: sub-table layout of its queries in h_meta (filter words = tuples + 1, song
+// slots dense = span or open addressing = 2 * head rows + 32) from the scanned tuple / head-row offsets at the queries'
+// first entries
+struct Group { int qa, qb; bool dense; int64_t nf, ns; };
+Group make_group(int qa, int qb, const int64_t *h_off_all, const int64_t *h_off_head, int64_t span, QMeta *h_meta);
+
+// vote tuples per group of queries: SIA_VOTE_GROUP_TUPLES (default 2^29), bounded by what the device has left
+int group_tuple_budget(::sia_index *ix, int64_t &budget);
+
+__device__ __forceinline__ uint32_t mix32(uint32_t k) {
+  k ^= k >> 16; k *= 0x85ebca6bu; k ^= k >> 13; k *= 0xc2b2ae35u; k ^= k >> 16;
+  return k;
+}
+__device__ __forceinline__ uint32_t slot_of(uint32_t h, uint32_t cap) { return (uint32_t)(((uint64_t)h * cap) >> 32); }
+
+// song slot of `song` in query m's song table (dense: the id itself; else find-or-insert by open addressing)
+template <bool DENSE>
+__device__ __forceinline__ int64_t song_slot(const QMeta &m, uint32_t song, uint32_t *__restrict__ song_key) {
+  if (DENSE) return song < m.song_cap ? m.song_base + song : -1;
+  uint32_t t = slot_of(mix32(song), m.song_cap);
+  for (uint32_t probes = 0; probes < m.song_cap; ++probes) {     // bounded: a full table (inconsistent inputs) cannot hang
+    const uint32_t old = atomicCAS(&song_key[m.song_base + t], 0u, song + 1u);
+    if (old == 0u || old == song + 1u) return m.song_base + t;
+    if (++t == m.song_cap) t = 0;
+  }
+  return -1;
+}
+
+// count one vote tuple (song, biased diff) in query m's bin table; returns the bin's count including this tuple
+// (0 and flag 8 if the table is full, which the sizing rules out)
+__device__ __forceinline__ unsigned long long bin_count(const QMeta &m, uint32_t song, uint32_t dbits, const Tables &T,
+                                                        uint32_t &fresh, int32_t *__restrict__ flags) {
+  const unsigned long long key = (((unsigned long long)song << kDiffBits) | dbits) + 1ull;     // never 0
+  uint32_t s = slot_of(mix32(song * 0x9e3779b1u + dbits), m.bin_cap);
+  for (uint32_t probes = 0; probes < m.bin_cap; ++probes) {
+    const int64_t at = m.bin_base + s;
+    const unsigned long long old = atomicCAS(T.bins + at, 0ull, key);
+    if (old == 0ull) ++fresh;
+    if (old == 0ull || old == key) return (unsigned long long)atomicAdd(T.bin_cnt + at, 1u) + 1ull;
+    if (++s == m.bin_cap) s = 0;
+  }
+  atomicOr(flags, 8);
+  return 0;
+}
+
+// song best key: count (high) | inverted biased diff, so the largest key is the largest count with the smallest
+// difference (Python's max() keeps the first maximum, recognizer.py:308)
+__device__ __forceinline__ unsigned long long best_key(unsigned long long count, uint32_t dbits) {
+  return (count << kDiffBits) | (kDiffMask - dbits);
+}
+
+// raise a song's best to at least `val`; true if this call raised it.  Best only grows, so a (possibly stale) read
+// that already covers the value makes the atomic unnecessary.
+__device__ __forceinline__ bool best_raise(unsigned long long *best, unsigned long long val) {
+  return __ldcg(best) < val && atomicMax(best, val) < val;
+}
+
+// keep the song's best (count, smallest diff) current
+template <bool DENSE>
+__device__ __forceinline__ void song_update(const QMeta &m, uint32_t song, uint32_t dbits, unsigned long long count,
+                                            const Tables &T, int32_t *__restrict__ flags) {
+  const int64_t ss = song_slot<DENSE>(m, song, T.song_key);
+  if (ss < 0) { atomicOr(flags, 8); return; }
+  best_raise(&T.song_best[ss], best_key(count, dbits));
+}
+
+}  // namespace tvote
+
+// ---- one pass of queries through the lookup (index_query.cu) --------------------------------------------------
+// pack the pairs [h_query_starts[0], h_query_starts[nq]) of nq queries (d_qs: the same starts on the device) into
+// ea (alt buffer eb), sort and look them up (lookup_sorted), check the offsets / ids.
+int lookup_queries(::sia_index *ix, const uint8_t *d_hash, const int32_t *d_qoff, const int64_t *h_query_starts,
+                   const int64_t *d_qs, int nq, ulonglong2 *ea, ulonglong2 *eb, Lookup &L, cudaStream_t s);
+// scanned tuple / head-row offsets at the queries' first entries: h_goff[0..nq] = off_all, h_goff[nq+1..] = off_head
+// (d_goff: 2 * (nq + 1) device scratch).  Synchronises the stream.
+int query_offsets(const Lookup &L, const int64_t *d_qs, int64_t i0, int nq, int64_t *d_goff, std::vector<int64_t> &h_goff,
+                  cudaStream_t s);
+
 // ---- partitioned vote (index_pvote.cu) ------------------------------------------------------------------------
 // The vote tuples of every query are split by a hash of the SONG into partitions small enough for an exact hash table
 // in shared memory: one scatter pass (posting runs / received vote keys -> per-(query, partition) regions, staged and

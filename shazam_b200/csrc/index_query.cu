@@ -29,31 +29,12 @@
 #include <cstring>
 
 using namespace sia;
+using namespace sia::tvote;
 
 namespace {
 
-constexpr int kQidBits = SIA_KEY_QID_BITS, kSongBits = SIA_KEY_SONG_BITS, kDiffBits = SIA_KEY_DIFF_BITS;
-constexpr int64_t kMaxQueriesPerPass = 1ll << kQidBits;
-constexpr uint64_t kDiffMask = (1ull << kDiffBits) - 1;
-constexpr int kTopK = 4;                  // results extracted per scan of a query's song table
 constexpr int kVoteTuples = 4096;         // vote tuples per block of the entry-walking kernels (512 per warp): the tuples
                                           // in flight on the whole GPU then belong to 2-3 queries, whose filters stay in L2
-
-struct QMeta {
-  int64_t bin_base, song_base, filt_base;   // first slot / word of the query's sub-tables inside the group's tables
-  int64_t cand_base;                        // first entry of the query's candidate list
-  uint32_t bin_cap, song_cap, filt_words, cand;   // cand: tuples in twice-hit buckets (pass 1), sizes the bin table
-  uint32_t cursor, pad_;                    // candidates collected so far (pass 2)
-};
-
-struct Tables {
-  unsigned long long *bins;       // [nb] key words ((song << 25 | biased diff) + 1; 0 = empty)
-  uint32_t *bin_cnt;              // [nb]
-  unsigned long long *song_best;  // [ns]
-  uint32_t *song_key;             // [ns] open addressing only (song + 1)
-  uint32_t *filter;               // [nf]
-  unsigned long long *cand;       // [nb / 2] candidate vote keys (query | song | biased diff), per-query lists
-};
 
 // ---- lookup ---------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
@@ -162,54 +143,6 @@ __global__ void gather_offsets_kernel(const int64_t *__restrict__ off_all, const
     out[q] = off_all[e];
     out[nq + 1 + q] = off_head[e];
   }
-}
-
-// ---- vote tables ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t mix32(uint32_t k) {
-  k ^= k >> 16; k *= 0x85ebca6bu; k ^= k >> 13; k *= 0xc2b2ae35u; k ^= k >> 16;
-  return k;
-}
-__device__ __forceinline__ uint32_t slot_of(uint32_t h, uint32_t cap) { return (uint32_t)(((uint64_t)h * cap) >> 32); }
-
-// song slot of `song` in query m's song table (dense: the id itself; else find-or-insert by open addressing)
-template <bool DENSE>
-__device__ __forceinline__ int64_t song_slot(const QMeta &m, uint32_t song, uint32_t *__restrict__ song_key) {
-  if (DENSE) return song < m.song_cap ? m.song_base + song : -1;
-  uint32_t t = slot_of(mix32(song), m.song_cap);
-  for (uint32_t probes = 0; probes < m.song_cap; ++probes) {     // bounded: a full table (inconsistent inputs) cannot hang
-    const uint32_t old = atomicCAS(&song_key[m.song_base + t], 0u, song + 1u);
-    if (old == 0u || old == song + 1u) return m.song_base + t;
-    if (++t == m.song_cap) t = 0;
-  }
-  return -1;
-}
-
-// count one vote tuple (song, biased diff) in query m's bin table; returns the bin's count including this tuple
-// (0 and flag 8 if the table is full, which the sizing rules out)
-__device__ __forceinline__ unsigned long long bin_count(const QMeta &m, uint32_t song, uint32_t dbits, const Tables &T,
-                                                        uint32_t &fresh, int32_t *__restrict__ flags) {
-  const unsigned long long key = (((unsigned long long)song << kDiffBits) | dbits) + 1ull;     // never 0
-  uint32_t s = slot_of(mix32(song * 0x9e3779b1u + dbits), m.bin_cap);
-  for (uint32_t probes = 0; probes < m.bin_cap; ++probes) {
-    const int64_t at = m.bin_base + s;
-    const unsigned long long old = atomicCAS(T.bins + at, 0ull, key);
-    if (old == 0ull) ++fresh;
-    if (old == 0ull || old == key) return (unsigned long long)atomicAdd(T.bin_cnt + at, 1u) + 1ull;
-    if (++s == m.bin_cap) s = 0;
-  }
-  atomicOr(flags, 8);
-  return 0;
-}
-
-// keep the song's best (count, smallest diff) current: best only grows, so a (possibly stale) read that already
-// covers the value makes the atomic unnecessary
-template <bool DENSE>
-__device__ __forceinline__ void song_update(const QMeta &m, uint32_t song, uint32_t dbits, unsigned long long count,
-                                            const Tables &T, int32_t *__restrict__ flags) {
-  const int64_t ss = song_slot<DENSE>(m, song, T.song_key);
-  if (ss < 0) { atomicOr(flags, 8); return; }
-  const unsigned long long val = (count << kDiffBits) | (kDiffMask - dbits);
-  if (__ldcg(&T.song_best[ss]) < val) atomicMax(&T.song_best[ss], val);
 }
 
 // duplicate filter: 2 bits per bucket (seen, seen twice), 16 buckets per 32-bit word, ~16 buckets per tuple
@@ -1005,6 +938,58 @@ int vote_scratch_finish_and_reserve(int device, size_t bytes) {
   return g_vote_tables[device].reserve(bytes);
 }
 
+namespace tvote {
+
+Group make_group(int qa, int qb, const int64_t *h_off_all, const int64_t *h_off_head, int64_t span, QMeta *h_meta) {
+  Group g{qa, qb, false, 0, 0};
+  const int64_t h_all = h_off_head[qb] - h_off_head[qa];
+  const int64_t ns_hashed = 2 * h_all + 32ll * (qb - qa);
+  g.dense = span * (qb - qa) * 8 <= ns_hashed * 12 * 2;
+  int64_t fb = 0, sb = 0;
+  for (int q = qa; q < qb; ++q) {
+    const int64_t t = h_off_all[q + 1] - h_off_all[q], h = h_off_head[q + 1] - h_off_head[q];
+    QMeta &m = h_meta[q];
+    m.bin_base = 0; m.bin_cap = 0; m.cand = 0; m.cand_base = 0; m.cursor = 0; m.pad_ = 0;
+    m.filt_base = fb; m.filt_words = (uint32_t)(t + 1);
+    m.song_base = sb; m.song_cap = g.dense ? (uint32_t)span : (uint32_t)(2 * h + 32);
+    fb += m.filt_words; sb += m.song_cap;
+  }
+  g.nf = fb; g.ns = sb;
+  return g;
+}
+
+int group_tuple_budget(::sia_index *ix, int64_t &budget) {
+  budget = getenv("SIA_VOTE_GROUP_TUPLES") ? std::max(1ll, atoll(getenv("SIA_VOTE_GROUP_TUPLES"))) : (512ll << 20);
+  size_t free_b = 0, total_b = 0;
+  SIA_CUDA(cudaMemGetInfo(&free_b, &total_b));
+  budget = std::max<int64_t>(1 << 20, std::min<int64_t>(budget, (int64_t)((free_b + ix->arena3.cap) * 0.6 / 40)));
+  return SIA_OK;
+}
+
+}  // namespace tvote
+
+int lookup_queries(::sia_index *ix, const uint8_t *d_hash, const int32_t *d_qoff, const int64_t *h_query_starts,
+                   const int64_t *d_qs, int nq, ulonglong2 *ea, ulonglong2 *eb, Lookup &L, cudaStream_t s) {
+  const int64_t i0 = h_query_starts[0], n = h_query_starts[nq] - i0;
+  int64_t max_entries = 0;
+  for (int q = 0; q < nq; ++q) max_entries = std::max(max_entries, h_query_starts[q + 1] - h_query_starts[q]);
+  pack_queries_kernel<<<grid_for(n), 256, 0, s>>>(d_hash, d_qoff, nullptr, d_qs, nq, i0, n, ea, ix->status);
+  SIA_CHECK_LAUNCH();
+  int rc = lookup_sorted(ix, ix->arena, ea, eb, n, d_qs, i0, nq, max_entries, L, s);
+  if (rc) return rc;
+  return check_status(ix, s, 2 | 4, "query: offset outside 0..2^24-1 (or a posting run of 2^32 rows)");
+}
+
+int query_offsets(const Lookup &L, const int64_t *d_qs, int64_t i0, int nq, int64_t *d_goff, std::vector<int64_t> &h_goff,
+                  cudaStream_t s) {
+  h_goff.assign(2 * (size_t)(nq + 1), 0);
+  gather_offsets_kernel<<<grid_for(nq + 1), 256, 0, s>>>(L.off_all, L.off_head, d_qs, i0, nq, d_goff);
+  SIA_CHECK_LAUNCH();
+  SIA_CUDA(cudaMemcpyAsync(h_goff.data(), d_goff, h_goff.size() * 8, cudaMemcpyDeviceToHost, s));
+  SIA_CUDA(cudaStreamSynchronize(s));
+  return SIA_OK;
+}
+
 }  // namespace sia
 
 extern "C" {
@@ -1071,13 +1056,9 @@ int sia_index_query_batch(sia_index *ix, const uint8_t *d_hash, const int32_t *d
   for (int32_t *o : {d_out_song, d_out_diff, d_out_count, d_out_rows})
     SIA_CUDA(cudaMemsetAsync(o, 0, sizeof(int32_t) * (size_t)n_queries * topn, s));
 
-  // vote tuples per group of queries (one set of launches per group): bounded by what the device has left
-  int64_t tuple_budget = getenv("SIA_VOTE_GROUP_TUPLES") ? std::max(1ll, atoll(getenv("SIA_VOTE_GROUP_TUPLES"))) : (512ll << 20);
-  {
-    size_t free_b = 0, total_b = 0;
-    SIA_CUDA(cudaMemGetInfo(&free_b, &total_b));
-    tuple_budget = std::max<int64_t>(1 << 20, std::min<int64_t>(tuple_budget, (int64_t)((free_b + ix->arena3.cap) * 0.6 / 40)));
-  }
+  // vote tuples per group of queries (one set of launches per group)
+  int64_t tuple_budget = 0;
+  if ((rc = group_tuple_budget(ix, tuple_budget))) return rc;
   const bool timing = getenv("SIA_QUERY_TIMING") != nullptr;       // stage times of every pass on stderr
   const char *vote_env = getenv("SIA_VOTE");                       // "tables": the table vote for every query (A/B tests)
   const bool use_pvote = topn <= kPvMaxTopn && !(vote_env && !strcmp(vote_env, "tables"));
@@ -1099,43 +1080,17 @@ int sia_index_query_batch(sia_index *ix, const uint8_t *d_hash, const int32_t *d
     SIA_CUDA(cudaMemcpyAsync(d_qs, h_query_starts + q0, sizeof(int64_t) * (nq + 1), cudaMemcpyHostToDevice, s));
     const auto h0 = std::chrono::steady_clock::now();
     SIA_CUDA(cudaEventRecord(ix->ev_q[0], s));
-    int64_t max_entries = 0;
-    for (int q = 0; q < nq; ++q) max_entries = std::max(max_entries, h_query_starts[q0 + q + 1] - h_query_starts[q0 + q]);
-    pack_queries_kernel<<<grid_for(n), 256, 0, s>>>(d_hash, d_qoff, nullptr, d_qs, nq, i0, n, ea, ix->status);
-    SIA_CHECK_LAUNCH();
     Lookup L;
-    if ((rc = lookup_sorted(ix, ix->arena, ea, eb, n, d_qs, i0, nq, max_entries, L, s))) return rc;
-    if ((rc = check_status(ix, s, 2 | 4, "query: offset outside 0..2^24-1 (or a posting run of 2^32 rows)"))) return rc;
+    if ((rc = lookup_queries(ix, d_hash, d_qoff, h_query_starts + q0, d_qs, nq, ea, eb, L, s))) return rc;
     SIA_CUDA(cudaEventRecord(ix->ev_q[1], s));
     if (h_stats) { h_stats[1] += L.head_rows; h_stats[2] += L.tuples; }
     // After the sort query q still owns entries [starts[q]-i0, starts[q+1]-i0) (duplicates stay, with no
     // postings), so the scanned offsets at those positions split the pass into groups that fit the budget.
-    std::vector<int64_t> h_goff(2 * (size_t)(nq + 1));
-    gather_offsets_kernel<<<grid_for(nq + 1), 256, 0, s>>>(L.off_all, L.off_head, d_qs, i0, nq, d_goff);
-    SIA_CHECK_LAUNCH();
-    SIA_CUDA(cudaMemcpyAsync(h_goff.data(), d_goff, h_goff.size() * 8, cudaMemcpyDeviceToHost, s));
-    SIA_CUDA(cudaStreamSynchronize(s));
+    std::vector<int64_t> h_goff;
+    if ((rc = query_offsets(L, d_qs, i0, nq, d_goff, h_goff, s))) return rc;
     const int64_t *h_off_all = h_goff.data(), *h_off_head = h_goff.data() + nq + 1;
-    struct Group { int qa, qb; bool dense; int64_t nf, ns; };
     std::vector<QMeta> h_meta(nq);
-    // queries [qa, qb) as one group of the table vote: sub-table layout of its queries
-    auto make_group = [&](int qa, int qb) {
-      Group g{qa, qb, false, 0, 0};
-      const int64_t h_all = h_off_head[qb] - h_off_head[qa];
-      const int64_t ns_hashed = 2 * h_all + 32ll * (qb - qa);
-      g.dense = span * (qb - qa) * 8 <= ns_hashed * 12 * 2;
-      int64_t fb = 0, sb = 0;
-      for (int q = qa; q < qb; ++q) {
-        const int64_t t = h_off_all[q + 1] - h_off_all[q], h = h_off_head[q + 1] - h_off_head[q];
-        QMeta &m = h_meta[q];
-        m.bin_base = 0; m.bin_cap = 0; m.cand = 0; m.cand_base = 0; m.cursor = 0; m.pad_ = 0;
-        m.filt_base = fb; m.filt_words = (uint32_t)(t + 1);
-        m.song_base = sb; m.song_cap = g.dense ? (uint32_t)span : (uint32_t)(2 * h + 32);
-        fb += m.filt_words; sb += m.song_cap;
-      }
-      g.nf = fb; g.ns = sb;
-      return g;
-    };
+    auto make_group = [&](int qa, int qb) { return tvote::make_group(qa, qb, h_off_all, h_off_head, span, h_meta.data()); };
     for (int q = 0; q < nq; ++q)
       SIA_REQUIRE(h_off_all[q + 1] - h_off_all[q] < (1ll << 31), SIA_E_UNSUPPORTED, "query_batch: more than 2^31 vote tuples in one query");
     std::vector<Group> groups;               // what the table vote has to do

@@ -192,6 +192,29 @@ class FingerprintIndex:
             return (*outs, nres, list(stats))
         return (*outs, nres)
 
+    def query_batch_apriori(self, digests: torch.Tensor, qoffsets: torch.Tensor, query_starts: np.ndarray, topn: int,
+                            batch_hashes: int = 1000, want_stats: bool = False):
+        """The a-priori early exit of ``recognizer_apriori.py:246-310`` for Q queries: each query's distinct hashes are
+        read in batches of ``batch_hashes`` in ascending digest order, and the query stops once its best song has more
+        than twice the matched DB rows of the runner-up.  Returns the five tensors of ``query_batch`` at that point,
+        plus ``batches[Q]`` (batches read) and ``exit[Q]`` (1 if the rule fired) (+ stats: query pairs, DB rows read,
+        vote tuples read, batches read)."""
+        self.finalize()
+        qs = np.ascontiguousarray(query_starts, np.int64)
+        Q = len(qs) - 1
+        d = digests.contiguous()
+        o = qoffsets.to(torch.int32).contiguous()
+        assert d.is_cuda and o.is_cuda and d.dtype == torch.uint8
+        outs = [torch.zeros((Q, topn), dtype=torch.int32, device=self.tdev) for _ in range(4)]
+        per_q = [torch.zeros(Q, dtype=torch.int32, device=self.tdev) for _ in range(3)]      # nres, batches, exit
+        stats = (C.c_int64 * 4)()
+        N.check(self.lib.sia_index_query_apriori(self._h, C.c_void_p(d.data_ptr()), C.c_void_p(o.data_ptr()),
+                                                 qs.ctypes.data_as(C.POINTER(C.c_int64)), Q, int(topn), int(batch_hashes),
+                                                 *[C.c_void_p(t.data_ptr()) for t in outs + per_q], stats, self._stream()))
+        if want_stats:
+            return (*outs, *per_q, list(stats))
+        return (*outs, *per_q)
+
     def trim(self) -> None:
         """Release build / lookup / vote scratch (re-allocated on demand); the table stays."""
         self.finalize()

@@ -51,7 +51,8 @@ def return_matches(hashes, batch_size: int = 1000, apriori: bool = False):
     ``batch_size`` distinct hashes the matches so far are aligned, and the lookup stops as soon as the best song has
     more than twice the matched hashes of the runner-up.  It changes ``hashes_matched`` (fewer batches are read), so
     it is off by default and outside the parity tests; the return value then has the reference's third element,
-    the aligned results at the point of exit (``[]`` if the exit never triggered)."""
+    the aligned results at the point of exit (``[]`` if the exit never triggered).  This is the tuple-returning
+    drop-in; ``recognize_batch(..., apriori_batch=batch_size)`` runs the same rule on the device for many queries."""
     mapper = {}
     for hsh, offset in hashes:
         mapper.setdefault(hsh.upper(), []).append(offset)
@@ -120,10 +121,15 @@ def align_matches(matches, dedup_hashes, queried_hashes, topn: int = TOPN):
     return [_result_dict(s, d, dedup_hashes[s], queried_hashes) for s, d in zip(song, dif)]
 
 
-def recognize_batch(queries: Sequence, topn: int = TOPN, want_stats: bool = False):
+def recognize_batch(queries: Sequence, topn: int = TOPN, want_stats: bool = False, apriori_batch: Optional[int] = None):
     """Array fast path for many queries at once.  ``queries[i]`` is ``(digests uint8[n,10],
     offsets int32[n])`` (host arrays or CUDA tensors).  Returns, per query, the list of result
-    dicts ``align_matches`` would return for ``len(set(pairs))`` queried hashes."""
+    dicts ``align_matches`` would return for ``len(set(pairs))`` queried hashes.
+
+    ``apriori_batch=B`` applies the early exit of ``recognizer_apriori.py:246-310`` on the device
+    (``FingerprintIndex.query_batch_apriori``): the distinct hashes are read in batches of B in ascending digest
+    order, and a query's results are those at the batch where its best song first had more than twice the matched
+    rows of the runner-up (``hashes_matched_in_input`` = rows read up to then), else those of the whole query."""
     index = db.index
     dig, off, starts, nq_hashes = [], [], [0], []
     for d, o in queries:
@@ -135,7 +141,10 @@ def recognize_batch(queries: Sequence, topn: int = TOPN, want_stats: bool = Fals
         return []
     D = torch.cat(dig) if dig else torch.empty((0, N.HASH_BYTES), dtype=torch.uint8, device=index.tdev)
     O = torch.cat(off)
-    out = index.query_batch(D, O, np.array(starts, np.int64), topn, want_stats=want_stats)
+    if apriori_batch is None:
+        out = index.query_batch(D, O, np.array(starts, np.int64), topn, want_stats=want_stats)
+    else:
+        out = index.query_batch_apriori(D, O, np.array(starts, np.int64), topn, apriori_batch, want_stats=want_stats)
     song, dif, cnt, rows, nres = [t.cpu().numpy() for t in out[:5]]
     results = []
     for q in range(len(queries)):
@@ -148,7 +157,7 @@ def recognize_batch(queries: Sequence, topn: int = TOPN, want_stats: bool = Fals
             nq = 0
         results.append([_result_dict(int(song[q, r]), int(dif[q, r]), int(rows[q, r]), nq) for r in range(int(nres[q]))])
     if want_stats:
-        return results, out[5]
+        return results, out[-1]
     return results
 
 
