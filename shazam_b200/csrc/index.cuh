@@ -20,7 +20,9 @@
 
 #include <algorithm>
 #include <cstdlib>
+#include <functional>
 #include <string>
+#include <utility>
 #include <vector>
 
 namespace sia {
@@ -187,8 +189,9 @@ struct Tables {
 struct Group { int qa, qb; bool dense; int64_t nf, ns; };
 Group make_group(int qa, int qb, const int64_t *h_off_all, const int64_t *h_off_head, int64_t span, QMeta *h_meta);
 
-// vote tuples per group of queries: SIA_VOTE_GROUP_TUPLES (default 2^29), bounded by what the device has left
-int group_tuple_budget(::sia_index *ix, int64_t &budget);
+// the groups [qa, qb) of consecutive queries q of a pass with keep[q] != 0 (keep NULL: every query), each within
+// `budget` vote tuples or a single query; groups without tuples are left out
+std::vector<std::pair<int, int>> split_groups(const int64_t *h_off_all, int nq, int64_t budget, const uint32_t *keep);
 
 __device__ __forceinline__ uint32_t mix32(uint32_t k) {
   k ^= k >> 16; k *= 0x85ebca6bu; k ^= k >> 13; k *= 0xc2b2ae35u; k ^= k >> 16;
@@ -249,15 +252,51 @@ __device__ __forceinline__ void song_update(const QMeta &m, uint32_t song, uint3
 
 }  // namespace tvote
 
-// ---- one pass of queries through the lookup (index_query.cu) --------------------------------------------------
-// pack the pairs [h_query_starts[0], h_query_starts[nq]) of nq queries (d_qs: the same starts on the device) into
-// ea (alt buffer eb), sort and look them up (lookup_sorted), check the offsets / ids.
-int lookup_queries(::sia_index *ix, const uint8_t *d_hash, const int32_t *d_qoff, const int64_t *h_query_starts,
-                   const int64_t *d_qs, int nq, ulonglong2 *ea, ulonglong2 *eb, Lookup &L, cudaStream_t s);
-// scanned tuple / head-row offsets at the queries' first entries: h_goff[0..nq] = off_all, h_goff[nq+1..] = off_head
-// (d_goff: 2 * (nq + 1) device scratch).  Synchronises the stream.
-int query_offsets(const Lookup &L, const int64_t *d_qs, int64_t i0, int nq, int64_t *d_goff, std::vector<int64_t> &h_goff,
-                  cudaStream_t s);
+// SIA_QUERY_TIMING: events between the stages of a vote, created on first use (on the current device).  mark() does
+// nothing unless `on`; ms(a, b) waits for mark b.
+struct StageEvents {
+  bool on = false;
+  cudaEvent_t ev[9] = {};
+  void mark(int k, cudaStream_t s) {
+    if (!on) return;
+    if (!ev[k]) cudaEventCreate(&ev[k]);
+    cudaEventRecord(ev[k], s);
+  }
+  float ms(int a, int b) {
+    float t = 0;
+    cudaEventSynchronize(ev[b]);
+    cudaEventElapsedTime(&t, ev[a], ev[b]);
+    return t;
+  }
+  void release() { for (auto &e : ev) if (e) { cudaEventDestroy(e); e = nullptr; } }
+};
+
+// ---- the passes of a query call (index_query.cu) -----------------------------------------------------------------
+// outputs of a query call: [n_queries][topn] song / diff / count / rows, [n_queries] result counts and, a-priori only,
+// batches read and exit flags
+struct PvOut { int32_t *song, *diff, *count, *rows, *nres; };
+struct QueryOut : PvOut { int32_t *batches, *exit; };
+
+// one pass of up to kMaxQueriesPerPass queries [q0, q0 + nq), looked up: what its vote step gets
+struct QueryPass {
+  Lookup L;                                  // entries [i0, i0 + n) of the pass's pairs, sorted, with their runs
+  int64_t q0 = 0, i0 = 0, n = 0;
+  int nq = 0;
+  const int64_t *h_qs = nullptr, *d_qs = nullptr;   // entry offsets of the pass's queries (absolute) [nq + 1]
+  // scanned tuple / head-row offsets at the queries' first entries [nq + 1]; d_goff: both on the device, one after the other
+  const int64_t *h_off_all = nullptr, *h_off_head = nullptr, *d_goff = nullptr;
+  int64_t budget = 0;                        // vote tuples per group of queries
+  cudaStream_t s = nullptr;
+  size_t groups = 0;                         // set by the vote step: table-vote groups, for the SIA_QUERY_TIMING line
+};
+
+// The frame of sia_index_query_batch and sia_index_query_apriori: argument checks, zeroed outputs, then per pass the
+// lookup (scratch in ix->arena, extra_bytes(nq, n) more of it left for the vote step), the tuple offsets, vote(pass)
+// and the lookup / vote times (ix->last_lookup_ms, last_vote_ms; with `timing` one line per pass on stderr).  Fills
+// h_stats[0] (query pairs); the vote step fills h_stats[1..3].
+int query_passes(::sia_index *ix, const uint8_t *d_hash, const int32_t *d_qoff, const int64_t *h_query_starts,
+                 int32_t n_queries, int32_t topn, const QueryOut &out, int64_t *h_stats, cudaStream_t s, bool timing,
+                 size_t (*extra_bytes)(int nq, int64_t n), const std::function<int(QueryPass &)> &vote);
 
 // ---- partitioned vote (index_pvote.cu) ------------------------------------------------------------------------
 // The vote tuples of every query are split by a hash of the SONG into partitions small enough for an exact hash table
@@ -268,7 +307,6 @@ int query_offsets(const Lookup &L, const int64_t *d_qs, int64_t i0, int nq, int6
 // not fit (a song with > 16384 tuples, > 512 * 16384 tuples, thousands of tied bins in one partition) are flagged in d_qover and left to the table vote.
 constexpr int kPvMaxTopn = 32;
 constexpr int kPvMaxPeers = 16;
-struct PvOut { int32_t *song, *diff, *count, *rows, *nres; };
 // scratch bytes for `tuples` vote tuples of nq queries arriving from n_src sources (worst case)
 size_t pvote_bytes(int64_t tuples, int64_t nq, int n_src, int topn);
 // per entry of a lookup what the scatter walk reads (once per pass): d_info[L.n] (16 B each), d_qh[L.n]
@@ -279,7 +317,7 @@ int pvote_entries(Arena &ar, const Lookup &L, const longlong2 *d_info, const uin
                   int64_t i0, const int64_t *d_goff, const int64_t *h_goff, int qa, int qb, int qid_base, int topn, const PvOut &out,
                   uint32_t *d_qover, uint32_t *d_qbins /* [nq_pass], zeroed: distinct bins per query */,
                   unsigned long long *d_nbins /* NULL, or += the bins of the settled queries */, cudaStream_t s,
-                  double *stage_ms /* NULL, or += {layout, scatter, count + merge} */);
+                  StageEvents &tm /* marks 0..3 around layout, scatter, count + merge */);
 // slotted vote keys, each slot sorted by query id (else d_flags2[0] is set and the outputs are garbage); rows counted from the regions.
 // d_over_count: incremented once per flagged query.
 // hash-prefix sharding over peer memory (index_dist.cu: sia_index_scatter_peers / sia_vote_count_regions)
@@ -318,6 +356,7 @@ struct sia_index {
   sia::Arena arena;                 // build / lookup scratch
   sia::Arena arena3;                // vote tables
   cudaEvent_t ev_q[3] = {nullptr, nullptr, nullptr};   // start / after lookup / end of a query pass
+  sia::StageEvents ev_stage;        // SIA_QUERY_TIMING: between the stages of the vote
   double last_lookup_ms = 0, last_vote_ms = 0;          // device time of the last sia_index_query_batch call
   // hash-prefix sharding over peer memory: the lookup of the pass in flight (lives in `arena` until the next reserve)
   sia::Lookup dist_L;

@@ -243,70 +243,37 @@ extern "C" int sia_index_query_apriori(sia_index *ix, const uint8_t *d_hash, con
               "n_queries >= 0, topn >= 1 and batch_hashes >= 1 required");
   SIA_REQUIRE(n_queries == 0 || (d_out_song && d_out_diff && d_out_count && d_out_rows && d_out_nres && d_out_batches &&
                                  d_out_exit), SIA_E_INVALID, "NULL output");
-  SIA_REQUIRE(ix && h_query_starts, SIA_E_INVALID, "NULL argument");
-  SIA_REQUIRE(ix->n_pending == 0, SIA_E_INVALID, "index has pending rows: call sia_index_finalize first");
-  if (h_stats) h_stats[0] = h_stats[1] = h_stats[2] = h_stats[3] = 0;
-  if (n_queries == 0) return SIA_OK;
-  SIA_CUDA(cudaSetDevice(ix->device));
-  cudaStream_t s = (cudaStream_t)stream;
-  for (int q = 0; q < n_queries; ++q)
-    SIA_REQUIRE(h_query_starts[q] <= h_query_starts[q + 1], SIA_E_INVALID, "query_starts must be non-decreasing");
-  SIA_REQUIRE(h_query_starts[n_queries] == h_query_starts[0] || (d_hash && d_qoff), SIA_E_INVALID, "NULL input");
-  for (int32_t *o : {d_out_nres, d_out_batches, d_out_exit}) SIA_CUDA(cudaMemsetAsync(o, 0, sizeof(int32_t) * n_queries, s));
-  for (int32_t *o : {d_out_song, d_out_diff, d_out_count, d_out_rows})
-    SIA_CUDA(cudaMemsetAsync(o, 0, sizeof(int32_t) * (size_t)n_queries * topn, s));
-  int64_t tuple_budget = 0;
-  int rc = group_tuple_budget(ix, tuple_budget);
-  if (rc) return rc;
-  for (auto &e : ix->ev_q) if (!e) SIA_CUDA(cudaEventCreate(&e));
-  ix->last_lookup_ms = ix->last_vote_ms = 0;
+  const QueryOut out{{d_out_song, d_out_diff, d_out_count, d_out_rows, d_out_nres}, d_out_batches, d_out_exit};
   const int L = std::max(topn, 2);                   // the exit rule always looks at the top two
-  const int64_t span = (int64_t)ix->max_song + 1, B = batch_hashes;
-  for (int64_t q0 = 0; q0 < n_queries; q0 += kMaxQueriesPerPass) {
-    const int nq = (int)std::min<int64_t>(kMaxQueriesPerPass, n_queries - q0);
-    const int64_t i0 = h_query_starts[q0], n = h_query_starts[q0 + nq] - i0;
-    if (h_stats) h_stats[0] += n;
-    if (n == 0) continue;    // empty queries: 0 results, 0 batches
-    if ((rc = ix->arena.reserve((size_t)(nq + 1) * 8 * 3 + (size_t)nq * 4 + (size_t)n * (32 + 20 + 4 + 8) + lookup_bytes(n) +
-                                scan_tmp_bytes(n) + (1 << 20))))
-      return rc;
-    int64_t *d_qs = ix->arena.take<int64_t>(nq + 1);
-    int64_t *d_goff = ix->arena.take<int64_t>(2 * (size_t)(nq + 1));
-    uint32_t *d_nb = ix->arena.take<uint32_t>(nq);
-    ulonglong2 *ea = ix->arena.take<ulonglong2>(n), *eb = ix->arena.take<ulonglong2>(n);
-    SIA_REQUIRE(d_qs && d_goff && d_nb && ea && eb, SIA_E_NOMEM, "index scratch arena too small (query)");
-    SIA_CUDA(cudaMemcpyAsync(d_qs, h_query_starts + q0, sizeof(int64_t) * (nq + 1), cudaMemcpyHostToDevice, s));
-    SIA_CUDA(cudaEventRecord(ix->ev_q[0], s));
-    Lookup Lk;
-    if ((rc = lookup_queries(ix, d_hash, d_qoff, h_query_starts + q0, d_qs, nq, ea, eb, Lk, s))) return rc;
-    SIA_CUDA(cudaEventRecord(ix->ev_q[1], s));
+  const int64_t B = batch_hashes;
+  const auto vote = [&](QueryPass &p) -> int {
+    const int nq = p.nq;
+    const int64_t n = p.n, i0 = p.i0, q0 = p.q0;
+    const int64_t *h_off_all = p.h_off_all, *h_off_head = p.h_off_head, *d_qs = p.d_qs;
+    const Lookup &Lk = p.L;
+    cudaStream_t s = p.s;
     // distinct-hash rank of every entry: hr[i + 1] - 1 - hr[first entry of its query]
+    uint32_t *d_nb = ix->arena.take<uint32_t>(nq);
     uint32_t *d_head = ix->arena.take<uint32_t>(n);
     int64_t *d_hr = ix->arena.take<int64_t>(n + 1);
     void *d_stmp = ix->arena.take<char>(scan_tmp_bytes(n));
-    SIA_REQUIRE(d_head && d_hr && d_stmp, SIA_E_NOMEM, "index scratch arena too small (batches)");
+    SIA_REQUIRE(d_nb && d_head && d_hr && d_stmp, SIA_E_NOMEM, "index scratch arena too small (batches)");
     head_flags_kernel<<<grid_for(n), 256, 0, s>>>(Lk.ent, n, d_head);
     SIA_CHECK_LAUNCH();
-    if ((rc = exclusive_scan_u32(d_head, d_hr, n, d_stmp, s))) return rc;
+    int rc = exclusive_scan_u32(d_head, d_hr, n, d_stmp, s);
+    if (rc) return rc;
     query_batches_kernel<<<grid_for(nq), 256, 0, s>>>(d_hr, d_qs, i0, nq, B, d_nb, d_out_batches + q0);
     SIA_CHECK_LAUNCH();
     std::vector<uint32_t> h_nb(nq);
     SIA_CUDA(cudaMemcpyAsync(h_nb.data(), d_nb, sizeof(uint32_t) * nq, cudaMemcpyDeviceToHost, s));
-    std::vector<int64_t> h_goff;
-    if ((rc = query_offsets(Lk, d_qs, i0, nq, d_goff, h_goff, s))) return rc;     // synchronises: h_nb is there too
-    const int64_t *h_off_all = h_goff.data(), *h_off_head = h_goff.data() + nq + 1;
-    for (int q = 0; q < nq; ++q)
-      SIA_REQUIRE(h_off_all[q + 1] - h_off_all[q] < (1ll << 31), SIA_E_UNSUPPORTED, "query_apriori: more than 2^31 vote tuples in one query");
+    SIA_CUDA(cudaStreamSynchronize(s));
     std::vector<QMeta> h_meta(nq);
-    for (int qa = 0; qa < nq;) {
-      int qb = qa + 1;
-      while (qb < nq && h_off_all[qb + 1] - h_off_all[qa] <= tuple_budget) ++qb;
+    // queries without matches are in no group: 0 results, out_batches = K_q, no exit
+    for (const auto &[qa, qb] : split_groups(h_off_all, nq, p.budget, nullptr)) {
       const int gq = qb - qa;
-      const int64_t tuples = h_off_all[qb] - h_off_all[qa];
       uint32_t k_max = 0;
       for (int q = qa; q < qb; ++q) if (h_off_all[q + 1] > h_off_all[q]) k_max = std::max(k_max, h_nb[q]);
-      if (tuples == 0) { qa = qb; continue; }      // no matches: 0 results, out_batches = K_q, no exit
-      const Group g = make_group(qa, qb, h_off_all, h_off_head, span, h_meta.data());
+      const Group g = make_group(qa, qb, h_off_all, h_off_head, (int64_t)ix->max_song + 1, h_meta.data());
       int64_t nb_slots = 0, nc = 0;
       for (int q = qa; q < qb; ++q) {
         QMeta &m = h_meta[q];
@@ -316,7 +283,7 @@ extern "C" int sia_index_query_apriori(sia_index *ix, const uint8_t *d_hash, con
         m.cursor = 0;
         nb_slots += m.bin_cap; nc += m.cand;
       }
-      const int64_t e0 = h_query_starts[q0 + qa] - i0, ne = h_query_starts[q0 + qb] - i0 - e0;
+      const int64_t e0 = p.h_qs[qa] - i0, ne = p.h_qs[qb] - i0 - e0;
       const size_t bytes = (size_t)gq * (sizeof(QMeta) + 4 * 2 + 8 + 4 * 2 * L) + (size_t)nb_slots * 12 +
                            (size_t)g.ns * (8 + 4 + 4 + (g.dense ? 0 : 4)) + (size_t)nc * 4 + (size_t)ne * 4 +
                            (size_t)(k_max + 1) * (4 + 8) + scan_tmp_bytes(k_max) + 64 + (1 << 16);
@@ -381,17 +348,13 @@ extern "C" int sia_index_query_apriori(sia_index *ix, const uint8_t *d_hash, con
       SIA_CUDA(cudaStreamSynchronize(s));      // the tables are reused by the next group
       SIA_REQUIRE(!(h_flags & 8), SIA_E_CUDA, "query_apriori: vote table overflow (internal error)");
       if (h_stats) { h_stats[2] += (int64_t)h_st[0]; h_stats[1] += (int64_t)h_st[1]; }
-      qa = qb;
     }
-    SIA_CUDA(cudaEventRecord(ix->ev_q[2], s));
     std::vector<int32_t> h_batches(nq);
     SIA_CUDA(cudaMemcpyAsync(h_batches.data(), d_out_batches + q0, sizeof(int32_t) * nq, cudaMemcpyDeviceToHost, s));
     SIA_CUDA(cudaStreamSynchronize(s));
     if (h_stats) for (int32_t b : h_batches) h_stats[3] += b;
-    float t_lookup = 0, t_vote = 0;
-    cudaEventElapsedTime(&t_lookup, ix->ev_q[0], ix->ev_q[1]);
-    cudaEventElapsedTime(&t_vote, ix->ev_q[1], ix->ev_q[2]);
-    ix->last_lookup_ms += t_lookup; ix->last_vote_ms += t_vote;
-  }
-  return SIA_OK;
+    return SIA_OK;
+  };
+  return query_passes(ix, d_hash, d_qoff, h_query_starts, n_queries, topn, out, h_stats, (cudaStream_t)stream, false,
+                      [](int nq, int64_t n) { return (size_t)nq * 4 + (size_t)n * (4 + 8) + scan_tmp_bytes(n); }, vote);
 }

@@ -829,7 +829,7 @@ int pvote_entry_info(const Lookup &L, longlong2 *d_info, uint32_t *d_qh, cudaStr
 
 int pvote_entries(Arena &ar, const Lookup &L, const longlong2 *d_info, const uint32_t *d_qh, const uint64_t *post, const int64_t *d_qs,
                   int64_t i0, const int64_t *d_goff, const int64_t *h_goff, int qa, int qb, int qid_base, int topn, const PvOut &out,
-                  uint32_t *d_qover, uint32_t *d_qbins, unsigned long long *d_nbins, cudaStream_t s, double *stage_ms) {
+                  uint32_t *d_qover, uint32_t *d_qbins, unsigned long long *d_nbins, cudaStream_t s, StageEvents &tm) {
   const int nq = qb - qa;
   if (nq <= 0) return SIA_OK;
   int rc = pv_attrs();
@@ -851,8 +851,7 @@ int pvote_entries(Arena &ar, const Lookup &L, const longlong2 *d_info, const uin
   PvScratch S;
   SIA_REQUIRE(pv_take(ar, S, nq, nq, regions, region_tuples, blocks, topn), SIA_E_NOMEM,
               "index scratch arena too small (partitioned vote)");
-  static cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};     // SIA_QUERY_TIMING only
-  if (stage_ms) { if (!ev[0]) for (auto &e : ev) cudaEventCreate(&e); cudaEventRecord(ev[0], s); }
+  tm.mark(0, s);
   SIA_CUDA(cudaMemsetAsync(S.fill, 0, sizeof(uint32_t) * regions, s));
   pv_segs_entries_kernel<<<grid_for(nq), 256, 0, s>>>(d_goff, qa, nq, S.seg_lo, S.seg_cnt, 0, 0, 0);
   pv_layout_kernel<<<1, 1024, 0, s>>>(S.seg_cnt, nq, 1, tune, S.pq, S.q_ridx0, S.seg_blk0, S.tot);
@@ -862,19 +861,15 @@ int pvote_entries(Arena &ar, const Lookup &L, const longlong2 *d_info, const uin
   a.pq = S.pq; a.tot = S.tot; a.regions = S.regions; a.fill = S.fill; a.qover = d_qover; a.q_lo = qa;
   a.maxp = (int)std::min<uint32_t>(kMaxParts, (maxp + 511u) & ~511u);
   a.off = L.off_all; a.info = d_info; a.qh = d_qh; a.post = post; a.q_ent = d_qs; a.i0 = i0;
-  if (stage_ms) cudaEventRecord(ev[1], s);
+  tm.mark(1, s);
   pv_scatter_kernel<0><<<(unsigned)blocks, kScThreads, scatter_smem(a.maxp), s>>>(a);
-  if (stage_ms) cudaEventRecord(ev[2], s);
+  tm.mark(2, s);
   pv_count_kernel<<<(unsigned)ceil_div(regions, kRegionsPerCta), kCntThreads, kCountSmem, s>>>(S.regions, S.fill, S.pq, S.reg_q, S.tot, qa, d_qover, topn, S.cand,
                                                                      d_nbins ? d_qbins : nullptr);
   pv_merge_kernel<<<(unsigned)ceil_div((int64_t)nq * 32, 256), 256, 0, s>>>(S.cand, S.pq, nq, qa, qid_base, d_qover, topn, out, nullptr,
                                                                             d_qbins, d_nbins);
   SIA_CHECK_LAUNCH();
-  if (stage_ms) {
-    cudaEventRecord(ev[3], s);
-    cudaEventSynchronize(ev[3]);
-    for (int k = 0; k < 3; ++k) { float t = 0; cudaEventElapsedTime(&t, ev[k], ev[k + 1]); stage_ms[k] += t; }
-  }
+  tm.mark(3, s);
   return SIA_OK;
 }
 

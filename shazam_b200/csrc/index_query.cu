@@ -1,7 +1,13 @@
 // K4, query side — the SELECT ... WHERE hash IN (...) lookup (recognizer.py:60-64, 252-259) and the vote inside
 // align_matches (recognizer.py:303-310) for a batch of queries.  The default vote is the partitioned vote of
 // index_pvote.cu (called from here per group of queries); this file holds the lookup, the grouping, and the TABLE vote
-// described below — the path of queries the partitioned vote flags (a bin above a region's size) and of SIA_VOTE=tables.
+// described below — the path of queries the partitioned vote flags (a bin above a region's size) and of every query
+// when topn is above what the partitioned vote ranks (kPvMaxTopn).
+//
+// query_passes is the frame of both device query calls (sia_index_query_batch here, sia_index_query_apriori in
+// index_apriori.cu): argument checks, passes of up to kMaxQueriesPerPass queries, per pass the lookup and the tuple
+// offsets, then the caller's vote step.  split_groups cuts a pass into groups under the tuple budget, and table_vote
+// runs one attempt of the table vote over one group, for the entries of a lookup and for vote keys alike.
 //
 // Lookup: the (hash, offset) pairs of the queries are packed into 16-byte entries, sorted by (query, hash, offset)
 // — duplicates drop out, equal hashes of one query become adjacent — and each is looked up: directory -> binary
@@ -26,7 +32,7 @@
 #include "index.cuh"
 
 #include <chrono>
-#include <cstring>
+#include <type_traits>
 
 using namespace sia;
 using namespace sia::tvote;
@@ -224,6 +230,20 @@ __device__ __forceinline__ void tuple_pair_pass(const QMeta &m, bool va, uint32_
   }
 }
 
+// a warp's step left query cur_q: PASS_MARK adds the warp's candidate count to cur_q's, PASS_VOTE writes the buffered
+// candidates to cur_q's list (the buffer holds one query's candidates)
+template <int PASS>
+__device__ __forceinline__ void leave_query(uint32_t cur_q, uint32_t &acc, unsigned long long *__restrict__ cbuf, int &ncand,
+                                            QMeta *__restrict__ meta, const Tables &T, int lane, int32_t *__restrict__ flags) {
+  if (PASS == PASS_MARK) {
+#pragma unroll
+    for (int d = 16; d; d >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, d);
+    if (lane == 0 && acc) atomicAdd(&meta[cur_q].cand, acc);
+    acc = 0;
+  }
+  if (PASS == PASS_VOTE) cand_flush(cbuf, ncand, cur_q, meta, T.cand, lane, flags);
+}
+
 __device__ __forceinline__ unsigned long long cand_key(uint32_t q, uint32_t song, uint32_t dbits) {
   return ((unsigned long long)q << (kSongBits + kDiffBits)) | ((unsigned long long)song << kDiffBits) | dbits;
 }
@@ -312,14 +332,8 @@ entries_pass_kernel(const ulonglong2 *__restrict__ ent, int64_t e0, int64_t n, c
     const ulonglong2 e = ent[ei];
     const uint32_t q = (uint32_t)(e.y >> 40);
     if (PASS == PASS_SINGLES && !qflag[q]) continue;
-    if (PASS == PASS_MARK && q != cur_q) {                       // flush the candidate count of the previous query
-#pragma unroll
-      for (int d = 16; d; d >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, d);
-      if (lane == 0 && acc) atomicAdd(&meta[cur_q].cand, acc);
-      acc = 0; cur_q = q;
-    }
-    if (PASS == PASS_VOTE && q != cur_q) {                       // the buffer holds one query's candidates
-      cand_flush(cbuf, ncand, cur_q, meta, T.cand, lane, flags);
+    if ((PASS == PASS_MARK || PASS == PASS_VOTE) && q != cur_q) {
+      leave_query<PASS>(cur_q, acc, cbuf, ncand, meta, T, lane, flags);
       cur_q = q;
     }
     const QMeta m = meta[q];
@@ -348,14 +362,11 @@ entries_pass_kernel(const ulonglong2 *__restrict__ ent, int64_t e0, int64_t n, c
     }
     __syncwarp();
   }
-  if (PASS == PASS_VOTE) cand_flush(cbuf, ncand, cur_q, meta, T.cand, lane, flags);
-  if (PASS == PASS_MARK || (PASS == PASS_VOTE && n_bins)) {
+  leave_query<PASS>(cur_q, acc, cbuf, ncand, meta, T, lane, flags);
+  if (PASS == PASS_VOTE && n_bins) {                             // this warp's bins of count 1
 #pragma unroll
     for (int d = 16; d; d >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, d);
-    if (lane == 0 && acc) {
-      if (PASS == PASS_MARK) atomicAdd(&meta[cur_q].cand, acc);
-      else atomicAdd(n_bins, (unsigned long long)acc);
-    }
+    if (lane == 0 && acc) atomicAdd(n_bins, (unsigned long long)acc);
   }
 }
 
@@ -444,13 +455,7 @@ keys_pass_kernel(const uint64_t *__restrict__ keys, int64_t cap, const int64_t *
         }
         if (PASS == PASS_SINGLES && !qflag[qq]) continue;
         if (qq != cur_q) {
-          if (PASS == PASS_MARK) {                       // flush the candidate count of the previous query
-#pragma unroll
-            for (int d = 16; d; d >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, d);
-            if (lane == 0 && acc) atomicAdd(&meta[cur_q].cand, acc);
-            acc = 0;
-          }
-          if (PASS == PASS_VOTE) cand_flush(cbuf, ncand, cur_q, meta, T.cand, lane, flags);
+          leave_query<PASS>(cur_q, acc, cbuf, ncand, meta, T, lane, flags);
           cur_q = qq;
         }
         const QMeta m = meta[qq];
@@ -463,12 +468,7 @@ keys_pass_kernel(const uint64_t *__restrict__ keys, int64_t cap, const int64_t *
         __syncwarp();
       }
     }
-    if (PASS == PASS_MARK) {
-#pragma unroll
-      for (int d = 16; d; d >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, d);
-      if (lane == 0 && acc) atomicAdd(&meta[cur_q].cand, acc);
-    }
-    if (PASS == PASS_VOTE) cand_flush(cbuf, ncand, cur_q, meta, T.cand, lane, flags);
+    leave_query<PASS>(cur_q, acc, cbuf, ncand, meta, T, lane, flags);
   }
 }
 
@@ -676,6 +676,110 @@ int check_status(sia_index *ix, cudaStream_t s, int mask, const char *msg) {
 // scratch of the handle-less vote entry point, kept per device (cudaMalloc of GBs per call is slow)
 Arena g_vote_tables[64];
 
+// ---- the table vote: one attempt over one set of tables ---------------------------------------------------------
+// bin slots reserved for `tuples` tuples over nq queries: first for up to a quarter of the tuples landing in twice-hit
+// buckets (12 % on the benchmark's index), then — if pass 1 counted more — for all of them
+int64_t bin_slots_for(int64_t tuples, int64_t nq, int attempt) {
+  return (attempt == 0 ? tuples / 2 : 2 * tuples) + 32 * nq;
+}
+
+// bytes of the tables of group g for `tuples` tuples: filter + worst-case bins of the attempt (every tuple a
+// candidate) + songs + the pieces of the entries path
+size_t table_bytes(const Group &g, int64_t tuples, int attempt) {
+  const int64_t nq = g.qb - g.qa;
+  return (size_t)(tuples + nq) * 4 + (size_t)bin_slots_for(tuples, nq, attempt) * 16 + (size_t)g.ns * (g.dense ? 8 : 12) +
+         (size_t)(tuples / (kVoteTuples >> 3) + 16) * 4 + 8192;
+}
+
+// what a table vote reads and writes besides its tables
+struct TableVoteArgs {
+  QMeta *meta;                    // indexed by the query id of the tuples
+  uint32_t *qflag;                // per query: needs the singles pass
+  int64_t *total;                 // bin slots in use
+  int32_t *flags;                 // [0] device flags of the attempt, [1] queries of the group that need the singles pass
+  unsigned long long *n_bins;     // NULL, or += the distinct bins of count >= 2
+  const uint32_t *qsel;           // NULL, or only these queries (the ones the partitioned vote left over)
+  int qid_base, topn;             // output row of query q: q + qid_base
+  PvOut out;
+};
+
+template <int P> using PassTag = std::integral_constant<int, P>;
+
+template <bool D, class Pass>
+void table_vote_launches(const Pass &pass, const Group &g, const Tables &T, int64_t nb_cap, const TableVoteArgs &a,
+                         StageEvents &tm, cudaStream_t s) {
+  const std::bool_constant<D> dense{};
+  const int gq = g.qb - g.qa;
+  pass(dense, PassTag<PASS_MARK>{}, T);
+  tm.mark(2, s);
+  layout_bins_kernel<<<1, 1024, 0, s>>>(a.meta, g.qa, g.qb, a.total);
+  zero_bins_kernel<<<kNumSMs * 8, 256, 0, s>>>(T.bins, T.bin_cnt, a.total, nb_cap, a.flags);
+  tm.mark(3, s);
+  pass(dense, PassTag<PASS_VOTE>{}, T);
+  tm.mark(4, s);
+  cand_vote_kernel<D><<<kNumSMs * 8, 256, 0, s>>>(T.cand, a.meta, g.qa, g.qb, T, a.n_bins, a.flags);
+  tm.mark(5, s);
+  topn_kernel<D, false><<<gq, 256, 0, s>>>(T, a.meta, g.qa, a.qid_base, a.topn, a.qflag, a.flags + 1, a.qsel, a.out.song,
+                                           a.out.diff, a.out.count, a.out.rows, a.out.nres);
+  tm.mark(6, s);
+  pass(dense, PassTag<PASS_SINGLES>{}, T);
+  topn_kernel<D, true><<<gq, 256, 0, s>>>(T, a.meta, g.qa, a.qid_base, a.topn, a.qflag, a.flags + 1, a.qsel, a.out.song,
+                                          a.out.diff, a.out.count, a.out.rows, a.out.nres);
+  tm.mark(7, s);
+  pass(dense, PassTag<PASS_ROWS>{}, T);
+  tm.mark(8, s);
+}
+
+// One attempt of the table vote over the queries [g.qa, g.qb) of `tuples` vote tuples: carves the group's tables from
+// `ar` (bin slots for `attempt`), zeroes them, lays out the queries' QMeta on the device (layout()), then enqueues
+// mark → bin layout → zero bins → collect → candidate vote → top-n → singles → top-n → rows.  pass(dense, PassTag<P>,
+// tables) launches the walk of pass P over the caller's tuples (entries or vote keys; PASS_ROWS: the winners' rows).
+// tm gets marks 0..8: start, after the layout, then after each stage.
+template <class Layout, class Pass>
+int table_vote(Arena &ar, const Group &g, int64_t tuples, int attempt, const TableVoteArgs &a, const Layout &layout,
+               const Pass &pass, StageEvents &tm, cudaStream_t s) {
+  const int64_t nb_cap = bin_slots_for(tuples, g.qb - g.qa, attempt);
+  Tables T{};
+  T.filter = ar.take<uint32_t>(g.nf);
+  T.song_best = ar.take<unsigned long long>(g.ns);
+  T.song_key = g.dense ? nullptr : ar.take<uint32_t>(g.ns);
+  T.bins = ar.take<unsigned long long>(nb_cap);
+  T.bin_cnt = ar.take<uint32_t>(nb_cap);
+  T.cand = ar.take<unsigned long long>(nb_cap / 2 + 16);
+  SIA_REQUIRE(T.filter && T.song_best && (g.dense || T.song_key) && T.bins && T.bin_cnt && T.cand, SIA_E_NOMEM,
+              "index scratch arena too small (vote tables)");
+  tm.mark(0, s);
+  SIA_CUDA(cudaMemsetAsync(a.flags + 1, 0, sizeof(int32_t), s));
+  SIA_CUDA(cudaMemsetAsync(T.filter, 0, sizeof(uint32_t) * g.nf, s));
+  SIA_CUDA(cudaMemsetAsync(T.song_best, 0, sizeof(unsigned long long) * g.ns, s));
+  if (!g.dense) SIA_CUDA(cudaMemsetAsync(T.song_key, 0, sizeof(uint32_t) * g.ns, s));
+  int rc = layout();
+  if (rc) return rc;
+  tm.mark(1, s);
+  if (g.dense) table_vote_launches<true>(pass, g, T, nb_cap, a, tm, s);
+  else table_vote_launches<false>(pass, g, T, nb_cap, a, tm, s);
+  SIA_CHECK_LAUNCH();
+  return SIA_OK;
+}
+
+// after an attempt, from its device flags: retry when the bin tables outgrew attempt 0's reservation (tie-heavy
+// queries), to be voted again with attempt 1; a full table (flag 8) is an error, `overflow` says why
+int attempt_retry(int32_t h_flags, int attempt, const char *overflow, bool &retry) {
+  SIA_REQUIRE(!(h_flags & 8), SIA_E_CUDA, overflow);
+  retry = (h_flags & 32) != 0;
+  SIA_REQUIRE(!retry || attempt == 0, SIA_E_CUDA, "vote: bin table overflow (internal error)");
+  return SIA_OK;
+}
+
+// vote tuples per group of queries: SIA_VOTE_GROUP_TUPLES (default 2^29), bounded by what the device has left
+int group_tuple_budget(::sia_index *ix, int64_t &budget) {
+  budget = getenv("SIA_VOTE_GROUP_TUPLES") ? std::max(1ll, atoll(getenv("SIA_VOTE_GROUP_TUPLES"))) : (512ll << 20);
+  size_t free_b = 0, total_b = 0;
+  SIA_CUDA(cudaMemGetInfo(&free_b, &total_b));
+  budget = std::max<int64_t>(1 << 20, std::min<int64_t>(budget, (int64_t)((free_b + ix->arena3.cap) * 0.6 / 40)));
+  return SIA_OK;
+}
+
 }  // namespace
 
 namespace sia {
@@ -721,17 +825,6 @@ int lookup_sorted(::sia_index *ix, Arena &ar, ulonglong2 *a, ulonglong2 *b, int6
   return SIA_OK;
 }
 
-// bytes of vote tables for `tuples` tuples over nq queries: filter + worst-case bins (every tuple a candidate) + songs
-static size_t vote_table_bytes(int64_t tuples, int64_t nq, int64_t bin_slots, int64_t song_slots, bool dense) {
-  return (size_t)(tuples + nq) * 4 + (size_t)bin_slots * 16 + (size_t)song_slots * (dense ? 8 : 12) +
-         (size_t)(tuples / (kVoteTuples >> 3) + 16) * 4 + 8192;
-}
-// bin slots reserved for `tuples` tuples over nq queries: first for up to a quarter of the tuples landing in twice-hit
-// buckets (12 % on the benchmark's index), then — if pass 1 counted more — for all of them
-static int64_t bin_slots_for(int64_t tuples, int64_t nq, int attempt) {
-  return (attempt == 0 ? tuples / 2 : 2 * tuples) + 32 * nq;
-}
-
 Arena &vote_arena(int device) { return g_vote_tables[device]; }
 
 void vote_scratch_release(int device) {
@@ -753,87 +846,44 @@ struct KeyVote {
   int stage = 1;                   // 0: the partitioned vote is in flight; 1: the table vote
   uint32_t *d_small = nullptr;     // per device, allocated once: [0] unsorted, [1] flagged queries, [64..] per-query flags
   const uint32_t *qsel = nullptr;  // table vote: only these queries (the ones the partitioned vote left over)
-  cudaEvent_t ev[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // SIA_QUERY_TIMING only
-  bool timed = false;
+  StageEvents ev;                  // SIA_QUERY_TIMING
 };
 static KeyVote g_key_vote[64];
 
 // enqueue every launch of one attempt (0: bin slots for a quarter of the keys being candidates; 1: for all of them)
 static int key_vote_enqueue(KeyVote &v, int attempt) {
-  const uint32_t *qsel = v.qsel;
-  const int nq = v.n_queries, n_slots = v.n_slots, topn = v.topn;
-  const int64_t cap = v.cap;
-  const uint64_t *d_keys = v.d_keys;
-  const int64_t *d_counts = v.d_counts;
-  int32_t *d_out_song = v.o_song, *d_out_diff = v.o_diff, *d_out_count = v.o_count, *d_out_rows = v.o_rows, *d_out_nres = v.o_nres;
-  cudaStream_t s = v.s;
-  const int64_t T = (int64_t)n_slots * cap;             // upper bound of the keys
+  const int nq = v.n_queries;
+  const int64_t n_keys = (int64_t)v.n_slots * v.cap;     // upper bound of the keys
   Arena &ar = g_vote_tables[v.device];
   // song tables: dense (slot = song id) when that is the smaller layout, else open addressing
-  const int64_t span = (int64_t)v.max_song + 1;
-  const int64_t ns_hashed = 2 * T + 32ll * nq;
+  const int64_t span = (int64_t)v.max_song + 1, ns_hashed = 2 * n_keys + 32ll * nq;
   const bool dense = span * nq * 8 <= ns_hashed * 12;
-  const int64_t ns = dense ? span * nq : ns_hashed;
-  const int64_t nf = T + nq;
-  const int64_t nb_cap = bin_slots_for(T, nq, attempt);
-  int rc = ar.reserve(vote_table_bytes(T, nq, nb_cap, ns, dense) + (size_t)nq * (sizeof(QMeta) + 8) + 65536);
+  const Group g{0, nq, dense, n_keys + nq, dense ? span * nq : ns_hashed};
+  int rc = ar.reserve(table_bytes(g, n_keys, attempt) + (size_t)nq * (sizeof(QMeta) + 8) + 65536);
   if (rc) return rc;
   QMeta *meta = ar.take<QMeta>(nq);
   uint32_t *cnt = ar.take<uint32_t>(nq), *qflag = ar.take<uint32_t>(nq);
   int64_t *total = ar.take<int64_t>(1);
-  int32_t *flags = ar.take<int32_t>(2);          // [0] flags, [1] queries that need the singles pass
-  int32_t *nflag = flags + 1;
-  Tables Tb;
-  Tb.filter = ar.take<uint32_t>(nf);
-  Tb.song_best = ar.take<unsigned long long>(ns);
-  Tb.song_key = dense ? nullptr : ar.take<uint32_t>(ns);
-  Tb.bins = ar.take<unsigned long long>(nb_cap);
-  Tb.bin_cnt = ar.take<uint32_t>(nb_cap);
-  Tb.cand = ar.take<unsigned long long>(nb_cap / 2 + 16);
-  SIA_REQUIRE(meta && cnt && qflag && total && flags && Tb.filter && Tb.song_best && Tb.bins && Tb.bin_cnt && Tb.cand &&
-              (dense || Tb.song_key), SIA_E_NOMEM, "vote: scratch");
+  int32_t *flags = ar.take<int32_t>(2);
+  SIA_REQUIRE(meta && cnt && qflag && total && flags, SIA_E_NOMEM, "vote: scratch");
   v.d_flags = flags;
-  v.timed = getenv("SIA_QUERY_TIMING") != nullptr;
-  if (v.timed) { for (auto &e : v.ev) if (!e) cudaEventCreate(&e); cudaEventRecord(v.ev[0], s); }
-  SIA_CUDA(cudaMemsetAsync(cnt, 0, sizeof(uint32_t) * nq, s));
-  SIA_CUDA(cudaMemsetAsync(flags, 0, 2 * sizeof(int32_t), s));
-  SIA_CUDA(cudaMemsetAsync(Tb.filter, 0, sizeof(uint32_t) * nf, s));
-  SIA_CUDA(cudaMemsetAsync(Tb.song_best, 0, sizeof(unsigned long long) * ns, s));
-  if (!dense) SIA_CUDA(cudaMemsetAsync(Tb.song_key, 0, sizeof(uint32_t) * ns, s));
+  v.ev.on = getenv("SIA_QUERY_TIMING") != nullptr;
+  SIA_CUDA(cudaMemsetAsync(flags, 0, sizeof(int32_t), v.s));
   // blockIdx.y = slot; the x blocks of a slot stride over its keys (~32 resident blocks per SM in all)
-  const dim3 grid((unsigned)std::max<int64_t>(1, std::min<int64_t>(ceil_div(cap, 512), (kNumSMs * 32) / n_slots + 1)), (unsigned)n_slots);
-  count_keys_kernel<<<grid, 256, 0, s>>>(d_keys, cap, d_counts, nq, qsel, cnt, flags);
-  layout_keys_kernel<<<1, 1024, 0, s>>>(cnt, nq, dense ? span : 0, qsel, meta);
-#define SIA_KEYS_PASS(D, P)                                                                                            \
-  keys_pass_kernel<D, P><<<grid, 256, 0, s>>>(d_keys, cap, d_counts, nq, meta, Tb, qflag, nflag, qsel, topn,           \
-                                              d_out_song, d_out_nres, d_out_rows, flags)
-#define SIA_KSTAGE(k) do { if (v.timed) cudaEventRecord(v.ev[k], s); } while (0)
-#define SIA_KEYS_VOTE(D)                                                                                               \
-  do {                                                                                                                 \
-    SIA_KSTAGE(1);                                                                                                     \
-    SIA_KEYS_PASS(D, PASS_MARK);                                                                                       \
-    SIA_KSTAGE(2);                                                                                                     \
-    layout_bins_kernel<<<1, 1024, 0, s>>>(meta, 0, nq, total);                                                         \
-    zero_bins_kernel<<<kNumSMs * 8, 256, 0, s>>>(Tb.bins, Tb.bin_cnt, total, nb_cap, flags);                           \
-    SIA_KEYS_PASS(D, PASS_VOTE);                                                                                       \
-    SIA_KSTAGE(3);                                                                                                     \
-    cand_vote_kernel<D><<<kNumSMs * 8, 256, 0, s>>>(Tb.cand, meta, 0, nq, Tb, nullptr, flags);                         \
-    SIA_KSTAGE(4);                                                                                                     \
-    topn_kernel<D, false><<<nq, 256, 0, s>>>(Tb, meta, 0, 0, topn, qflag, nflag, qsel, d_out_song, d_out_diff,         \
-                                             d_out_count, d_out_rows, d_out_nres);                                     \
-    SIA_KEYS_PASS(D, PASS_SINGLES);                                                                                    \
-    topn_kernel<D, true><<<nq, 256, 0, s>>>(Tb, meta, 0, 0, topn, qflag, nflag, qsel, d_out_song, d_out_diff,          \
-                                            d_out_count, d_out_rows, d_out_nres);                                      \
-    SIA_KSTAGE(5);                                                                                                     \
-    SIA_KEYS_PASS(D, PASS_ROWS);                                                                                       \
-    SIA_KSTAGE(6);                                                                                                     \
-  } while (0)
-  if (dense) SIA_KEYS_VOTE(true); else SIA_KEYS_VOTE(false);
-#undef SIA_KEYS_VOTE
-#undef SIA_KEYS_PASS
-#undef SIA_KSTAGE
-  SIA_CHECK_LAUNCH();
-  return SIA_OK;
+  const dim3 grid((unsigned)std::max<int64_t>(1, std::min<int64_t>(ceil_div(v.cap, 512), (kNumSMs * 32) / v.n_slots + 1)),
+                  (unsigned)v.n_slots);
+  const TableVoteArgs a{meta, qflag, total, flags, nullptr, v.qsel, 0, v.topn, {v.o_song, v.o_diff, v.o_count, v.o_rows, v.o_nres}};
+  const auto layout = [&]() -> int {
+    SIA_CUDA(cudaMemsetAsync(cnt, 0, sizeof(uint32_t) * nq, v.s));
+    count_keys_kernel<<<grid, 256, 0, v.s>>>(v.d_keys, v.cap, v.d_counts, nq, v.qsel, cnt, flags);
+    layout_keys_kernel<<<1, 1024, 0, v.s>>>(cnt, nq, dense ? span : 0, v.qsel, meta);
+    return SIA_OK;
+  };
+  const auto pass = [&](auto d, auto p, const Tables &T) {
+    keys_pass_kernel<decltype(d)::value, decltype(p)::value><<<grid, 256, 0, v.s>>>(
+        v.d_keys, v.cap, v.d_counts, nq, meta, T, qflag, flags + 1, v.qsel, v.topn, v.o_song, v.o_nres, v.o_rows, flags);
+  };
+  return table_vote(ar, g, n_keys, attempt, a, layout, pass, v.ev, v.s);
 }
 
 // the partitioned vote of the keys (index_pvote.cu): shared-memory tables, streaming traffic only
@@ -843,12 +893,12 @@ static int key_pvote_enqueue(KeyVote &v) {
   int rc = ar.reserve(pvote_bytes((int64_t)v.n_slots * v.cap, v.n_queries, v.n_slots, v.topn) + 65536);
   if (rc) return rc;
   SIA_CUDA(cudaMemsetAsync(v.d_small, 0, sizeof(uint32_t) * (64 + (size_t)v.n_queries), v.s));
-  v.timed = getenv("SIA_QUERY_TIMING") != nullptr;
-  if (v.timed) { for (auto &e : v.ev) if (!e) cudaEventCreate(&e); cudaEventRecord(v.ev[0], v.s); }
+  v.ev.on = getenv("SIA_QUERY_TIMING") != nullptr;
+  v.ev.mark(0, v.s);
   const PvOut po{v.o_song, v.o_diff, v.o_count, v.o_rows, v.o_nres};
   rc = pvote_key_slots(ar, v.d_keys, v.n_slots, v.cap, v.d_counts, v.n_queries, v.topn, po, v.d_small + 64, v.d_small, v.s);
   if (rc) return rc;
-  if (v.timed) cudaEventRecord(v.ev[1], v.s);
+  v.ev.mark(1, v.s);
   return SIA_OK;
 }
 
@@ -863,12 +913,9 @@ int vote_key_slots_finish(int device) {
     uint32_t h2[2] = {0, 0};
     SIA_CUDA(cudaMemcpyAsync(h2, v.d_small, sizeof h2, cudaMemcpyDeviceToHost, v.s));
     SIA_CUDA(cudaStreamSynchronize(v.s));
-    if (v.timed) {
-      float t = 0;
-      cudaEventElapsedTime(&t, v.ev[0], v.ev[1]);
+    if (v.ev.on)
       fprintf(stderr, "[sia] key vote (partitioned): %d queries, %d slots x %lld: %.2f ms, unsorted %u, flagged queries %u\n",
-              v.n_queries, v.n_slots, (long long)v.cap, t, h2[0], h2[1]);
-    }
+              v.n_queries, v.n_slots, (long long)v.cap, v.ev.ms(0, 1), h2[0], h2[1]);
     if (!h2[0] && !h2[1]) return SIA_OK;
     // keys not grouped by query (any order is allowed): everything goes to the table vote; else only the flagged queries
     v.qsel = h2[0] ? nullptr : v.d_small + 64;
@@ -876,25 +923,22 @@ int vote_key_slots_finish(int device) {
     int rc = key_vote_enqueue(v, 0);
     if (rc) return rc;
   }
-  for (int attempt = 0; attempt < 2; ++attempt) {
+  for (int attempt = 0;; ++attempt) {
     int32_t h_flags = 0;
     SIA_CUDA(cudaMemcpyAsync(&h_flags, v.d_flags, sizeof h_flags, cudaMemcpyDeviceToHost, v.s));
     SIA_CUDA(cudaStreamSynchronize(v.s));
     SIA_REQUIRE(!(h_flags & 2), SIA_E_INVALID, "vote: query id outside 0..n_queries-1");
-    SIA_REQUIRE(!(h_flags & 8), SIA_E_CUDA, "vote: table overflow (internal error, or song id above max_song)");
-    if (v.timed) {
-      float t[6];
-      for (int k = 0; k < 6; ++k) cudaEventElapsedTime(&t[k], v.ev[k], v.ev[k + 1]);
-      fprintf(stderr, "[sia] key vote: %d queries, %d slots x %lld: memsets + count + layout %.2f ms, mark %.2f, bin layout + collect %.2f, "
-              "candidate vote %.2f, topn + singles %.2f, rows %.2f\n", v.n_queries, v.n_slots, (long long)v.cap, t[0], t[1], t[2], t[3],
-              t[4], t[5]);
-    }
-    if (!(h_flags & 32)) return SIA_OK;
-    SIA_REQUIRE(attempt == 0, SIA_E_CUDA, "vote: bin table overflow (internal error)");
-    int rc = key_vote_enqueue(v, 1);
+    bool retry = false;
+    int rc = attempt_retry(h_flags, attempt, "vote: table overflow (internal error, or song id above max_song)", retry);
     if (rc) return rc;
+    StageEvents &e = v.ev;
+    if (e.on)
+      fprintf(stderr, "[sia] key vote: %d queries, %d slots x %lld: memsets + count + layout %.2f ms, mark %.2f, bin layout + collect %.2f, "
+              "candidate vote %.2f, topn + singles %.2f, rows %.2f\n", v.n_queries, v.n_slots, (long long)v.cap, e.ms(0, 1),
+              e.ms(1, 2), e.ms(2, 4), e.ms(4, 5), e.ms(5, 7), e.ms(7, 8));
+    if (!retry) return SIA_OK;
+    if ((rc = key_vote_enqueue(v, 1))) return rc;
   }
-  return SIA_OK;
 }
 
 // defer != 0: return once everything is enqueued; vote_key_slots_finish(device) completes the call (one vote in flight
@@ -918,8 +962,7 @@ int vote_key_slots(int device, const uint64_t *d_keys, int n_slots, int64_t cap,
   v.o_song = d_out_song; v.o_diff = d_out_diff; v.o_count = d_out_count; v.o_rows = d_out_rows; v.o_nres = d_out_nres;
   v.s = s;
   v.qsel = nullptr;
-  const char *vote_env = getenv("SIA_VOTE");             // "tables": the table vote for every query (A/B tests)
-  if (topn <= kPvMaxTopn && !(vote_env && !strcmp(vote_env, "tables"))) {
+  if (topn <= kPvMaxTopn) {
     v.stage = 0;
     rc = key_pvote_enqueue(v);
   } else {
@@ -958,18 +1001,24 @@ Group make_group(int qa, int qb, const int64_t *h_off_all, const int64_t *h_off_
   return g;
 }
 
-int group_tuple_budget(::sia_index *ix, int64_t &budget) {
-  budget = getenv("SIA_VOTE_GROUP_TUPLES") ? std::max(1ll, atoll(getenv("SIA_VOTE_GROUP_TUPLES"))) : (512ll << 20);
-  size_t free_b = 0, total_b = 0;
-  SIA_CUDA(cudaMemGetInfo(&free_b, &total_b));
-  budget = std::max<int64_t>(1 << 20, std::min<int64_t>(budget, (int64_t)((free_b + ix->arena3.cap) * 0.6 / 40)));
-  return SIA_OK;
+std::vector<std::pair<int, int>> split_groups(const int64_t *h_off_all, int nq, int64_t budget, const uint32_t *keep) {
+  std::vector<std::pair<int, int>> groups;
+  for (int qa = 0; qa < nq;) {
+    if (keep && !keep[qa]) { ++qa; continue; }
+    int qb = qa + 1;
+    while (qb < nq && (!keep || keep[qb]) && h_off_all[qb + 1] - h_off_all[qa] <= budget) ++qb;
+    if (h_off_all[qb] > h_off_all[qa]) groups.emplace_back(qa, qb);
+    qa = qb;
+  }
+  return groups;
 }
 
 }  // namespace tvote
 
-int lookup_queries(::sia_index *ix, const uint8_t *d_hash, const int32_t *d_qoff, const int64_t *h_query_starts,
-                   const int64_t *d_qs, int nq, ulonglong2 *ea, ulonglong2 *eb, Lookup &L, cudaStream_t s) {
+// pack the pairs [h_query_starts[0], h_query_starts[nq]) of nq queries (d_qs: the same starts on the device) into
+// ea (alt buffer eb), sort and look them up (lookup_sorted), check the offsets / ids.
+static int lookup_queries(::sia_index *ix, const uint8_t *d_hash, const int32_t *d_qoff, const int64_t *h_query_starts,
+                          const int64_t *d_qs, int nq, ulonglong2 *ea, ulonglong2 *eb, Lookup &L, cudaStream_t s) {
   const int64_t i0 = h_query_starts[0], n = h_query_starts[nq] - i0;
   int64_t max_entries = 0;
   for (int q = 0; q < nq; ++q) max_entries = std::max(max_entries, h_query_starts[q + 1] - h_query_starts[q]);
@@ -980,13 +1029,79 @@ int lookup_queries(::sia_index *ix, const uint8_t *d_hash, const int32_t *d_qoff
   return check_status(ix, s, 2 | 4, "query: offset outside 0..2^24-1 (or a posting run of 2^32 rows)");
 }
 
-int query_offsets(const Lookup &L, const int64_t *d_qs, int64_t i0, int nq, int64_t *d_goff, std::vector<int64_t> &h_goff,
-                  cudaStream_t s) {
+// scanned tuple / head-row offsets at the queries' first entries: h_goff[0..nq] = off_all, h_goff[nq+1..] = off_head
+// (d_goff: 2 * (nq + 1) device scratch).  Synchronises the stream.
+static int query_offsets(const Lookup &L, const int64_t *d_qs, int64_t i0, int nq, int64_t *d_goff, std::vector<int64_t> &h_goff,
+                         cudaStream_t s) {
   h_goff.assign(2 * (size_t)(nq + 1), 0);
   gather_offsets_kernel<<<grid_for(nq + 1), 256, 0, s>>>(L.off_all, L.off_head, d_qs, i0, nq, d_goff);
   SIA_CHECK_LAUNCH();
   SIA_CUDA(cudaMemcpyAsync(h_goff.data(), d_goff, h_goff.size() * 8, cudaMemcpyDeviceToHost, s));
   SIA_CUDA(cudaStreamSynchronize(s));
+  return SIA_OK;
+}
+
+int query_passes(::sia_index *ix, const uint8_t *d_hash, const int32_t *d_qoff, const int64_t *h_query_starts,
+                 int32_t n_queries, int32_t topn, const QueryOut &out, int64_t *h_stats, cudaStream_t s, bool timing,
+                 size_t (*extra_bytes)(int nq, int64_t n), const std::function<int(QueryPass &)> &vote) {
+  SIA_REQUIRE(ix && h_query_starts, SIA_E_INVALID, "NULL argument");
+  SIA_REQUIRE(n_queries >= 0 && topn >= 1, SIA_E_INVALID, "n_queries >= 0 and topn >= 1 required");
+  SIA_REQUIRE(ix->n_pending == 0, SIA_E_INVALID, "index has pending rows: call sia_index_finalize first");
+  if (h_stats) h_stats[0] = h_stats[1] = h_stats[2] = h_stats[3] = 0;
+  if (n_queries == 0) return SIA_OK;
+  SIA_REQUIRE(out.song && out.diff && out.count && out.rows && out.nres, SIA_E_INVALID, "NULL output");
+  int rc = set_device(ix);
+  if (rc) return rc;
+  for (int q = 0; q < n_queries; ++q)
+    SIA_REQUIRE(h_query_starts[q] <= h_query_starts[q + 1], SIA_E_INVALID, "query_starts must be non-decreasing");
+  SIA_REQUIRE(h_query_starts[n_queries] == h_query_starts[0] || (d_hash && d_qoff), SIA_E_INVALID, "NULL input");
+  for (int32_t *o : {out.nres, out.batches, out.exit})
+    if (o) SIA_CUDA(cudaMemsetAsync(o, 0, sizeof(int32_t) * n_queries, s));
+  for (int32_t *o : {out.song, out.diff, out.count, out.rows})
+    SIA_CUDA(cudaMemsetAsync(o, 0, sizeof(int32_t) * (size_t)n_queries * topn, s));
+  QueryPass p;
+  p.s = s;
+  if ((rc = group_tuple_budget(ix, p.budget))) return rc;
+  for (auto &e : ix->ev_q) if (!e) SIA_CUDA(cudaEventCreate(&e));
+  ix->last_lookup_ms = ix->last_vote_ms = 0;
+  for (int64_t q0 = 0; q0 < n_queries; q0 += kMaxQueriesPerPass) {
+    const int nq = (int)std::min<int64_t>(kMaxQueriesPerPass, n_queries - q0);
+    const int64_t i0 = h_query_starts[q0], n = h_query_starts[q0 + nq] - i0;
+    if (h_stats) h_stats[0] += n;
+    if (n == 0) continue;    // the outputs of these queries stay zero
+    if ((rc = ix->arena.reserve((size_t)(nq + 1) * 8 * 3 + (size_t)n * 32 + lookup_bytes(n) + extra_bytes(nq, n) + (1 << 20))))
+      return rc;
+    int64_t *d_qs = ix->arena.take<int64_t>(nq + 1);
+    int64_t *d_goff = ix->arena.take<int64_t>(2 * (size_t)(nq + 1));
+    ulonglong2 *ea = ix->arena.take<ulonglong2>(n), *eb = ix->arena.take<ulonglong2>(n);
+    SIA_REQUIRE(d_qs && d_goff && ea && eb, SIA_E_NOMEM, "index scratch arena too small (query)");
+    SIA_CUDA(cudaMemcpyAsync(d_qs, h_query_starts + q0, sizeof(int64_t) * (nq + 1), cudaMemcpyHostToDevice, s));
+    const auto h0 = std::chrono::steady_clock::now();
+    SIA_CUDA(cudaEventRecord(ix->ev_q[0], s));
+    if ((rc = lookup_queries(ix, d_hash, d_qoff, h_query_starts + q0, d_qs, nq, ea, eb, p.L, s))) return rc;
+    SIA_CUDA(cudaEventRecord(ix->ev_q[1], s));
+    // After the sort query q still owns entries [starts[q]-i0, starts[q+1]-i0) (duplicates stay, with no
+    // postings), so the scanned offsets at those positions split the pass into groups that fit the budget.
+    std::vector<int64_t> h_goff;
+    if ((rc = query_offsets(p.L, d_qs, i0, nq, d_goff, h_goff, s))) return rc;
+    for (int q = 0; q < nq; ++q)
+      SIA_REQUIRE(h_goff[q + 1] - h_goff[q] < (1ll << 31), SIA_E_UNSUPPORTED, "query: more than 2^31 vote tuples in one query");
+    p.q0 = q0; p.i0 = i0; p.n = n; p.nq = nq;
+    p.h_qs = h_query_starts + q0; p.d_qs = d_qs;
+    p.h_off_all = h_goff.data(); p.h_off_head = h_goff.data() + nq + 1; p.d_goff = d_goff;
+    p.groups = 0;
+    if ((rc = vote(p))) return rc;
+    SIA_CUDA(cudaEventRecord(ix->ev_q[2], s));
+    SIA_CUDA(cudaStreamSynchronize(s));
+    float t_lookup = 0, t_vote = 0;
+    cudaEventElapsedTime(&t_lookup, ix->ev_q[0], ix->ev_q[1]); cudaEventElapsedTime(&t_vote, ix->ev_q[1], ix->ev_q[2]);
+    ix->last_lookup_ms += t_lookup; ix->last_vote_ms += t_vote;
+    if (timing) {
+      const double host_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - h0).count();
+      fprintf(stderr, "[sia] query pass: %d queries, %lld entries, %lld tuples, %zu groups: lookup %.2f ms, vote %.2f ms, host wall %.2f ms\n",
+              nq, (long long)n, (long long)p.L.tuples, p.groups, t_lookup, t_vote, host_ms);
+    }
+  }
   return SIA_OK;
 }
 
@@ -1040,72 +1155,25 @@ int sia_index_select_host(sia_index *ix, const uint8_t *h_hash, int64_t n, int32
 int sia_index_query_batch(sia_index *ix, const uint8_t *d_hash, const int32_t *d_qoff, const int64_t *h_query_starts,
                           int32_t n_queries, int32_t topn, int32_t *d_out_song, int32_t *d_out_diff,
                           int32_t *d_out_count, int32_t *d_out_rows, int32_t *d_out_nres, int64_t *h_stats, void *stream) {
-  SIA_REQUIRE(ix && h_query_starts, SIA_E_INVALID, "NULL argument");
-  SIA_REQUIRE(n_queries >= 0 && topn >= 1, SIA_E_INVALID, "n_queries >= 0 and topn >= 1 required");
-  SIA_REQUIRE(ix->n_pending == 0, SIA_E_INVALID, "index has pending rows: call sia_index_finalize first");
-  if (h_stats) h_stats[0] = h_stats[1] = h_stats[2] = h_stats[3] = 0;
-  if (n_queries == 0) return SIA_OK;
-  SIA_REQUIRE(d_out_song && d_out_diff && d_out_count && d_out_rows && d_out_nres, SIA_E_INVALID, "NULL output");
-  int rc = set_device(ix);
-  if (rc) return rc;
-  cudaStream_t s = (cudaStream_t)stream;
-  for (int q = 0; q < n_queries; ++q)
-    SIA_REQUIRE(h_query_starts[q] <= h_query_starts[q + 1], SIA_E_INVALID, "query_starts must be non-decreasing");
-  SIA_REQUIRE(h_query_starts[n_queries] == h_query_starts[0] || (d_hash && d_qoff), SIA_E_INVALID, "NULL input");
-  SIA_CUDA(cudaMemsetAsync(d_out_nres, 0, sizeof(int32_t) * n_queries, s));
-  for (int32_t *o : {d_out_song, d_out_diff, d_out_count, d_out_rows})
-    SIA_CUDA(cudaMemsetAsync(o, 0, sizeof(int32_t) * (size_t)n_queries * topn, s));
-
-  // vote tuples per group of queries (one set of launches per group)
-  int64_t tuple_budget = 0;
-  if ((rc = group_tuple_budget(ix, tuple_budget))) return rc;
+  const QueryOut out{{d_out_song, d_out_diff, d_out_count, d_out_rows, d_out_nres}, nullptr, nullptr};
   const bool timing = getenv("SIA_QUERY_TIMING") != nullptr;       // stage times of every pass on stderr
-  const char *vote_env = getenv("SIA_VOTE");                       // "tables": the table vote for every query (A/B tests)
-  const bool use_pvote = topn <= kPvMaxTopn && !(vote_env && !strcmp(vote_env, "tables"));
-  ix->last_lookup_ms = ix->last_vote_ms = 0;
-  for (auto &e : ix->ev_q) if (!e) SIA_CUDA(cudaEventCreate(&e));
-  static cudaEvent_t stage_ev[9] = {nullptr};          // SIA_QUERY_TIMING only: per-kernel times of the vote
-  double stage_ms[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-  const int64_t span = (int64_t)ix->max_song + 1;
-  for (int64_t q0 = 0; q0 < n_queries; q0 += kMaxQueriesPerPass) {
-    const int nq = (int)std::min<int64_t>(kMaxQueriesPerPass, n_queries - q0);
-    const int64_t i0 = h_query_starts[q0], n = h_query_starts[q0 + nq] - i0;
-    if (h_stats) h_stats[0] += n;
-    if (n == 0) continue;    // out_nres is already 0 for these queries
-    if ((rc = ix->arena.reserve((size_t)(nq + 1) * 8 * 3 + (size_t)n * (32 + 20) + lookup_bytes(n) + (1 << 20)))) return rc;
-    int64_t *d_qs = ix->arena.take<int64_t>(nq + 1);
-    int64_t *d_goff = ix->arena.take<int64_t>(2 * (size_t)(nq + 1));
-    ulonglong2 *ea = ix->arena.take<ulonglong2>(n), *eb = ix->arena.take<ulonglong2>(n);
-    SIA_REQUIRE(d_qs && d_goff && ea && eb, SIA_E_NOMEM, "index scratch arena too small (query)");
-    SIA_CUDA(cudaMemcpyAsync(d_qs, h_query_starts + q0, sizeof(int64_t) * (nq + 1), cudaMemcpyHostToDevice, s));
-    const auto h0 = std::chrono::steady_clock::now();
-    SIA_CUDA(cudaEventRecord(ix->ev_q[0], s));
-    Lookup L;
-    if ((rc = lookup_queries(ix, d_hash, d_qoff, h_query_starts + q0, d_qs, nq, ea, eb, L, s))) return rc;
-    SIA_CUDA(cudaEventRecord(ix->ev_q[1], s));
+  double stage_ms[8] = {0, 0, 0, 0, 0, 0, 0, 0};                   // table vote, summed over the call's groups
+  const auto vote = [&](QueryPass &p) -> int {
+    const int nq = p.nq;
+    const int64_t *h_off_all = p.h_off_all;
+    const Lookup &L = p.L;
+    cudaStream_t s = p.s;
+    StageEvents &tm = ix->ev_stage;
+    tm.on = timing;
     if (h_stats) { h_stats[1] += L.head_rows; h_stats[2] += L.tuples; }
-    // After the sort query q still owns entries [starts[q]-i0, starts[q+1]-i0) (duplicates stay, with no
-    // postings), so the scanned offsets at those positions split the pass into groups that fit the budget.
-    std::vector<int64_t> h_goff;
-    if ((rc = query_offsets(L, d_qs, i0, nq, d_goff, h_goff, s))) return rc;
-    const int64_t *h_off_all = h_goff.data(), *h_off_head = h_goff.data() + nq + 1;
-    std::vector<QMeta> h_meta(nq);
-    auto make_group = [&](int qa, int qb) { return tvote::make_group(qa, qb, h_off_all, h_off_head, span, h_meta.data()); };
-    for (int q = 0; q < nq; ++q)
-      SIA_REQUIRE(h_off_all[q + 1] - h_off_all[q] < (1ll << 31), SIA_E_UNSUPPORTED, "query_batch: more than 2^31 vote tuples in one query");
-    std::vector<Group> groups;               // what the table vote has to do
-    unsigned long long h_nb_total = 0;
-    if (use_pvote) {
+    int rc = SIA_OK;
+    std::vector<std::pair<int, int>> table_groups;    // what the table vote has to do
+    unsigned long long h_nb_pv = 0;
+    if (topn <= kPvMaxTopn) {
       // ---- partitioned vote (index_pvote.cu): shared-memory tables, streaming traffic only --------------------------
-      std::vector<std::pair<int, int>> pg;
+      const auto pg = split_groups(h_off_all, nq, p.budget, nullptr);
       size_t max_bytes = 0;
-      for (int qa = 0; qa < nq;) {
-        int qb = qa + 1;
-        while (qb < nq && h_off_all[qb + 1] - h_off_all[qa] <= tuple_budget) ++qb;
-        pg.emplace_back(qa, qb);
-        max_bytes = std::max(max_bytes, pvote_bytes(h_off_all[qb] - h_off_all[qa], qb - qa, 1, topn));
-        qa = qb;
-      }
+      for (const auto &[qa, qb] : pg) max_bytes = std::max(max_bytes, pvote_bytes(h_off_all[qb] - h_off_all[qa], qb - qa, 1, topn));
       if ((rc = ix->arena3.reserve(max_bytes + (size_t)nq * 8 + 65536))) return rc;
       uint32_t *d_qover = ix->arena3.take<uint32_t>(2 * (size_t)nq), *d_qbins = d_qover + nq;
       unsigned long long *d_nbins = ix->arena3.take<unsigned long long>(1);
@@ -1113,160 +1181,98 @@ int sia_index_query_batch(sia_index *ix, const uint8_t *d_hash, const int32_t *d
       const size_t fixed = ix->arena3.used;
       SIA_CUDA(cudaMemsetAsync(d_qover, 0, sizeof(uint32_t) * 2 * nq, s));
       SIA_CUDA(cudaMemsetAsync(d_nbins, 0, sizeof(unsigned long long), s));
-      const PvOut po{d_out_song, d_out_diff, d_out_count, d_out_rows, d_out_nres};
       double pv_ms[3] = {0, 0, 0};
-      longlong2 *d_info = ix->arena.take<longlong2>(n);
-      uint32_t *d_qh = ix->arena.take<uint32_t>(n);
+      longlong2 *d_info = ix->arena.take<longlong2>(p.n);
+      uint32_t *d_qh = ix->arena.take<uint32_t>(p.n);
       SIA_REQUIRE(d_info && d_qh, SIA_E_NOMEM, "index scratch arena too small (entry info)");
       if ((rc = pvote_entry_info(L, d_info, d_qh, s))) return rc;
-      for (const auto &g : pg) {
-        if (h_off_all[g.second] == h_off_all[g.first]) continue;
+      for (const auto &[qa, qb] : pg) {
         ix->arena3.used = fixed;
-        if ((rc = pvote_entries(ix->arena3, L, d_info, d_qh, ix->post, d_qs, i0, d_goff, h_off_all, g.first, g.second, (int)q0, topn, po, d_qover,
-                                d_qbins, h_stats ? d_nbins : nullptr, s, timing ? pv_ms : nullptr)))
+        if ((rc = pvote_entries(ix->arena3, L, d_info, d_qh, ix->post, p.d_qs, p.i0, p.d_goff, h_off_all, qa, qb, (int)p.q0, topn, out,
+                                d_qover, d_qbins, h_stats ? d_nbins : nullptr, s, tm)))
           return rc;
-        const int64_t e0 = h_query_starts[q0 + g.first] - i0, ne = h_query_starts[q0 + g.second] - i0 - e0;
-        entries_rows_kernel<<<grid_for(ne * 32), 256, 0, s>>>(L.ent, e0, ne, L.first, L.cnt_head, ix->post, (int)q0, topn,
-                                                             d_out_song, d_out_nres, d_out_rows);
+        if (tm.on) for (int k = 0; k < 3; ++k) pv_ms[k] += tm.ms(k, k + 1);
+        const int64_t e0 = p.h_qs[qa] - p.i0, ne = p.h_qs[qb] - p.i0 - e0;
+        entries_rows_kernel<<<grid_for(ne * 32), 256, 0, s>>>(L.ent, e0, ne, L.first, L.cnt_head, ix->post, (int)p.q0, topn,
+                                                             out.song, out.nres, out.rows);
         SIA_CHECK_LAUNCH();
       }
       std::vector<uint32_t> h_qover(nq);
       SIA_CUDA(cudaMemcpyAsync(h_qover.data(), d_qover, sizeof(uint32_t) * nq, cudaMemcpyDeviceToHost, s));
-      SIA_CUDA(cudaMemcpyAsync(&h_nb_total, d_nbins, sizeof h_nb_total, cudaMemcpyDeviceToHost, s));
+      SIA_CUDA(cudaMemcpyAsync(&h_nb_pv, d_nbins, sizeof h_nb_pv, cudaMemcpyDeviceToHost, s));
       SIA_CUDA(cudaStreamSynchronize(s));
       // queries that did not fit their partitions (a bin of thousands of matches, > 2048 partitions): table vote
-      for (int qa = 0; qa < nq;) {
-        if (!h_qover[qa]) { ++qa; continue; }
-        int qb = qa + 1;
-        while (qb < nq && h_qover[qb] && h_off_all[qb + 1] - h_off_all[qa] <= tuple_budget) ++qb;
-        groups.push_back(make_group(qa, qb));
-        qa = qb;
-      }
+      table_groups = split_groups(h_off_all, nq, p.budget, h_qover.data());
       if (timing)
         fprintf(stderr, "[sia]   partitioned vote, %zu group(s): layout %.2f ms, scatter %.2f, count + merge %.2f; %zu group(s) of flagged "
-                "queries go to the table vote\n", pg.size(), pv_ms[0], pv_ms[1], pv_ms[2], groups.size());
+                "queries go to the table vote\n", pg.size(), pv_ms[0], pv_ms[1], pv_ms[2], table_groups.size());
     } else {
-      for (int qa = 0; qa < nq;) {
-        int qb = qa + 1;
-        while (qb < nq && h_off_all[qb + 1] - h_off_all[qa] <= tuple_budget) ++qb;
-        groups.push_back(make_group(qa, qb));
-        qa = qb;
-      }
+      table_groups = split_groups(h_off_all, nq, p.budget, nullptr);
     }
-    int32_t h_flags = 0;
+    std::vector<QMeta> h_meta(nq);
+    std::vector<Group> groups;
+    for (const auto &[qa, qb] : table_groups)
+      groups.push_back(make_group(qa, qb, h_off_all, p.h_off_head, (int64_t)ix->max_song + 1, h_meta.data()));
+    p.groups = groups.size();
     unsigned long long h_nb = 0;
-    // attempt 0 reserves bin slots for a quarter of the tuples being candidates; if pass 1 counts more in some group
-    // (tie-heavy queries) the device flags it and the pass is voted again with room for all of them
-    for (int attempt = 0; attempt < 2 && !groups.empty(); ++attempt) {
+    for (int attempt = 0; !groups.empty(); ++attempt) {
       size_t max_bytes = 0;
-      for (const Group &g : groups)
-        max_bytes = std::max(max_bytes, vote_table_bytes(h_off_all[g.qb] - h_off_all[g.qa], g.qb - g.qa,
-                                                         bin_slots_for(h_off_all[g.qb] - h_off_all[g.qa], g.qb - g.qa, attempt),
-                                                         g.ns, g.dense));
+      for (const Group &g : groups) max_bytes = std::max(max_bytes, table_bytes(g, h_off_all[g.qb] - h_off_all[g.qa], attempt));
       if ((rc = ix->arena3.reserve(max_bytes + (size_t)nq * (sizeof(QMeta) + 4) + 65536))) return rc;
       QMeta *d_meta = ix->arena3.take<QMeta>(nq);
       uint32_t *qflag = ix->arena3.take<uint32_t>(nq);
       int64_t *d_total = ix->arena3.take<int64_t>(1);
       unsigned long long *d_nbins = ix->arena3.take<unsigned long long>(1);
-      int32_t *d_flags = ix->arena3.take<int32_t>(2);     // [0] flags, [1] queries of the group that need the singles pass
-      int32_t *d_nflag = d_flags + 1;
+      int32_t *d_flags = ix->arena3.take<int32_t>(2);
       const size_t fixed = ix->arena3.used;
       SIA_REQUIRE(d_meta && qflag && d_total && d_nbins && d_flags, SIA_E_NOMEM, "index scratch arena too small (vote)");
-      SIA_CUDA(cudaMemcpyAsync(d_meta, h_meta.data(), sizeof(QMeta) * nq, cudaMemcpyHostToDevice, s));
       SIA_CUDA(cudaMemsetAsync(d_nbins, 0, sizeof(unsigned long long), s));
-      SIA_CUDA(cudaMemsetAsync(d_flags, 0, 2 * sizeof(int32_t), s));
+      SIA_CUDA(cudaMemsetAsync(d_flags, 0, sizeof(int32_t), s));
+      const TableVoteArgs a{d_meta, qflag, d_total, d_flags, d_nbins, nullptr, (int)p.q0, topn, out};
       for (const Group &g : groups) {
-        const int64_t e0 = h_query_starts[q0 + g.qa] - i0, ne = h_query_starts[q0 + g.qb] - i0 - e0;
+        const int64_t e0 = p.h_qs[g.qa] - p.i0, ne = p.h_qs[g.qb] - p.i0 - e0;
         const int64_t tuples = h_off_all[g.qb] - h_off_all[g.qa];
-        if (tuples == 0) continue;           // out_nres is already 0 for these queries
         ix->arena3.used = fixed;
-        const int64_t nb_cap = bin_slots_for(tuples, g.qb - g.qa, attempt);
-        Tables Tb;
-        Tb.filter = ix->arena3.take<uint32_t>(g.nf);
-        Tb.song_best = ix->arena3.take<unsigned long long>(g.ns);
-        Tb.song_key = g.dense ? nullptr : ix->arena3.take<uint32_t>(g.ns);
-        Tb.bins = ix->arena3.take<unsigned long long>(nb_cap);
-        Tb.bin_cnt = ix->arena3.take<uint32_t>(nb_cap);
-        Tb.cand = ix->arena3.take<unsigned long long>(nb_cap / 2 + 16);
-        SIA_REQUIRE(Tb.filter && Tb.song_best && Tb.bins && Tb.bin_cnt && Tb.cand && (g.dense || Tb.song_key), SIA_E_NOMEM,
-                    "index scratch arena too small (vote tables)");
-        SIA_CUDA(cudaMemsetAsync(Tb.filter, 0, sizeof(uint32_t) * g.nf, s));
-        SIA_CUDA(cudaMemsetAsync(Tb.song_best, 0, sizeof(unsigned long long) * g.ns, s));
-        if (!g.dense) SIA_CUDA(cudaMemsetAsync(Tb.song_key, 0, sizeof(uint32_t) * g.ns, s));
         const unsigned blocks = (unsigned)ceil_div(tuples, kVoteTuples);
-        const int gq = g.qb - g.qa;
         const int64_t n_pieces = (int64_t)blocks * 8;
         uint32_t *piece_ent = ix->arena3.take<uint32_t>(n_pieces);
         SIA_REQUIRE(piece_ent != nullptr, SIA_E_NOMEM, "index scratch arena too small (vote pieces)");
         piece_entries_kernel<<<grid_for(n_pieces), 256, 0, s>>>(L.off_all, e0, ne, n_pieces, piece_ent);
-#define SIA_ENT_PASS(D, P)                                                                                              \
-        entries_pass_kernel<D, P><<<blocks, 256, 0, s>>>(L.ent, e0, ne, L.first, L.off_all, piece_ent, ix->post, d_meta, Tb,   \
-                                                         qflag, d_nflag, d_nbins, d_flags)
-#define SIA_STAGE(k) do { if (timing) cudaEventRecord(stage_ev[k], s); } while (0)
-#define SIA_ENT_VOTE(D)                                                                                                 \
-        do {                                                                                                            \
-          SIA_STAGE(0);                                                                                                 \
-          SIA_ENT_PASS(D, PASS_MARK);                                                                                   \
-          SIA_STAGE(1);                                                                                                 \
-          layout_bins_kernel<<<1, 1024, 0, s>>>(d_meta, g.qa, g.qb, d_total);                                           \
-          zero_bins_kernel<<<kNumSMs * 8, 256, 0, s>>>(Tb.bins, Tb.bin_cnt, d_total, nb_cap, d_flags);                  \
-          SIA_STAGE(2);                                                                                                 \
-          SIA_ENT_PASS(D, PASS_VOTE);                                                                                   \
-          SIA_STAGE(8);                                                                                                 \
-          cand_vote_kernel<D><<<kNumSMs * 8, 256, 0, s>>>(Tb.cand, d_meta, g.qa, g.qb, Tb, d_nbins, d_flags);           \
-          SIA_STAGE(3);                                                                                                 \
-          topn_kernel<D, false><<<gq, 256, 0, s>>>(Tb, d_meta, g.qa, (int)q0, topn, qflag, d_nflag, nullptr, d_out_song, \
-                                                   d_out_diff, d_out_count, d_out_rows, d_out_nres);                    \
-          SIA_STAGE(4);                                                                                                 \
-          SIA_ENT_PASS(D, PASS_SINGLES);                                                                                \
-          topn_kernel<D, true><<<gq, 256, 0, s>>>(Tb, d_meta, g.qa, (int)q0, topn, qflag, d_nflag, nullptr, d_out_song,  \
-                                                  d_out_diff, d_out_count, d_out_rows, d_out_nres);                     \
-          SIA_STAGE(5);                                                                                                 \
-        } while (0)
-        SIA_CUDA(cudaMemsetAsync(d_nflag, 0, sizeof(int32_t), s));
-        if (timing) { if (!stage_ev[0]) for (auto &e : stage_ev) cudaEventCreate(&e); cudaEventRecord(stage_ev[7], s); }
-        if (g.dense) SIA_ENT_VOTE(true); else SIA_ENT_VOTE(false);
-        entries_rows_kernel<<<grid_for(ne * 32), 256, 0, s>>>(L.ent, e0, ne, L.first, L.cnt_head, ix->post, (int)q0, topn,
-                                                             d_out_song, d_out_nres, d_out_rows);
-        SIA_STAGE(6);
-        if (timing) {
-          cudaEventSynchronize(stage_ev[6]);
-          float t;
-          cudaEventElapsedTime(&t, stage_ev[7], stage_ev[0]); stage_ms[0] += t;      // memsets of the tables
-          for (int k = 0; k < 6; ++k) { cudaEventElapsedTime(&t, stage_ev[k], stage_ev[k + 1]); stage_ms[k + 1] += t; }
-          cudaEventElapsedTime(&t, stage_ev[8], stage_ev[3]); stage_ms[7] += t;        // the dense candidate vote inside "vote"
+        const auto layout = [&]() -> int {
+          SIA_CUDA(cudaMemcpyAsync(d_meta + g.qa, h_meta.data() + g.qa, sizeof(QMeta) * (g.qb - g.qa), cudaMemcpyHostToDevice, s));
+          return SIA_OK;
+        };
+        const auto pass = [&](auto d, auto pt, const Tables &T) {
+          if constexpr (decltype(pt)::value == PASS_ROWS)
+            entries_rows_kernel<<<grid_for(ne * 32), 256, 0, s>>>(L.ent, e0, ne, L.first, L.cnt_head, ix->post, (int)p.q0, topn,
+                                                                 out.song, out.nres, out.rows);
+          else
+            entries_pass_kernel<decltype(d)::value, decltype(pt)::value><<<blocks, 256, 0, s>>>(
+                L.ent, e0, ne, L.first, L.off_all, piece_ent, ix->post, d_meta, T, qflag, d_flags + 1, d_nbins, d_flags);
+        };
+        if ((rc = table_vote(ix->arena3, g, tuples, attempt, a, layout, pass, tm, s))) return rc;
+        if (tm.on) {      // memsets, mark, bin layout + zero, collect + candidate vote, candidate vote, topn, singles + topn, rows
+          const int to[8] = {1, 2, 3, 5, 5, 6, 7, 8};
+          for (int k = 0; k < 8; ++k) stage_ms[k] += tm.ms(k, to[k]);
         }
-#undef SIA_STAGE
-#undef SIA_ENT_VOTE
-#undef SIA_ENT_PASS
-        SIA_CHECK_LAUNCH();
       }
+      int32_t h_flags = 0;
       SIA_CUDA(cudaMemcpyAsync(&h_flags, d_flags, sizeof h_flags, cudaMemcpyDeviceToHost, s));
       SIA_CUDA(cudaMemcpyAsync(&h_nb, d_nbins, sizeof h_nb, cudaMemcpyDeviceToHost, s));
       SIA_CUDA(cudaStreamSynchronize(s));      // the lookup scratch and the tables are reused by the next pass / call
-      SIA_REQUIRE(!(h_flags & 8), SIA_E_CUDA, "query: vote table overflow (internal error)");
-      if (!(h_flags & 32)) break;
-      SIA_REQUIRE(attempt == 0, SIA_E_CUDA, "query: bin table overflow (internal error)");
+      bool retry = false;
+      if ((rc = attempt_retry(h_flags, attempt, "query: vote table overflow (internal error)", retry))) return rc;
+      if (!retry) break;
     }
-    h_nb += h_nb_total;
-    SIA_CUDA(cudaEventRecord(ix->ev_q[2], s));
-    SIA_CUDA(cudaStreamSynchronize(s));
-    {
-      float t_lookup = 0, t_vote = 0;
-      cudaEventElapsedTime(&t_lookup, ix->ev_q[0], ix->ev_q[1]); cudaEventElapsedTime(&t_vote, ix->ev_q[1], ix->ev_q[2]);
-      ix->last_lookup_ms += t_lookup; ix->last_vote_ms += t_vote;
-      if (timing) {
-        const double host_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - h0).count();
-        fprintf(stderr, "[sia] query pass: %d queries, %lld entries, %lld tuples, %zu groups: lookup %.2f ms, vote %.2f ms, host wall %.2f ms\n",
-                nq, (long long)n, (long long)L.tuples, groups.size(), t_lookup, t_vote, host_ms);
-        fprintf(stderr, "[sia]   vote stages (ms): table memsets %.2f, mark %.2f, bin layout + zero %.2f, collect + candidate vote %.2f "
-                "(candidate vote %.2f), topn %.2f, singles + topn %.2f, rows %.2f\n", stage_ms[0], stage_ms[1], stage_ms[2],
-                stage_ms[3], stage_ms[7], stage_ms[4], stage_ms[5], stage_ms[6]);
-      }
-    }
-    if (h_stats) h_stats[3] += (int64_t)h_nb;
-  }
-  return SIA_OK;
+    if (h_stats) h_stats[3] += (int64_t)(h_nb + h_nb_pv);
+    if (timing)
+      fprintf(stderr, "[sia]   vote stages (ms): table memsets %.2f, mark %.2f, bin layout + zero %.2f, collect + candidate vote %.2f "
+              "(candidate vote %.2f), topn %.2f, singles + topn %.2f, rows %.2f\n", stage_ms[0], stage_ms[1], stage_ms[2],
+              stage_ms[3], stage_ms[4], stage_ms[5], stage_ms[6], stage_ms[7]);
+    return SIA_OK;
+  };
+  return query_passes(ix, d_hash, d_qoff, h_query_starts, n_queries, topn, out, h_stats, (cudaStream_t)stream, timing,
+                      [](int, int64_t n) { return (size_t)n * 20; }, vote);   // the partitioned vote's entry info
 }
 
 int sia_index_query_timing(const sia_index *ix, double *h_ms2) {

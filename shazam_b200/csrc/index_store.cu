@@ -439,6 +439,7 @@ int sia_index_destroy(sia_index *ix) {
   if (ix->stage) cudaFree(ix->stage);
   if (ix->insert_done) cudaEventDestroy(ix->insert_done);
   for (cudaEvent_t e : ix->ev_q) if (e) cudaEventDestroy(e);
+  ix->ev_stage.release();
   ix->arena.release();
   ix->arena3.release();
   delete ix;

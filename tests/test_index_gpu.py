@@ -641,7 +641,7 @@ def test_vote_large_table_vs_oracle(gpudb, monkeypatch, id_stride, off_range):
         out = ix.query_batch(qd, qo, qs, topn, want_stats=True)
         return [t.cpu().numpy() for t in out[:5]], out[5]
 
-    for topn in (1, 3, 9):
+    for topn in (1, 3, 9, 40):                          # 40 > kPvMaxTopn: the table vote for every query
         want = _np_vote(t_q, t_song, t_diff, head, nq, topn)
         assert want[4].max() == topn
         assert want[2][70, 0] == n_big and want[0][70, 0] == (nsongs + 1) * id_stride and want[1][70, 0] == 16
@@ -652,11 +652,11 @@ def test_vote_large_table_vs_oracle(gpudb, monkeypatch, id_stride, off_range):
             assert [tuple(b) for b in best] == [(int(want[0][q, r]), int(want[1][q, r]), int(want[2][q, r])) for r in range(want[4][q])]
             assert [dd[b[0]] for b in best] == [int(want[3][q, r]) for r in range(want[4][q])]
         # default = the partitioned vote (shared-memory tables; query 70's bin of 33000 matches does not fit a region and
-        # goes to the table vote); SIA_PVOTE_CAP: small regions, so that most queries are split or handed over;
-        # SIA_VOTE=tables: the table vote for every query
-        names = ("SIA_VOTE_GROUP_TUPLES", "SIA_PVOTE_CAP", "SIA_VOTE")
-        for setting in ((None, None, None), ("1000", None, None), ("200000", None, None), (str(1 << 40), None, None),
-                        (None, "64", None), ("200000", "1024", None), (None, None, "tables"), ("200000", None, "tables")):
+        # goes to the table vote); SIA_PVOTE_CAP: small regions, so that most queries are split or handed over; regions
+        # of 2 tuples overflow for almost every query, which then goes to the table vote
+        names = ("SIA_VOTE_GROUP_TUPLES", "SIA_PVOTE_CAP")
+        for setting in ((None, None), ("1000", None), ("200000", None), (str(1 << 40), None),
+                        (None, "64"), ("200000", "1024"), (None, "2"), ("200000", "2")):
             for name, val in zip(names, setting):
                 if val is None:
                     monkeypatch.delenv(name, raising=False)
