@@ -71,7 +71,12 @@ int sia_version(void);
 typedef struct sia_fp_params {
   double  Fs;            /* sampling rate; enters only as the 1/Fs PSD scale */
   int32_t wsize;         /* must be 4096 */
-  double  wratio;        /* must be 0.5 */
+  double  wratio;        /* DEFAULT_OVERLAP_RATIO 0.5: noverlap = (int32_t)(4096.0 * wratio) (Python's
+                          * int(wsize * wratio)) must be 0..4095; frame k of a track starts at sample k * hop,
+                          * hop = 4096 - noverlap.  noverlap >= 4096 or NaN: SIA_E_INVALID; noverlap < 0:
+                          * SIA_E_UNSUPPORTED.  Peak times, t1 and dt <= MAX_HASH_TIME_DELTA count frames of this hop:
+                          * an index is built and queried at one wratio.  Offsets stored in an index are < 2^24, so
+                          * a track inserted there has at most 2^24 frames (2^24 * hop samples; ~380 s at hop 1). */
   int32_t fan_value;     /* DEFAULT_FAN_VALUE 5; partners per peak = fan_value-1; <= 64 */
   double  amp_min;       /* DEFAULT_AMP_MIN 10 (dB); negative values enable the erosion term */
   int32_t connectivity;  /* CONNECTIVITY_MASK: 2 = square (reference default), 1 = diamond */
@@ -95,6 +100,9 @@ int sia_ctx_digest_table(sia_ctx *ctx, int enable);
 
 /* frames mlab.specgram yields for a track of n samples (short input -> 1 padded frame) */
 int64_t sia_num_frames(int64_t n_samples);
+/* the same at the hop of p: 1 + (max(n, 4096) - 4096) / hop; <0 (SIA_E_*, sia_last_error) if p is rejected or
+ * n_samples < 0.  Host only: needs no device. */
+int64_t sia_fp_frames(const sia_fp_params *p, int64_t n_samples);
 
 /* De-interleave decoded PCM on the device — the `data[chn::n_channels]` of read(), __init__.py:91-95:
  * d_out[c * channel_stride + i] = d_in[i * n_channels + c] for i < n_frames, c < n_channels.  channel_stride >=
@@ -170,7 +178,7 @@ int sia_ctx_timing(sia_ctx *ctx, int enable, double *h_ms_out, int32_t *h_launch
  * The handle keeps per-stream state in HBM (allocated at create, two copies: ~2 * (8 KB + nbhd * 16.6 KB) per stream,
  * plus one max_chunk_frames spectrogram for new rows) and uses its context's workspaces: calls on a context and its
  * stream handles must be serialised by the caller, and stream handles are destroyed before their context.
- * Parameters as sia_fingerprint_batch (wsize 4096, wratio 0.5 only). */
+ * Parameters as sia_fingerprint_batch (wsize 4096 only). */
 typedef struct sia_stream sia_stream;
 int sia_stream_create(sia_ctx *ctx, int32_t n_streams, const sia_fp_params *p, sia_stream **out);
 int sia_stream_destroy(sia_stream *st);

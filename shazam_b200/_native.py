@@ -47,6 +47,7 @@ SIGNATURES = {
     "sia_ctx_destroy": (C.c_int, [_p]),
     "sia_ctx_digest_table": (C.c_int, [_p, C.c_int]),
     "sia_num_frames": (C.c_int64, [C.c_int64]),
+    "sia_fp_frames": (C.c_int64, [C.POINTER(FpParams), C.c_int64]),
     "sia_deinterleave_i16": (C.c_int, [_p, C.c_int64, C.c_int32, _p, C.c_int64, _p]),
     "sia_stft_db": (C.c_int, [_p, _p, _i64p, _i64p, C.c_int32, C.POINTER(FpParams), _p, C.c_int32, _i64p, _p]),
     "sia_peaks": (C.c_int, [_p, _p, C.c_int32, _i64p, C.c_int32, C.POINTER(FpParams), _p, _p, C.c_int64, _p, _p, _p]),
@@ -127,6 +128,16 @@ def default_params() -> FpParams:
     return p
 
 
-def num_frames(n_samples: int) -> int:
+def hop_of(p: FpParams) -> int:
+    """Samples between frame starts: ``wsize - int(wsize * wratio)`` (``__init__.py:235``, ``noverlap``).
+    Parameters the library rejects raise its error here."""
+    rc = lib().sia_fp_frames(C.byref(p), 0)
+    if rc < 0:
+        check(rc)
+    return int(p.wsize) - int(p.wsize * p.wratio)
+
+
+def num_frames(n_samples: int, hop: int = HOP) -> int:
+    """Frames of a track of ``n_samples`` at ``hop`` (mlab.specgram: a short input is one zero-padded frame)."""
     n = max(int(n_samples), NFFT)
-    return (n - HOP) // HOP
+    return 1 + (n - NFFT) // int(hop)

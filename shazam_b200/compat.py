@@ -53,16 +53,14 @@ def fingerprint(channel_samples, Fs: int = RATE, wsize: int = DEFAULT_WINDOW_SIZ
                 wratio: float = DEFAULT_OVERLAP_RATIO, fan_value: int = DEFAULT_FAN_VALUE,
                 amp_min: int = DEFAULT_AMP_MIN):
     """``__init__.py:212-245``: FFT the channel, log transform, local maxima, hashes.
-    Returns ``[(hex20, t1), ...]`` in the reference's order."""
+    Returns ``[(hex20, t1), ...]`` in the reference's order.  Any ``wratio`` with
+    ``0 <= int(4096 * wratio) <= 4095``; ``t1`` counts frames of that overlap."""
+    if wsize != DEFAULT_WINDOW_SIZE:
+        raise N.SiaError(N.E_UNSUPPORTED, f"only wsize=4096 is implemented (got {wsize})")
     fp = get_fingerprinter()
     batch = fp.fingerprint_tracks([as_pcm_int16(channel_samples)], Fs=Fs, fan_value=fan_value, amp_min=amp_min,
-                                  connectivity=CONNECTIVITY_MASK, nbhd=PEAK_NEIGHBORHOOD_SIZE) \
-        if (wsize == DEFAULT_WINDOW_SIZE and wratio == DEFAULT_OVERLAP_RATIO) else _unsupported(wsize, wratio)
+                                  connectivity=CONNECTIVITY_MASK, nbhd=PEAK_NEIGHBORHOOD_SIZE, wratio=wratio)
     return list(zip(digests_to_hex(batch.hash), batch.t1.tolist()))
-
-
-def _unsupported(wsize, wratio):
-    raise N.SiaError(N.E_UNSUPPORTED, f"only wsize=4096, wratio=0.5 are implemented (got {wsize}, {wratio})")
 
 
 def get_2D_peaks(arr2D, plot: bool = False, amp_min=DEFAULT_AMP_MIN):

@@ -31,7 +31,12 @@ namespace sia {
 int check_params(const sia_fp_params *p) {
   SIA_REQUIRE(p != nullptr, SIA_E_INVALID, "params is NULL");
   SIA_REQUIRE(p->wsize == SIA_NFFT, SIA_E_UNSUPPORTED, "only wsize=4096 (DEFAULT_WINDOW_SIZE) is implemented");
-  SIA_REQUIRE(p->wratio == 0.5, SIA_E_UNSUPPORTED, "only wratio=0.5 (DEFAULT_OVERLAP_RATIO) is implemented");
+  // noverlap = int(4096 * wratio) must be 0..4095; tested on the product before the conversion to an integer
+  const double noverlap = SIA_NFFT * p->wratio;
+  SIA_REQUIRE(!(noverlap != noverlap) && noverlap < SIA_NFFT, SIA_E_INVALID,
+              "wratio must give noverlap = int(4096 * wratio) <= 4095 (a hop of at least one sample)");
+  SIA_REQUIRE(noverlap > -1.0, SIA_E_UNSUPPORTED,
+              "wratio < 0 (noverlap < 0: gaps between frames) is not implemented");
   SIA_REQUIRE(p->Fs > 0, SIA_E_INVALID, "Fs must be positive");
   SIA_REQUIRE(p->fan_value >= 1 && p->fan_value <= 64, SIA_E_INVALID, "fan_value must be in 1..64");
   SIA_REQUIRE(p->connectivity == 1 || p->connectivity == 2, SIA_E_INVALID, "connectivity must be 1 or 2");
@@ -97,7 +102,8 @@ struct MetaView {
 
 // max_samples > 0 additionally bounds the (8-sample padded) PCM of a chunk — the staging buffer of the
 // host pipeline.
-int plan_chunks(sia_ctx *c, const int64_t *h_len, int n_tracks, int64_t max_samples, std::vector<Chunk> &chunks) {
+int plan_chunks(sia_ctx *c, const sia_fp_params *p, const int64_t *h_len, int n_tracks, int64_t max_samples,
+                std::vector<Chunk> &chunks) {
   chunks.clear();
   size_t meta = 0;
   int b = 0;
@@ -105,7 +111,7 @@ int plan_chunks(sia_ctx *c, const int64_t *h_len, int n_tracks, int64_t max_samp
     Chunk ch{b, b, 0, 0, meta};
     int64_t samples = 0;
     while (ch.b1 < n_tracks) {
-      const int64_t fr = sia_num_frames(h_len[ch.b1]);
+      const int64_t fr = fp_frames(p, h_len[ch.b1]);
       if (fr > c->max_frames) {
         char buf[256];
         snprintf(buf, sizeof buf, "track %d has %lld frames; the context workspace holds %lld (raise max_chunk_frames, "
@@ -131,7 +137,8 @@ int plan_chunks(sia_ctx *c, const int64_t *h_len, int n_tracks, int64_t max_samp
 
 // Fill the host copy of every chunk's metadata.  dev_starts[b] = sample offset of track b inside the
 // device PCM buffer the chunk's kernels will read.
-void fill_meta(const std::vector<Chunk> &chunks, const int64_t *dev_starts, const int64_t *h_len, int64_t *h_meta) {
+void fill_meta(const std::vector<Chunk> &chunks, const sia_fp_params *p, const int64_t *dev_starts, const int64_t *h_len,
+               int64_t *h_meta) {
   for (const Chunk &ch : chunks) {
     const int nb = ch.b1 - ch.b0;
     MetaView m(h_meta + ch.meta_off, nb);
@@ -141,7 +148,7 @@ void fill_meta(const std::vector<Chunk> &chunks, const int64_t *dev_starts, cons
       m.track_len[i] = h_len[ch.b0 + i];
       m.frame_starts[i] = fr;
       m.ttile_starts[i] = tt;
-      const int64_t f = sia_num_frames(h_len[ch.b0 + i]);
+      const int64_t f = fp_frames(p, h_len[ch.b0 + i]);
       fr += f;
       tt += ceil_div(f, kPeakTileT);
     }
@@ -159,7 +166,7 @@ int run_stft(sia_ctx *c, const int16_t *d_pcm, const MetaView &m, int nb, int64_
   a.d_pcm = d_pcm; a.d_track_starts = m.track_starts; a.d_track_len = m.track_len; a.d_frame_starts = m.frame_starts;
   a.n_tracks = nb; a.total_frames = frames; a.d_spec = d_spec; a.out_type = out_type;
   a.frames_per_cta = 8;      // frames per CTA run (K1's PCM cursor keeps a clamped 32-bit remainder: runs stay short)
-  a.compute = p->compute; a.Fs = p->Fs;
+  a.compute = p->compute; a.Fs = p->Fs; a.hop = fp_hop(p);
   Timer t(c, s, T_STFT, 1);
   return stft_db_launch(a, c->tf, c->td, s);
 }
@@ -315,6 +322,13 @@ int64_t sia_num_frames(int64_t n_samples) {
   return (n - SIA_HOP) / SIA_HOP;
 }
 
+int64_t sia_fp_frames(const sia_fp_params *p, int64_t n_samples) {
+  int rc = check_params(p);
+  if (rc) return rc;
+  SIA_REQUIRE(n_samples >= 0, SIA_E_INVALID, "negative track length");
+  return fp_frames(p, n_samples);
+}
+
 int sia_ctx_create(int device, int64_t max_chunk_frames, sia_ctx **out) {
   SIA_REQUIRE(out != nullptr, SIA_E_INVALID, "out is NULL");
   *out = nullptr;
@@ -424,9 +438,9 @@ int sia_stft_db(sia_ctx *c, const int16_t *d_pcm, const int64_t *h_track_starts,
   for (int b = 0; b < n_tracks; ++b) {
     SIA_REQUIRE(h_track_starts[b] % 8 == 0, SIA_E_INVALID, "track_starts must be multiples of 8 samples");
     SIA_REQUIRE(h_track_len[b] >= 0, SIA_E_INVALID, "negative track length");
-    one[0].frames += sia_num_frames(h_track_len[b]);
+    one[0].frames += fp_frames(p, h_track_len[b]);
   }
-  fill_meta(one, h_track_starts, h_track_len, h.data());
+  fill_meta(one, p, h_track_starts, h_track_len, h.data());
   if ((rc = ensure_meta(c, h.size()))) return rc;
   SIA_CUDA(cudaMemcpyAsync(c->d_meta, h.data(), h.size() * sizeof(int64_t), cudaMemcpyHostToDevice, s));
   SIA_CUDA(cudaStreamSynchronize(s));   // h is a stack-lifetime buffer
@@ -499,12 +513,12 @@ int sia_fingerprint_batch(sia_ctx *c, const int16_t *d_pcm, const int64_t *h_tra
     SIA_REQUIRE(h_track_len[b] >= 0, SIA_E_INVALID, "negative track length");
   }
   std::vector<Chunk> chunks;
-  if ((rc = plan_chunks(c, h_track_len, n_tracks, 0, chunks))) return rc;
+  if ((rc = plan_chunks(c, p, h_track_len, n_tracks, 0, chunks))) return rc;
   size_t meta_total = 0;
   for (auto &ch : chunks) meta_total += MetaView::size(ch.b1 - ch.b0);
   if ((rc = ensure_meta(c, meta_total))) return rc;
   if ((rc = ensure_pinned(c, meta_total + 8))) return rc;
-  fill_meta(chunks, h_track_starts, h_track_len, c->h_pinned);
+  fill_meta(chunks, p, h_track_starts, h_track_len, c->h_pinned);
   SIA_CUDA(cudaMemcpyAsync(c->d_meta, c->h_pinned, meta_total * sizeof(int64_t), cudaMemcpyHostToDevice, s));
   SIA_CUDA(cudaMemsetAsync(c->status, 0, sizeof(int32_t), s));
   SIA_CUDA(cudaMemsetAsync(c->hash_base, 0, sizeof(int64_t), s));
@@ -555,11 +569,20 @@ int sia_fingerprint_batch_host(sia_ctx *c, const int16_t *h_pcm, const int64_t *
     SIA_CUDA(cudaStreamCreateWithFlags(&c->s_comp, cudaStreamNonBlocking));
     SIA_CUDA(cudaStreamCreateWithFlags(&c->s_d2h, cudaStreamNonBlocking));
   }
-  if (!c->pcm_stage[0]) {
-    // the longest admissible track has (max_frames+1)*2048 + 2047 samples; plan_chunks keeps chunks inside
-    c->pcm_stage_samples = (c->max_frames + 4) * (int64_t)SIA_HOP;
+  // The longest admissible track (max_frames frames at hop h) has (max_frames-1)*h + 4095 + h samples, 8-sample padded
+  // + 8 in the staging buffer; plan_chunks keeps chunks inside.  Sized for hop 2048 at first, grown for a longer hop.
+  const int64_t stage_need = (c->max_frames + 1) * (int64_t)std::max(fp_hop(p), SIA_HOP) + 3 * SIA_HOP;
+  if (c->pcm_stage_samples < stage_need) {
     for (int i = 0; i < 2; ++i) {
-      SIA_CUDA(cudaMalloc(&c->pcm_stage[i], (size_t)c->pcm_stage_samples * sizeof(int16_t)));
+      if (c->pcm_stage[i]) cudaFree(c->pcm_stage[i]);
+      c->pcm_stage[i] = nullptr;
+    }
+    c->pcm_stage_samples = 0;
+    for (int i = 0; i < 2; ++i) SIA_CUDA(cudaMalloc(&c->pcm_stage[i], (size_t)stage_need * sizeof(int16_t)));
+    c->pcm_stage_samples = stage_need;
+  }
+  if (!c->hash_stage[0]) {
+    for (int i = 0; i < 2; ++i) {
       SIA_CUDA(cudaMalloc(&c->hash_stage[i], (size_t)c->cap_chunk_hashes * SIA_HASH_BYTES));
       SIA_CUDA(cudaMalloc(&c->t1_stage[i], (size_t)c->cap_chunk_hashes * sizeof(int32_t)));
     }
@@ -567,7 +590,7 @@ int sia_fingerprint_batch_host(sia_ctx *c, const int16_t *h_pcm, const int64_t *
   for (int b = 0; b < n_tracks; ++b) SIA_REQUIRE(h_track_len[b] >= 0, SIA_E_INVALID, "negative track length");
 
   std::vector<Chunk> chunks;
-  if ((rc = plan_chunks(c, h_track_len, n_tracks, c->pcm_stage_samples, chunks))) return rc;
+  if ((rc = plan_chunks(c, p, h_track_len, n_tracks, c->pcm_stage_samples, chunks))) return rc;
   const int nchunks = (int)chunks.size();
   size_t meta_total = 0;
   for (auto &ch : chunks) meta_total += MetaView::size(ch.b1 - ch.b0);
@@ -607,7 +630,7 @@ int sia_fingerprint_batch_host(sia_ctx *c, const int16_t *h_pcm, const int64_t *
   int64_t *h_meta_out = c->h_pinned + meta_total;   // per-chunk readback of track_hash_starts etc.
   int64_t *h_counts = h_meta_out + meta_total;      // [nchunks] hashes per chunk
   int32_t *h_status = reinterpret_cast<int32_t *>(h_counts + nchunks);
-  fill_meta(chunks, dev_start.data(), h_track_len, h_meta_in);
+  fill_meta(chunks, p, dev_start.data(), h_track_len, h_meta_in);
   SIA_CUDA(cudaMemcpyAsync(c->d_meta, h_meta_in, meta_total * sizeof(int64_t), cudaMemcpyHostToDevice, c->s_comp));
   SIA_CUDA(cudaMemsetAsync(c->status, 0, sizeof(int32_t), c->s_comp));
 

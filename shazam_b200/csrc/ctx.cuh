@@ -73,6 +73,13 @@ struct Timer {
 };
 
 int check_params(const sia_fp_params *p);
+// Frame geometry of parameters that passed check_params: noverlap = int(wsize * wratio) (truncated, like Python's
+// int()), frame k of a track starts at sample k * hop, and a track of n samples has 1 + (max(n, 4096) - 4096) / hop
+// frames (mlab.specgram: a short input is zero-padded to one frame, a trailing partial frame is dropped).
+inline int fp_hop(const sia_fp_params *p) { return SIA_NFFT - (int32_t)(SIA_NFFT * p->wratio); }
+inline int64_t fp_frames(const sia_fp_params *p, int64_t n_samples) {
+  return 1 + ((n_samples < SIA_NFFT ? SIA_NFFT : n_samples) - SIA_NFFT) / fp_hop(p);
+}
 int ensure_meta(sia_ctx *c, size_t n_i64);     // d_meta holds at least n_i64 int64
 int ensure_pinned(sia_ctx *c, size_t n_i64);   // h_pinned holds at least n_i64 int64
 

@@ -1,5 +1,6 @@
 // K1 — batched 4096-point STFT -> dB spectrogram, replacing
 //   mlab.specgram(x, NFFT=4096, Fs, window_hanning, noverlap=2048)[0]   (__init__.py:232-237)
+//   (any noverlap 0..4095 through the kAnyHop staging below; 2048 = wratio 0.5 is the tuned path)
 //   10*log10(P) with P==0 -> 0                                           (__init__.py:241)
 //
 // One CTA (128 threads) transforms one frame at a time and walks a run of consecutive
@@ -222,13 +223,24 @@ __device__ __forceinline__ void emit_special(OutT *__restrict__ row, const T *__
   emit_pair<T, OutT>(row, pr[a], pi[a], pr[b], pi[b], tw.x, tw.y, k, k == 0 ? sc_edge : sc_mid);
 }
 
-template <typename T, typename OutT>
+// PCM ring of the any-hop staging (kAnyHop): 513 16-byte chunks = 4104 samples, one chunk more than a frame, because
+// a frame that starts off an 8-sample boundary touches 513 chunks.  Chunk c of a track (samples [8c, 8c+8)) lives in
+// slot c mod 513, so sample n of the track is ring word (n/2) mod 2052.  Word 2052 mirrors word 0, so the word after
+// any ring word is read without a wrap test.
+constexpr int kRingChunks = 513;
+constexpr int kRingSamples = 8 * kRingChunks;
+constexpr int kRingWords = kRingSamples / 2;
+
+// kAnyHop = false: frame k of a track starts at sample 2048 k (wratio 0.5), staged in two half-blocks.
+// kAnyHop = true:  frame k starts at sample k * hop, hop in 1..4096, staged in the 513-chunk ring above.
+// Passes A-C and the dB epilogue are shared: a frame gives the same bits whatever the hop.
+template <typename T, typename OutT, bool kAnyHop>
 __global__ void __launch_bounds__(128, sizeof(T) == 8 ? kStftCtasF64 : 6)
 stft_db_kernel(const int16_t *__restrict__ pcm, const int64_t *__restrict__ track_starts,
                const int64_t *__restrict__ track_len, const int64_t *__restrict__ frame_starts, int n_tracks,
                int64_t total_frames, int frames_per_cta, OutT *__restrict__ out, DbScale sc_mid, DbScale sc_edge,
                const typename Vec2<T>::type *__restrict__ winB, const typename Vec2<T>::type *__restrict__ twA,
-               const typename Vec2<T>::type *__restrict__ twB, const typename Vec2<T>::type *__restrict__ twP) {
+               const typename Vec2<T>::type *__restrict__ twB, const typename Vec2<T>::type *__restrict__ twP, int hop) {
   using V2 = typename Vec2<T>::type;
   __shared__ __align__(16) V2 sbuf[kBufElems];      // (re, im) interleaved: one 128-bit (64-bit) access per element
   constexpr int kL2Stride = sizeof(T) == 8 ? 257 : 258;
@@ -238,7 +250,9 @@ stft_db_kernel(const int16_t *__restrict__ pcm, const int64_t *__restrict__ trac
   // cp.async into the slot of half-block k while passes B and C run, so the DRAM latency of the PCM never sits
   // in front of pass A.  Bytes past the end of a track are zero-filled (src-size), which is exactly
   // mlab.specgram's zero padding of a short input.
-  __shared__ __align__(16) uint32_t spcm[2][1024];
+  // kAnyHop: the same schedule on the 513-chunk ring (kRingWords + 1 words used): after pass A of frame k, the
+  // chunks frame k+1 adds are fetched into the slots of chunks no later frame reads.
+  __shared__ __align__(16) uint32_t spcm[2][kAnyHop ? 1028 : 1024];
   __shared__ T sspc[2][2][16];     // parked columns 0 / 128 of the last two frames (re, im)
 
   const int t = threadIdx.x;
@@ -272,6 +286,44 @@ stft_db_kernel(const int16_t *__restrict__ pcm, const int64_t *__restrict__ trac
   int slot = 0;
   bool primed = false;
 
+  // kAnyHop: the ring holds the track's samples up to fe, a multiple of 8; cur_src / cur_rest are the track's PCM and
+  // bytes left from fe on.  For the current frame, starting at sample s: s_mod = s mod kRingSamples, lead = fe - s
+  // (-7..4103).  kRingSamples is a multiple of 8, so s and s_mod share their residue mod 8.
+  int s_mod = 0, lead = 0;
+  auto set_ring = [&](int tr, int64_t k) {
+    const int64_t s = k * hop, fe = s & ~(int64_t)7;
+    s_mod = (int)(s % kRingSamples);
+    lead = (int)(fe - s);
+    const int64_t rest = (track_len[tr] - fe) * 2;
+    cur_rest = (int)max(min(rest, (int64_t)1 << 30), -((int64_t)1 << 30));
+    cur_src = reinterpret_cast<const char *>(pcm + track_starts[tr] + fe);
+  };
+  auto fetch_frame = [&]() {      // the chunks from fe up to the end of the current frame: at most kRingChunks
+    const int n = (SIA_NFFT - lead + 7) >> 3;
+    int fe_mod = s_mod + lead;
+    if (fe_mod < 0) fe_mod += kRingSamples;
+    if (fe_mod >= kRingSamples) fe_mod -= kRingSamples;
+    for (int i = t; i < n; i += 128) {
+      int pos = fe_mod + 8 * i;
+      if (pos >= kRingSamples) pos -= kRingSamples;
+      const int nbytes = min(max(cur_rest - 16 * i, 0), 16);
+      const char *src = nbytes ? cur_src + 16 * i : reinterpret_cast<const char *>(pcm);
+      asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n" ::"r"(spcm_base + 2 * (uint32_t)pos), "l"(src),
+                   "r"(nbytes));
+      if (pos == 0)      // the mirror word behind the ring
+        asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;\n" ::"r"(spcm_base + 4 * (uint32_t)kRingWords),
+                     "l"(src), "r"(min(nbytes, 4)));
+    }
+    lead += 8 * n;
+    cur_src += 16 * n;
+    cur_rest -= 16 * n;
+  };
+  auto next_frame = [&]() {
+    s_mod += hop;
+    if (s_mod >= kRingSamples) s_mod -= kRingSamples;
+    lead -= hop;
+  };
+
   const int64_t g_first = g;
   for (; g < g_end; ++g) {
     // lanes 1..9: finish the previous frame (its parked columns became visible at the barrier)
@@ -281,21 +333,40 @@ stft_db_kernel(const int16_t *__restrict__ pcm, const int64_t *__restrict__ trac
     while (g >= frame_starts[trk + 1]) ++trk;
     const int64_t k = g - frame_starts[trk];
     if (!primed) {                       // first frame of the run or of a track: both half-blocks, synchronously
-      set_cursor(trk, k);
-      fetch_half(slot);
-      fetch_half(slot ^ 1);
+      if constexpr (kAnyHop) {
+        set_ring(trk, k);
+        fetch_frame();
+      } else {
+        set_cursor(trk, k);
+        fetch_half(slot);
+        fetch_half(slot ^ 1);
+      }
       asm volatile("cp.async.wait_all;\n" ::: "memory");
       __syncthreads();
     }
     primed = g + 1 < frame_starts[trk + 1];           // the next frame continues this track
-    const uint32_t *__restrict__ h0 = spcm[slot], *__restrict__ h1 = spcm[slot ^ 1];
 
     T xr[16], xi[16];
     // ---- pass A: window, pack even/odd samples as complex, FFT16 over a -----------------
     {
       uint32_t w[16];
+      if constexpr (kAnyHop) {
+        // samples s + 256a + 2t, +1: ring words j, j+1 shifted right by 16 bits when s is odd
+        const uint32_t *__restrict__ ring = &spcm[0][0];
+        const int sh = (s_mod & 1) << 4;
+        int j = (s_mod >> 1) + t;
+        if (j >= kRingWords) j -= kRingWords;
 #pragma unroll
-      for (int a = 0; a < 8; ++a) { w[a] = h0[128 * a + t]; w[a + 8] = h1[128 * a + t]; }
+        for (int a = 0; a < 16; ++a) {
+          w[a] = __funnelshift_r(ring[j], ring[j + 1], sh);
+          j += 128;
+          if (j >= kRingWords) j -= kRingWords;
+        }
+      } else {
+        const uint32_t *__restrict__ h0 = spcm[slot], *__restrict__ h1 = spcm[slot ^ 1];
+#pragma unroll
+        for (int a = 0; a < 8; ++a) { w[a] = h0[128 * a + t]; w[a + 8] = h1[128 * a + t]; }
+      }
       const V2 wb0 = __ldg(winB + 2 * t), wb1 = __ldg(winB + 2 * t + 1);   // window phase of samples 2t, 2t+1
       // np.hanning: w[m] = 0.5 - 0.5*cos(2*pi*m/4095), m = 256a + 2t (+1).  cos(a*D + B_t), D = 2*pi*256/4095, by the
       // three-term recurrence c[a+1] = 2cos(D) c[a] - c[a-1]: one FMA per sample (16 steps: error growth ~1e-15)
@@ -351,7 +422,10 @@ stft_db_kernel(const int16_t *__restrict__ pcm, const int64_t *__restrict__ trac
 #endif
     }
     __syncthreads();
-    if (primed && g + 1 < g_end) fetch_half(slot);                 // half-block k+2; pass A has consumed this slot
+    if (primed && g + 1 < g_end) {
+      if constexpr (kAnyHop) { next_frame(); fetch_frame(); }     // what frame k+1 adds; pass A is done with frame k
+      else fetch_half(slot);                                       // half-block k+2; pass A has consumed this slot
+    }
     // ---- pass B: FFT16 over b -----------------------------------------------------------
     {
       const int ka = t >> 3, c = t & 7;
@@ -538,10 +612,11 @@ static int launch(const StftLaunch &a, const StftTables<T> &tb, cudaStream_t s) 
   // 80 % of the SM's 228 KB L1/shared storage as shared memory = 182 KB: room for the 4 resident CTAs (4 x 44.5 KB) and
   // ~70 KB of L1 for the twiddle / window tables, which the maximum carveout squeezes out (measured 38.3 ms at 100 %,
   // 36.5 ms at 80 %)
-  SIA_CUDA(cudaFuncSetAttribute(stft_db_kernel<T, OutT>, cudaFuncAttributePreferredSharedMemoryCarveout, 80));
-  stft_db_kernel<T, OutT><<<(unsigned)blocks, 128, 0, s>>>(
+  auto kernel = a.hop == SIA_HOP ? stft_db_kernel<T, OutT, false> : stft_db_kernel<T, OutT, true>;
+  SIA_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 80));
+  kernel<<<(unsigned)blocks, 128, 0, s>>>(
       a.d_pcm, a.d_track_starts, a.d_track_len, a.d_frame_starts, a.n_tracks, a.total_frames, G, (OutT *)a.d_spec,
-      sc_mid, sc_edge, (const V2 *)tb.win2, (const V2 *)tb.twA, (const V2 *)tb.twB, (const V2 *)tb.twP);
+      sc_mid, sc_edge, (const V2 *)tb.win2, (const V2 *)tb.twA, (const V2 *)tb.twB, (const V2 *)tb.twP, a.hop);
   SIA_CHECK_LAUNCH();
   return SIA_OK;
 }

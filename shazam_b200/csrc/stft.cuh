@@ -25,6 +25,7 @@ struct StftLaunch {
   int out_type;   // SIA_F32 / SIA_F64
   int compute;    // SIA_F32 / SIA_F64
   double Fs;
+  int hop;        // frame k of a track starts at sample k * hop, 1..4096 (SIA_HOP: the half-block staging)
 };
 
 int stft_tables_create(StftTables<float> &f, StftTables<double> &d);

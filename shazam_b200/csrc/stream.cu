@@ -34,7 +34,7 @@ constexpr int kRowVec = SIA_F_STRIDE / 4;   // float4 per spectrogram row
 constexpr int kTailCap = SIA_NFFT;          // tail slot (samples) per stream
 constexpr int kPeakCap = 64;                // peak slots per stream (fan_value - 1 <= 63 are carried)
 
-inline int64_t complete_frames(int64_t n) { return n >= SIA_NFFT ? 1 + (n - SIA_NFFT) / SIA_HOP : 0; }
+inline int64_t complete_frames(int64_t n, int hop) { return n >= SIA_NFFT ? 1 + (n - SIA_NFFT) / hop : 0; }
 
 // per-chunk metadata (nb streams); every array lives in d_meta
 struct StreamMeta {
@@ -168,6 +168,7 @@ struct sia_stream {
   sia_ctx *c = nullptr;
   int32_t n = 0;
   sia_fp_params p{};
+  int hop = 0;                         // frame k starts at sample k * hop (fp_hop of p)
   int r2 = 0;                          // 2 * nbhd carried rows
   int cur = 0;                         // state copy of the last successful push
   int16_t *tails[2] = {nullptr, nullptr};
@@ -204,7 +205,7 @@ int sia_stream_create(sia_ctx *c, int32_t n_streams, const sia_fp_params *p, sia
   SIA_CUDA(cudaSetDevice(c->device));
   sia_stream *st = new (std::nothrow) sia_stream();
   SIA_REQUIRE(st != nullptr, SIA_E_NOMEM, "out of host memory");
-  st->c = c; st->n = n_streams; st->p = *p; st->r2 = 2 * p->nbhd;
+  st->c = c; st->n = n_streams; st->p = *p; st->hop = fp_hop(p); st->r2 = 2 * p->nbhd;
   st->L.assign(n_streams, 0); st->F.assign(n_streams, 0); st->npk.assign(n_streams, 0);
   const size_t S = (size_t)n_streams;
   auto alloc = [&](void **q, size_t bytes) -> int {
@@ -243,7 +244,7 @@ int sia_stream_push(sia_stream *st, const int16_t *d_pcm, const int64_t *h_block
   SIA_REQUIRE(!any_pcm || d_pcm, SIA_E_INVALID, "d_pcm is NULL");
   sia_ctx *c = st->c;
   const sia_fp_params &p = st->p;
-  const int nbhd = p.nbhd;
+  const int nbhd = p.nbhd, hop = st->hop;
   SIA_CUDA(cudaSetDevice(c->device));
   cudaStream_t s = (cudaStream_t)stream;
 
@@ -255,18 +256,18 @@ int sia_stream_push(sia_stream *st, const int16_t *d_pcm, const int64_t *h_block
     Plan &q = pl[b];
     const int64_t F = st->F[b], L = st->L[b];
     q.end = h_end && h_end[b];
-    q.tail = L - F * SIA_HOP;
+    q.tail = L - F * hop;
     q.st_start = stage_total;
     q.st_len = q.tail + h_block_len[b];
     stage_total += (q.st_len + 7) / 8 * 8;
     const int64_t Ln = L + h_block_len[b];
-    int64_t Fn = complete_frames(Ln);
+    int64_t Fn = complete_frames(Ln, hop);
     if (q.end && Fn == 0) Fn = 1;       // short input: one zero-padded frame, like the batch path
     q.f_new = Fn;
     q.n_new = Fn - F;
     q.r_old = std::min<int64_t>(st->r2, F);
     q.r_new = q.end ? 0 : std::min<int64_t>(st->r2, Fn);
-    q.tail_new = q.end ? 0 : q.st_len - q.n_new * SIA_HOP;
+    q.tail_new = q.end ? 0 : q.st_len - q.n_new * hop;
     q.t_base = F - q.r_old;
     const int64_t h_old = F - 1 - nbhd, h_new = q.end ? Fn - 1 : Fn - 1 - nbhd;
     q.lo = std::max<int64_t>(h_old + 1, 0) - q.t_base;
@@ -357,7 +358,7 @@ int sia_stream_push(sia_stream *st, const int16_t *d_pcm, const int64_t *h_block
       StftLaunch a;
       a.d_pcm = st->stage; a.d_track_starts = m.st_start; a.d_track_len = m.st_len; a.d_frame_starts = m.fs1;
       a.n_tracks = nb; a.total_frames = ch.new_rows; a.d_spec = st->k1_rows; a.out_type = SIA_F32;
-      a.frames_per_cta = 8; a.compute = p.compute; a.Fs = p.Fs;
+      a.frames_per_cta = 8; a.compute = p.compute; a.Fs = p.Fs; a.hop = hop;
       if (ch.new_rows > 0) {
         Timer t(c, s, T_STFT, 1);
         if ((rc = stft_db_launch(a, c->tf, c->td, s))) return rc;

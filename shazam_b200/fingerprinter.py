@@ -97,6 +97,9 @@ class Fingerprinter:
 
     Defaults follow the reference's constants (``__init__.py:40-51``): window 4096, overlap
     0.5, fan 5, amp_min 10 dB, square 21x21 footprint (CONNECTIVITY_MASK 2, neighbourhood 10).
+    ``wratio`` (the overlap ratio) may be any value with ``0 <= int(4096 * wratio) <= 4095``; peak times
+    and ``t1`` then count frames of hop ``4096 - int(4096 * wratio)``, so an index is built and queried
+    at one ``wratio``.
     ``compute='f64'`` runs the FFT in double precision (every bin within 1e-3 dB of the
     reference's float64 specgram); ``'f32'`` is the fast mode.
     """
@@ -160,7 +163,8 @@ class Fingerprinter:
         """K1: int16 PCM on the device -> dB spectrogram [frames, F_STRIDE] (time-major)."""
         starts = np.ascontiguousarray(starts, np.int64)
         lens = np.ascontiguousarray(lens, np.int64)
-        frames = int(sum(N.num_frames(n) for n in lens))
+        hop = N.hop_of(p)
+        frames = int(sum(N.num_frames(n, hop) for n in lens))
         spec = torch.full((frames, N.F_STRIDE), float("-inf"), dtype=out_dtype, device=self.tdev)
         total = C.c_int64()
         N.check(self.lib.sia_stft_db(self._h, C.c_void_p(d_pcm.data_ptr()), _i64(starts), _i64(lens), len(lens),
@@ -225,7 +229,7 @@ class Fingerprinter:
             hsh, t1 = out
             cap = t1.numel()
         else:
-            cap = int(cap_hashes) if cap_hashes is not None else self.default_cap(lens, p.fan_value)
+            cap = int(cap_hashes) if cap_hashes is not None else self.default_cap(lens, p.fan_value, N.hop_of(p))
             hsh = torch.empty((cap, N.HASH_BYTES), dtype=torch.uint8, device=self.tdev)
             t1 = torch.empty(cap, dtype=torch.int32, device=self.tdev)
         ths = np.zeros(nt + 1, np.int64)
@@ -252,7 +256,7 @@ class Fingerprinter:
             hsh, t1 = out
             cap = t1.numel() if isinstance(t1, torch.Tensor) else len(t1)
         else:
-            cap = int(cap_hashes) if cap_hashes is not None else self.default_cap(lens, p.fan_value)
+            cap = int(cap_hashes) if cap_hashes is not None else self.default_cap(lens, p.fan_value, N.hop_of(p))
             hsh = np.empty((cap, N.HASH_BYTES), np.uint8)
             t1 = np.empty(cap, np.int32)
         hp = hsh.data_ptr() if isinstance(hsh, torch.Tensor) else hsh.ctypes.data
@@ -265,8 +269,8 @@ class Fingerprinter:
         return FingerprintBatch(hsh[:total.value], t1[:total.value], ths)
 
     @staticmethod
-    def default_cap(lens, fan_value: int) -> int:
-        frames = sum(N.num_frames(int(n)) for n in lens)
+    def default_cap(lens, fan_value: int, hop: int = N.HOP) -> int:
+        frames = sum(N.num_frames(int(n), hop) for n in lens)
         return int(max(4096, frames * 8 * max(fan_value - 1, 1)))
 
     def deinterleave(self, d_interleaved: torch.Tensor, n_channels: int):
@@ -281,7 +285,7 @@ class Fingerprinter:
         return out, np.arange(n_channels, dtype=np.int64) * stride, np.full(n_channels, n_frames, np.int64)
 
     def fingerprint_interleaved(self, pcm_interleaved, n_channels: int, Fs=44100, fan_value=5, amp_min=10,
-                                connectivity=2, nbhd=10, compute="f64") -> FingerprintBatch:
+                                connectivity=2, nbhd=10, compute="f64", wratio=0.5) -> FingerprintBatch:
         """All channels of one decoded file as one GPU batch (SURVEY §8f-1): the interleaved samples are copied
         once, split on the device and fingerprinted channel by channel; digests stay in HBM (one track per
         channel), e.g. for ``ingest.union_channels_device``."""
@@ -290,8 +294,8 @@ class Fingerprinter:
             host = host.copy()
         x = torch.from_numpy(host).to(self.tdev)
         d_pcm, starts, lens = self.deinterleave(x, n_channels)
-        p = self.params(Fs, fan_value, amp_min, connectivity, nbhd, compute)
-        cap = self.default_cap(lens, fan_value)
+        p = self.params(Fs, fan_value, amp_min, connectivity, nbhd, compute, wratio=wratio)
+        cap = self.default_cap(lens, fan_value, N.hop_of(p))
         for _ in range(6):
             try:
                 return self.fingerprint_device(d_pcm, starts, lens, p, cap_hashes=cap)
@@ -302,12 +306,12 @@ class Fingerprinter:
         raise N.CapacityError(N.E_CAPACITY, "hash output keeps overflowing")
 
     def fingerprint_tracks(self, tracks: Sequence[np.ndarray], Fs=44100, fan_value=5, amp_min=10,
-                           connectivity=2, nbhd=10, compute="f64") -> FingerprintBatch:
+                           connectivity=2, nbhd=10, compute="f64", wratio=0.5) -> FingerprintBatch:
         """Convenience: list of int16 arrays -> host digests (with a capacity retry)."""
         tracks = [as_pcm_int16(t) for t in tracks]
         pcm, starts, lens = pack_tracks(tracks)
-        p = self.params(Fs, fan_value, amp_min, connectivity, nbhd, compute)
-        cap = self.default_cap(lens, fan_value)
+        p = self.params(Fs, fan_value, amp_min, connectivity, nbhd, compute, wratio=wratio)
+        cap = self.default_cap(lens, fan_value, N.hop_of(p))
         for _ in range(6):
             try:
                 return self.fingerprint_host(pcm, starts, lens, p, cap_hashes=cap)

@@ -34,13 +34,14 @@ class StreamFingerprinter:
     with a bigger output buffer or smaller blocks."""
 
     def __init__(self, fp: Fingerprinter, n_streams: int, Fs=44100, fan_value=5, amp_min=10, connectivity=2,
-                 nbhd=10, compute="f64"):
+                 nbhd=10, compute="f64", wratio=0.5):
         if not torch.cuda.is_available():
             raise RuntimeError("sia_b200 needs a CUDA device (B200); there is no CPU fallback")
         self.fp = fp
         self.lib = fp.lib
         self.n_streams = int(n_streams)
-        self.p = fp.params(Fs, fan_value, amp_min, connectivity, nbhd, compute)
+        self.p = fp.params(Fs, fan_value, amp_min, connectivity, nbhd, compute, wratio=wratio)
+        self.hop = N.hop_of(self.p)
         h = C.c_void_p()
         N.check(self.lib.sia_stream_create(fp._h, self.n_streams, C.byref(self.p), C.byref(h)))
         self._h = h
@@ -69,7 +70,7 @@ class StreamFingerprinter:
     def default_cap(self, lens) -> int:
         """Hash rows a push of blocks of these lengths needs at most, with the batch path's allowance per frame."""
         fan = int(self.p.fan_value)
-        frames = int(sum(int(n) // N.HOP + 2 + int(self.p.nbhd) for n in lens))
+        frames = int(sum(int(n) // self.hop + 2 + int(self.p.nbhd) for n in lens))
         return int(max(4096, (frames * 8 + self.n_streams * fan) * max(fan - 1, 1)))
 
     def push_device(self, d_pcm: torch.Tensor, starts, lens, end=None, out: Optional[tuple] = None,
