@@ -48,7 +48,8 @@ extern "C" {
 #define SIA_ROW_WORDS   65     /* 32-bit words per row of the peak bitmap */
 #define SIA_HASH_BYTES  10     /* FINGERPRINT_REDUCTION(20 hex chars)/2, __init__.py:51 */
 #define SIA_MAX_DT      200    /* MAX_HASH_TIME_DELTA, __init__.py:50 */
-#define SIA_MAX_NBHD    16     /* largest PEAK_NEIGHBORHOOD_SIZE supported (reference: 10) */
+#define SIA_MAX_NBHD    64     /* largest PEAK_NEIGHBORHOOD_SIZE supported (reference: 10); 64 frames are ~3 s at
+                                 * hop 2048, against MAX_HASH_TIME_DELTA = 200 frames */
 
 enum {
   SIA_OK = 0,
@@ -80,7 +81,9 @@ typedef struct sia_fp_params {
   int32_t fan_value;     /* DEFAULT_FAN_VALUE 5; partners per peak = fan_value-1; <= 64 */
   double  amp_min;       /* DEFAULT_AMP_MIN 10 (dB); negative values enable the erosion term */
   int32_t connectivity;  /* CONNECTIVITY_MASK: 2 = square (reference default), 1 = diamond */
-  int32_t nbhd;          /* PEAK_NEIGHBORHOOD_SIZE 10; 1..SIA_MAX_NBHD */
+  int32_t nbhd;          /* PEAK_NEIGHBORHOOD_SIZE 10; 1..SIA_MAX_NBHD (64) with either connectivity: the window
+                          * (2*nbhd+1 square, or |dt| + |df| <= nbhd) is clipped to the track's frames and bins
+                          * 0..2048; nbhd < 1 or > 64: SIA_E_INVALID */
   int32_t compute;       /* SIA_F64 (default; |dB error| << 1e-3 on every bin) or SIA_F32 */
 } sia_fp_params;
 
@@ -176,7 +179,7 @@ int sia_ctx_timing(sia_ctx *ctx, int enable, double *h_ms_out, int32_t *h_launch
  * carried 2*nbhd rows + its new frames of each stream to fit max_chunk_frames.
  *
  * The handle keeps per-stream state in HBM (allocated at create, two copies: ~2 * (8 KB + nbhd * 16.6 KB) per stream,
- * plus one max_chunk_frames spectrogram for new rows) and uses its context's workspaces: calls on a context and its
+ * 2.1 MB at nbhd 64, plus one max_chunk_frames spectrogram for new rows) and uses its context's workspaces: calls on a context and its
  * stream handles must be serialised by the caller, and stream handles are destroyed before their context.
  * Parameters as sia_fingerprint_batch (wsize 4096 only). */
 typedef struct sia_stream sia_stream;

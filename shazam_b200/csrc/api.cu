@@ -40,7 +40,7 @@ int check_params(const sia_fp_params *p) {
   SIA_REQUIRE(p->Fs > 0, SIA_E_INVALID, "Fs must be positive");
   SIA_REQUIRE(p->fan_value >= 1 && p->fan_value <= 64, SIA_E_INVALID, "fan_value must be in 1..64");
   SIA_REQUIRE(p->connectivity == 1 || p->connectivity == 2, SIA_E_INVALID, "connectivity must be 1 or 2");
-  SIA_REQUIRE(p->nbhd >= 1 && p->nbhd <= SIA_MAX_NBHD, SIA_E_INVALID, "nbhd must be in 1..16");
+  SIA_REQUIRE(p->nbhd >= 1 && p->nbhd <= SIA_MAX_NBHD, SIA_E_INVALID, "nbhd must be in 1..64");
   SIA_REQUIRE(p->compute == SIA_F32 || p->compute == SIA_F64, SIA_E_INVALID, "compute must be SIA_F32 or SIA_F64");
   return SIA_OK;
 }

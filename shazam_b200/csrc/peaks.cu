@@ -9,7 +9,7 @@
 //   peak = (A == max(window)) and not all(window == 0) and A > amp_min.
 // The all-zero term can only matter when amp_min < 0 and is compiled in only then.
 //
-// Stage 1 writes a bitmap, 1 bit per spectrogram element.  Three kernels:
+// Stage 1 writes a bitmap, 1 bit per spectrogram element.  Four kernels:
 //   peaks_square_warp_tma_kernel  the pipeline's kernel (float32 dB, square 21x21 = CONNECTIVITY_MASK 2, the reference
 //     default, amp_min >= 0): persistent CTAs walk 64-frame x 96-bin tiles; the 84 x 120 halo tile arrives by one TMA
 //     tensor copy (cp.async.bulk.tensor.2d, out-of-range elements arrive as zeros), double-buffered on two mbarriers;
@@ -20,7 +20,11 @@
 //     64-frame x 128-bin tile + halo in shared memory; the separable filter as a sliding max down the frames with
 //     threads along bins, a transposed store, then a sliding max along the bins with threads along frames (register
 //     windows, log-doubling); plain bitmap [frame][65 words];
-//   peaks_generic_kernel<T>  any half-width <= SIA_MAX_NBHD, square or diamond, brute force from the same tile.
+//   peaks_footprint_kernel<T, EROSION>  every other footprint, half-width 1..SIA_MAX_NBHD, square or diamond: halo tile
+//     in shared memory, van Herk / Gil-Werman sliding maxima along lines (square: time then bins; diamond: two lattice
+//     classes of an antidiagonal then a diagonal pass), the erosion term by the same filter on |A|; plain bitmap;
+//   peaks_generic_kernel<T>  the diamond at half-width <= 3 (float32 input) or 1 (float64), brute force: it is faster
+//     there (DESIGN §14).
 // Stage 2 (peaks_rowcount/extract): bitmap -> per-row popcounts -> scan -> ordered
 //   (t asc, f asc) peak lists per track, which is the order generate_hashes' stable
 //   sort by time produces (__init__.py:194-195).
@@ -42,6 +46,7 @@ namespace {
 
 constexpr int kThreads = 256;
 constexpr int RC = 16;  // outputs per thread in the sliding passes
+constexpr size_t kMaxSmemOptin = 227 * 1024;  // dynamic shared memory one CTA may opt in to (sm_100)
 
 template <typename T> __device__ __forceinline__ T neg_inf();
 template <> __device__ __forceinline__ float neg_inf<float>() { return -CUDART_INF_F; }
@@ -392,13 +397,217 @@ int launch_square_warp(const PeaksLaunch &a, cudaStream_t s) {
   return SIA_OK;
 }
 
-// ---- generic path: any half-width <= SIA_MAX_NBHD, square or diamond, brute force -----------------
+// ---- footprint-general path: any half-width r in 1..SIA_MAX_NBHD, square or diamond ------------------------------
+// van Herk / Gil-Werman sliding max along one line: out[k] = max(in[k .. k+W-1]) for the outputs k of block q,
+// [q*W, min(q*W + W, n)); in[] holds n + W - 1 values.  Suffix maxima of block q, then prefix maxima of block q+1
+// combined into the outputs: about 3 max operations per output whatever W is.  ACC folds the result into out[].
+template <typename T, bool ACC>
+__device__ __forceinline__ void vh_block(const T *__restrict__ in, int is, T *__restrict__ out, int os, int n, int W,
+                                         int q) {
+  const int k0 = q * W;
+  T s = neg_inf<T>();
+  for (int k = k0 + W - 1; k >= k0; --k) {
+    s = max(s, in[k * is]);
+    if (k < n) out[k * os] = ACC ? max(out[k * os], s) : s;
+  }
+  T p = neg_inf<T>();
+  const int jend = min(k0 + 2 * W - 1, n + W - 1);
+  for (int j = k0 + W; j < jend; ++j) {
+    p = max(p, in[j * is]);
+    out[(j - W + 1) * os] = max(out[(j - W + 1) * os], p);
+  }
+}
+
+// Shared-memory shape of one footprint tile: TT output frames x TF output bins (TF a multiple of 32), halo r.
+//   A  [TT+2r][(TF+2r)|1]  the spectrogram around the tile, -inf outside the track and outside bins 0..2048
+//   I  square: [TT][(TF+2r)|1] max along time;  diamond: [TT+r][(TF+r)|1] max along one antidiagonal segment
+//   M  [TT][TF+1]           the window maximum
+//   bits [TT][TF/32]
+struct FootprintTile {
+  int r, tt, tf;
+  bool diamond;
+  __host__ __device__ int a_stride() const { return (tf + 2 * r) | 1; }
+  __host__ __device__ int i_rows() const { return diamond ? tt + r : tt; }
+  __host__ __device__ int i_stride() const { return diamond ? (tf + r) | 1 : a_stride(); }
+  size_t smem(size_t elem) const {
+    const size_t vals = (size_t)(tt + 2 * r) * a_stride() + (size_t)i_rows() * i_stride() + (size_t)tt * (tf + 1);
+    return vals * elem + (size_t)tt * (tf / 32) * sizeof(uint32_t);
+  }
+};
+
+constexpr int kFpThreads = 512;
+
+// Reached from r = 2 on float64 input and from r = 4 on float32: smaller diamonds take the brute-force kernel.
+// The L1 ball |dt| + |df| <= r is, in the rotated coordinates u = dt + df, v = dt - df, the square max(|u|, |v|) <= r
+// on the lattice u = v (mod 2).  Its even class (u, v even) is {(i+j, i-j) : i, j in [-k0, k0]}, k0 = floor(r/2),
+// and its odd class {(1+i+j, i-j) : i, j in [-k1, k1-1]}, k1 = floor((r+1)/2): each a Minkowski sum of one segment
+// along the antidiagonal (1,-1) and one along the diagonal (1,1), of r+1 and r points (in either order).  So the
+// diamond max is the larger of two separable maxima, antidiagonal pass first (D1) then diagonal pass (D2).  D1 is
+// evaluated on every position its diagonal segments reach, also outside the track or the bin range: such a
+// position takes the max of the in-range points of its segment (the rest are -inf in A), so the clipped window is
+// exact near every border.
+template <typename T>
+__device__ __forceinline__ void diamond_class(const T *__restrict__ A, T *__restrict__ B, T *__restrict__ M,
+                                              const FootprintTile &g, int odd) {
+  const int r = g.r, TT = g.tt, TF = g.tf, AS = g.a_stride(), BS = g.i_stride(), MS = TF + 1;
+  const int kk = odd ? (r + 1) / 2 : r / 2;
+  const int Wc = odd ? 2 * kk : 2 * kk + 1;  // segment length
+  const int a = -kk, ct = odd;               // segment offsets a .. a+Wc-1; odd class shifted one frame
+  const int pt0 = a + ct, BR = TT + Wc - 1, BC = TF + Wc - 1;   // D1 positions: frames pt0.., bins a.. (tile-local)
+  // D1: B(p) = max_k A(p_t + a + k, p_f - a - k).  Line u = p_t + p_f, window start at A row m = p_t + a.
+  {
+    const int u0 = pt0 + a, nu = BR + BC - 1;
+    const int nq = (min(BR, BC) + Wc - 1) / Wc;
+    for (int task = threadIdx.x; task < nu * nq; task += blockDim.x) {
+      const int q = task / nu, u = u0 + (task - q * nu);
+      const int m_lo = max(pt0 + a, u - BC + 1), m_hi = min(pt0 + a + BR, u + 1);
+      const int n = m_hi - m_lo;
+      if (q * Wc >= n) continue;
+      vh_block<T, false>(A + (m_lo + r) * AS + (u - m_lo + r), AS - 1, B + (m_lo - a - pt0) * BS + (u - m_lo), BS - 1,
+                         n, Wc, q);
+    }
+  }
+  __syncthreads();
+  // D2: M(t, f) = max(M, max_k B(t + k, f + k)) in B's own coordinates, along the diagonals d = f - t
+  {
+    const int nd = TT + TF - 1;
+    const int nq = (min(TT, TF) + Wc - 1) / Wc;
+    for (int task = threadIdx.x; task < nd * nq; task += blockDim.x) {
+      const int q = task / nd, d = task - q * nd - (TT - 1);
+      const int t_lo = max(0, -d), n = min(TT, TF - d) - t_lo;
+      if (q * Wc >= n) continue;
+      if (odd) vh_block<T, true>(B + t_lo * BS + t_lo + d, BS + 1, M + t_lo * MS + t_lo + d, MS + 1, n, Wc, q);
+      else vh_block<T, false>(B + t_lo * BS + t_lo + d, BS + 1, M + t_lo * MS + t_lo + d, MS + 1, n, Wc, q);
+    }
+  }
+  __syncthreads();
+}
+
+// One CTA per 64-frame time tile x TF bins; it walks the time tile in sub-tiles of TT frames.  Per sub-tile:
+// stage A, filter (square: time pass then bin pass; diamond: two classes of D1 + D2), compare the centre with M.
+// EROSION (amp_min < 0) stages |A| in a second round and runs the same filter: the window is all zero iff
+// max |A| == 0 there.
+template <typename T, bool EROSION>
+__global__ void __launch_bounds__(kFpThreads)
+peaks_footprint_kernel(const T *__restrict__ spec, const int64_t *__restrict__ frame_starts,
+                       const int64_t *__restrict__ ttile_starts, int n_tracks, double amp_min, const FootprintTile g,
+                       uint32_t *__restrict__ bitmap) {
+  const int r = g.r, TT = g.tt, TF = g.tf, AS = g.a_stride(), IS = g.i_stride(), MS = TF + 1, WPR = TF / 32;
+  const int AR = TT + 2 * r, AC = TF + 2 * r, W = 2 * r + 1;
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  T *A = reinterpret_cast<T *>(smem_raw);
+  T *I = A + (size_t)AR * AS;
+  T *M = I + (size_t)g.i_rows() * IS;
+  uint32_t *bits = reinterpret_cast<uint32_t *>(M + (size_t)TT * MS);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+
+  const int nft = (SIA_NBINS + TF - 1) / TF;
+  const int64_t tt = blockIdx.x / nft;
+  const int f0 = (int)(blockIdx.x - tt * nft) * TF;
+  const int trk = find_segment(ttile_starts, n_tracks, tt);
+  const int64_t row_lo = frame_starts[trk], row_hi = frame_starts[trk + 1];
+  const int64_t rt = row_lo + (tt - ttile_starts[trk]) * kPeakTileT;
+
+  for (int sub = 0; sub < kPeakTileT; sub += TT) {
+    const int64_t r0 = rt + sub;
+    if (r0 >= row_hi) break;
+    for (int round = 0; round < (EROSION ? 2 : 1); ++round) {
+      for (int i = warp; i < AR; i += nwarps) {
+        const int64_t gr = r0 - r + i;
+        const bool row_ok = gr >= row_lo && gr < row_hi;
+        for (int j = lane; j < AC; j += 32) {
+          const int f = f0 - r + j;
+          T v = neg_inf<T>();
+          if (row_ok && f >= 0 && f < SIA_NBINS) {
+            v = spec[gr * SIA_F_STRIDE + f];
+            if (round && v < (T)0 && v != neg_inf<T>()) v = -v;   // -inf stays 'outside', as in the other kernels
+          }
+          A[i * AS + j] = v;
+        }
+      }
+      __syncthreads();
+      if (!g.diamond) {
+        const int nq = (TT + W - 1) / W;
+        for (int task = threadIdx.x; task < AC * nq; task += blockDim.x) {   // along time, thread = bin column
+          const int q = task / AC, c = task - q * AC;
+          vh_block<T, false>(A + c, AS, I + c, IS, TT, W, q);
+        }
+        __syncthreads();
+        const int nq2 = (TF + W - 1) / W;
+        for (int task = threadIdx.x; task < TT * nq2; task += blockDim.x) {  // along bins, thread = frame row
+          const int q = task / TT, t = task - q * TT;
+          vh_block<T, false>(I + t * IS, 1, M + t * MS, 1, TF, W, q);
+        }
+        __syncthreads();
+      } else {
+        diamond_class<T>(A, I, M, g, 0);
+        diamond_class<T>(A, I, M, g, 1);
+      }
+      for (int t = warp; t < TT; t += nwarps) {
+        const bool row_ok = r0 + t < row_hi;
+        for (int w = 0; w < WPR; ++w) {
+          const int c = 32 * w + lane;
+          if (round == 0) {
+            const T ctr = A[(t + r) * AS + c + r];
+            const bool pk = row_ok && f0 + c < SIA_NBINS && ctr == M[t * MS + c] && (double)ctr > amp_min;
+            const uint32_t word = __ballot_sync(0xffffffffu, pk);
+            if (lane == 0) bits[t * WPR + w] = word;
+          } else {
+            const uint32_t zero = __ballot_sync(0xffffffffu, M[t * MS + c] == (T)0);
+            if (lane == 0) bits[t * WPR + w] &= ~zero;
+          }
+        }
+      }
+      __syncthreads();
+    }
+    for (int idx = threadIdx.x; idx < TT * WPR; idx += blockDim.x) {
+      const int t = idx / WPR, w = idx - t * WPR;
+      const int gw = f0 / 32 + w;
+      if (r0 + t < row_hi && gw < SIA_ROW_WORDS) bitmap[(r0 + t) * kBitmapRowWords + gw] = bits[idx];
+    }
+  }
+}
+
+// The tile shape for (element size, r, footprint): the largest share of output bins among the staged ones that fits
+// one CTA's shared memory.
+FootprintTile footprint_tile(size_t elem, int r, bool diamond) {
+  FootprintTile best{r, 0, 0, diamond};
+  double best_eff = -1.0;
+  for (int tf : {128, 64, 32})
+    for (int tt = kPeakTileT; tt >= 1; tt /= 2) {
+      const FootprintTile g{r, tt, tf, diamond};
+      if (g.smem(elem) > (size_t)kMaxSmemOptin) continue;
+      const double eff = (double)tt * tf / ((double)(tt + 2 * r) * (tf + 2 * r));
+      if (eff > best_eff) { best_eff = eff; best = g; }
+    }
+  return best;
+}
+
+template <typename T, bool E>
+int launch_footprint(const PeaksLaunch &a, cudaStream_t s) {
+  const FootprintTile g = footprint_tile(sizeof(T), a.nbhd, a.connectivity == 1);
+  SIA_REQUIRE(g.tt > 0, SIA_E_UNSUPPORTED, "peaks: no footprint tile fits shared memory");
+  const size_t smem = g.smem(sizeof(T));
+  auto kern = peaks_footprint_kernel<T, E>;
+  SIA_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const int64_t blocks = a.total_ttiles * ((SIA_NBINS + g.tf - 1) / g.tf);
+  kern<<<(unsigned)blocks, kFpThreads, smem, s>>>((const T *)a.d_spec, a.d_frame_starts, a.d_ttile_starts, a.n_tracks,
+                                                 a.amp_min, g, a.d_bitmap);
+  SIA_CHECK_LAUNCH();
+  return SIA_OK;
+}
+
+// ---- brute force: the diamond at small half-widths, where it is faster than the footprint kernel ----
+// Measured (DESIGN §14): faster at nbhd 1 and 3 on float32 input, at nbhd 1 only on float64.
+constexpr int kBruteMaxNbhd = 3;
+inline int brute_max_nbhd(int in_type) { return in_type == SIA_F64 ? 1 : kBruteMaxNbhd; }
+
 template <typename T>
 __global__ void __launch_bounds__(kThreads)
 peaks_generic_kernel(const T *__restrict__ spec, const int64_t *__restrict__ frame_starts,
                      const int64_t *__restrict__ ttile_starts, int n_tracks, double amp_min, int nb, int diamond,
                      int erosion, uint32_t *__restrict__ bitmap) {
-  constexpr int TT = kPeakTileT, TF = kPeakTileF, N = SIA_MAX_NBHD;
+  constexpr int TT = kPeakTileT, TF = kPeakTileF, N = kBruteMaxNbhd;
   constexpr int ROWS = TT + 2 * N, COLS = TF + 2 * N;
   constexpr int AS = COLS | 1;
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -448,7 +657,7 @@ int launch_square(const PeaksLaunch &a, cudaStream_t s) {
 
 template <typename T>
 int launch_generic(const PeaksLaunch &a, cudaStream_t s) {
-  constexpr int N = SIA_MAX_NBHD;
+  constexpr int N = kBruteMaxNbhd;
   constexpr int ROWS = kPeakTileT + 2 * N, COLS = kPeakTileF + 2 * N, AS = COLS | 1;
   const size_t smem = sizeof(T) * ROWS * AS;
   auto kern = peaks_generic_kernel<T>;
@@ -583,11 +792,11 @@ extract_kernel(const uint32_t *__restrict__ bitmap, const int64_t *__restrict__ 
 int peaks_bitmap_launch(const PeaksLaunch &a, cudaStream_t s, bool *striped) {
   *striped = false;
   if (a.total_ttiles == 0) return SIA_OK;
-  SIA_REQUIRE(a.nbhd >= 1 && a.nbhd <= SIA_MAX_NBHD, SIA_E_UNSUPPORTED, "peaks: nbhd must be in 1..16");
+  SIA_REQUIRE(a.nbhd >= 1 && a.nbhd <= SIA_MAX_NBHD, SIA_E_UNSUPPORTED, "peaks: nbhd must be in 1..64");
   SIA_REQUIRE(a.connectivity == 1 || a.connectivity == 2, SIA_E_UNSUPPORTED, "peaks: connectivity must be 1 or 2");
   const bool erosion = a.amp_min < 0;
   if (a.connectivity == 2 && a.nbhd == 10) {
-    // (double + erosion would need 255 KB of shared memory: it takes the generic kernel)
+    // (double + erosion would need 255 KB of shared memory: it takes the footprint kernel)
     if (a.in_type == SIA_F64 && !erosion) return launch_square<double, 10, false>(a, s);
     if (a.in_type == SIA_F32 && !erosion) {
       *striped = true;
@@ -595,7 +804,10 @@ int peaks_bitmap_launch(const PeaksLaunch &a, cudaStream_t s, bool *striped) {
     }
     if (a.in_type == SIA_F32) return launch_square<float, 10, true>(a, s);
   }
-  return a.in_type == SIA_F64 ? launch_generic<double>(a, s) : launch_generic<float>(a, s);
+  if (a.connectivity == 1 && a.nbhd <= brute_max_nbhd(a.in_type))
+    return a.in_type == SIA_F64 ? launch_generic<double>(a, s) : launch_generic<float>(a, s);
+  if (a.in_type == SIA_F64) return erosion ? launch_footprint<double, true>(a, s) : launch_footprint<double, false>(a, s);
+  return erosion ? launch_footprint<float, true>(a, s) : launch_footprint<float, false>(a, s);
 }
 
 int peaks_rowcount_launch(const uint32_t *d_bitmap, bool striped, int64_t total_frames, uint32_t *d_row_count,

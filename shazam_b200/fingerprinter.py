@@ -135,6 +135,8 @@ class Fingerprinter:
     @staticmethod
     def params(Fs=44100, fan_value=5, amp_min=10, connectivity=2, nbhd=10, compute="f64",
                wsize=4096, wratio=0.5) -> N.FpParams:
+        """``fingerprint()``'s parameters; ``connectivity`` 2 (square) or 1 (diamond) and ``nbhd`` 1..64 set the peak
+        footprint (``CONNECTIVITY_MASK``, ``PEAK_NEIGHBORHOOD_SIZE``)."""
         p = N.default_params()
         p.Fs = float(Fs)
         p.wsize = int(wsize)
