@@ -11,8 +11,9 @@
 //
 // Stage 1 writes a bitmap, 1 bit per spectrogram element.  Four kernels:
 //   peaks_square_warp_tma_kernel  the pipeline's kernel (float32 dB, square 21x21 = CONNECTIVITY_MASK 2, the reference
-//     default, amp_min >= 0): persistent CTAs walk 64-frame x 96-bin tiles; the 84 x 120 halo tile arrives by one TMA
-//     tensor copy (cp.async.bulk.tensor.2d, out-of-range elements arrive as zeros), double-buffered on two mbarriers;
+//     default, amp_min >= 0): persistent CTAs (4 per SM) walk 64-frame x 96-bin tiles; the 84 x 120 halo tile arrives
+//     by one TMA tensor copy (cp.async.bulk.tensor.2d, out-of-range elements arrive as zeros) into one buffer on an
+//     mbarrier, the next tile prefetched into L2 meanwhile (cp.async.bulk.prefetch.tensor);
 //     each warp owns 16 frames, each lane a float4 column: vertical 21-max in registers (van Herk / Gil-Werman: suffix
 //     maxima of one block of rows, prefix maxima of the next, one max to combine), horizontal 21-max across lanes with
 //     shuffles; 4 ballots per frame go to a striped bitmap [frame][22 strips][4 words];
@@ -225,10 +226,10 @@ peaks_square_kernel(const T *__restrict__ spec, const int64_t *__restrict__ fram
 
 // ---- production path: float32, square 21x21, amp_min >= 0 ------------------------------------------------
 // One CTA = 64 frames x 96 bins (3 bitmap words per frame); 4 warps, warp q owns frames 16q..16q+15.
-// The 84 x 120 halo tile is staged in shared memory as float4 (conflict-free 128-bit accesses).  Each lane
-// owns one float4 column: it slides the 21-frame max down its 4 bins entirely in registers (log-doubling,
-// 36 float4 in flight), then takes the 21-bin max across lanes with 10 shuffles of per-lane prefix /
-// suffix / block maxima — no second shared-memory pass, no transposes.  Lanes 0..23 produce the 96
+// The 84 x 120 halo tile is staged in shared memory as float4.  Each lane owns one float4 column: it slides
+// the 21-frame max down its 4 bins entirely in registers (van Herk, two bins at a time), then takes the
+// 21-bin max across lanes with 10 shuffles of per-lane prefix / suffix / block maxima — no second
+// shared-memory pass, no transposes.  Lanes 0..23 produce the 96
 // outputs, lanes 24..29 carry the +-12-bin halo columns, lanes 30..31 idle.
 constexpr int kW2Rows = kPeakTileT;                                 // 64
 constexpr int kW2Bins = 96;
@@ -245,14 +246,22 @@ __device__ __forceinline__ void warp_tile_peaks(const float4 *__restrict__ A, ui
   auto src = [&](int k) { return lane < kW2Cols4 ? (lane + k + kW2Cols4) % kW2Cols4 : lane; };
   const int s_m1 = src(-1), s_m2 = src(-2), s_m3 = src(-3), s_p1 = src(1), s_p2 = src(2), s_p3 = src(3);
 
+  // the vertical pass one half of the column at a time (bins 0,1 then 2,3): 72 values in flight instead of 144, so
+  // the kernel fits the registers of kW2CtasPerSM resident CTAs
   float vx[36], vy[36], vz[36], vw[36];
+  const float2 *A2 = reinterpret_cast<const float2 *>(A);
 #pragma unroll
   for (int i = 0; i < 36; ++i) {
-    const float4 t = A[(16 * q + i) * kW2Cols4 + col];
-    vx[i] = t.x; vy[i] = t.y; vz[i] = t.z; vw[i] = t.w;
+    const float2 t = A2[2 * ((16 * q + i) * kW2Cols4 + col)];
+    vx[i] = t.x; vy[i] = t.y;
   }
   vanherk21_36(vx);
   vanherk21_36(vy);
+#pragma unroll
+  for (int i = 0; i < 36; ++i) {
+    const float2 t = A2[2 * ((16 * q + i) * kW2Cols4 + col) + 1];
+    vz[i] = t.x; vw[i] = t.y;
+  }
   vanherk21_36(vz);
   vanherk21_36(vw);
 
@@ -297,54 +306,63 @@ __device__ __forceinline__ void warp_tile_peaks(const float4 *__restrict__ A, ui
   }
 }
 
-// Persistent kernel: 2 CTAs per SM walk the tiles with a stride of the grid, two tile buffers
-// each; the TMA copy of the next tile is in flight while the current one is filtered, so no warp ever waits for
-// the tile it is about to read (the copy engine does the staging, the 128 threads only compute).
+// Persistent kernel: 4 CTAs per SM walk the tiles with a stride of the grid, one tile buffer each.  The next tile is
+// prefetched into L2 while the current one is filtered, and copied into the buffer once the buffer is free.  One
+// buffer (41 KB) instead of two lets 4 CTAs = 16 warps share an SM instead of 2 CTAs = 8 warps, which hides the
+// latency of the filter's dependent max / shuffle chains; the copy waits of one CTA are covered by the other three.
+constexpr int kW2CtasPerSM = 4;
 constexpr size_t kW2TileBytes = sizeof(float4) * kW2TileRows * kW2Cols4;
-constexpr size_t kW2PersistSmem = 2 * kW2TileBytes + 128;
+constexpr size_t kW2PersistSmem = kW2TileBytes + 128;
 
-__global__ void __launch_bounds__(kW2Threads, 2)
+__global__ void __launch_bounds__(kW2Threads, kW2CtasPerSM)
 peaks_square_warp_tma_kernel(const int64_t *__restrict__ frame_starts, const int64_t *__restrict__ ttile_starts, int n_tracks,
                              int64_t n_tiles, float amp_lo, uint32_t *__restrict__ bitmap,
                              const __grid_constant__ CUtensorMap tmap) {
   extern __shared__ __align__(128) unsigned char w2_smem[];
-  float4 *bufs[2] = {reinterpret_cast<float4 *>(w2_smem), reinterpret_cast<float4 *>(w2_smem + kW2TileBytes)};
-  unsigned long long *bars = reinterpret_cast<unsigned long long *>(w2_smem + 2 * kW2TileBytes);
-  const uint32_t bar0 = (uint32_t)__cvta_generic_to_shared(bars);
+  float4 *A = reinterpret_cast<float4 *>(w2_smem);
+  unsigned long long *bar = reinterpret_cast<unsigned long long *>(w2_smem + kW2TileBytes);
+  const uint32_t bar0 = (uint32_t)__cvta_generic_to_shared(bar);
   const uint32_t base0 = (uint32_t)__cvta_generic_to_shared(w2_smem);
   if (threadIdx.x == 0) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;\n" ::"r"(bar0));
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;\n" ::"r"(bar0 + 8));
     asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
   }
   __syncthreads();
-  // thread 0: start the tensor copy of tile `tile` into buffer b
-  auto issue = [&](int64_t tile, int b) {
+  // tensor coordinates (first bin, first frame) of the halo tile of `tile`
+  auto coords = [&](int64_t tile, int &x, int &y) {
     const int64_t tt = tile / kW2Strips;
     const int strip = (int)(tile - tt * kW2Strips);
     const int trk = find_segment(ttile_starts, n_tracks, tt);
-    const int64_t r0 = frame_starts[trk] + (tt - ttile_starts[trk]) * kW2Rows;
+    x = strip * kW2Bins - 12;
+    y = (int)(frame_starts[trk] + (tt - ttile_starts[trk]) * kW2Rows - 10);
+  };
+  // thread 0: start the tensor copy of tile `tile` into the buffer
+  auto issue = [&](int64_t tile) {
+    int x, y;
+    coords(tile, x, y);
     asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");   // earlier generic writes (zeroed frames) vs the copy
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n" ::"r"(bar0 + 8 * b), "r"((uint32_t)kW2TileBytes)
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n" ::"r"(bar0), "r"((uint32_t)kW2TileBytes)
                  : "memory");
     asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];\n"
-                 ::"r"(base0 + (uint32_t)(b * kW2TileBytes)), "l"(reinterpret_cast<uint64_t>(&tmap)),
-                 "r"(strip * kW2Bins - 12), "r"((int)(r0 - 10)), "r"(bar0 + 8 * b) : "memory");
+                 ::"r"(base0), "l"(reinterpret_cast<uint64_t>(&tmap)), "r"(x), "r"(y), "r"(bar0) : "memory");
   };
   int64_t tile = blockIdx.x;
-  if (threadIdx.x == 0 && tile < n_tiles) issue(tile, 0);
+  if (threadIdx.x == 0 && tile < n_tiles) issue(tile);
   for (int k = 0; tile < n_tiles; tile += gridDim.x, ++k) {
-    const int b = k & 1;
-    // the other buffer was released by the barrier that ended the previous iteration
-    if (threadIdx.x == 0 && tile + gridDim.x < n_tiles) issue(tile + gridDim.x, b ^ 1);
+    const bool has_next = tile + gridDim.x < n_tiles;
+    if (threadIdx.x == 0 && has_next) {
+      int x, y;
+      coords(tile + gridDim.x, x, y);
+      asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];\n"
+                   ::"l"(reinterpret_cast<uint64_t>(&tmap)), "r"(x), "r"(y) : "memory");
+    }
     const int64_t tt = tile / kW2Strips;
     const int strip = (int)(tile - tt * kW2Strips);
     const int trk = find_segment(ttile_starts, n_tracks, tt);
     const int64_t row_lo = frame_starts[trk], row_hi = frame_starts[trk + 1];
     const int64_t r0 = row_lo + (tt - ttile_starts[trk]) * kW2Rows;
     asm volatile("{\n.reg .pred P1;\nLAB_WAIT:\nmbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n@P1 bra DONE;\nbra LAB_WAIT;\nDONE:\n}\n"
-                 ::"r"(bar0 + 8 * b), "r"((k >> 1) & 1) : "memory");
-    float4 *A = bufs[b];
+                 ::"r"(bar0), "r"(k & 1) : "memory");
     const int64_t g_first = r0 - 10;
     if (g_first < row_lo || g_first + kW2TileRows > row_hi) {      // first / last tiles of a track: zero the other tracks' frames
       for (int i = threadIdx.x; i < kW2TileRows * kW2Cols4; i += kW2Threads) {
@@ -353,8 +371,9 @@ peaks_square_warp_tma_kernel(const int64_t *__restrict__ frame_starts, const int
       }
       __syncthreads();
     }
-    warp_tile_peaks(A, base0 + (uint32_t)(b * kW2TileBytes), r0, row_hi, strip, strip * kW2Bins, amp_lo, bitmap);
-    __syncthreads();                                               // buffer b may be refilled two tiles from now
+    warp_tile_peaks(A, base0, r0, row_hi, strip, strip * kW2Bins, amp_lo, bitmap);
+    __syncthreads();                                               // every warp is done with the buffer
+    if (threadIdx.x == 0 && has_next) issue(tile + gridDim.x);
   }
 }
 
@@ -390,7 +409,7 @@ int launch_square_warp(const PeaksLaunch &a, cudaStream_t s) {
   int rc = make_spec_tensor_map((const float *)a.d_spec, a.total_frames, &tm);
   if (rc) return rc;
   SIA_CUDA(cudaFuncSetAttribute(peaks_square_warp_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kW2PersistSmem));
-  const unsigned grid = (unsigned)std::min<int64_t>(blocks, 2 * kNumSMs);
+  const unsigned grid = (unsigned)std::min<int64_t>(blocks, kW2CtasPerSM * kNumSMs);
   peaks_square_warp_tma_kernel<<<grid, kW2Threads, kW2PersistSmem, s>>>(a.d_frame_starts, a.d_ttile_starts, a.n_tracks, blocks,
                                                                         amp_lo, a.d_bitmap, tm);
   SIA_CHECK_LAUNCH();
